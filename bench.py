@@ -2,6 +2,7 @@
 """Benchmark of the GP prior term (Woodbury NLL + dNLL/dZ) -- BASELINE.json's metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -12,9 +13,12 @@ BASELINE.json configs[2] (N=1M, L=256, Q=4096: the configuration the north-star 
 fits one B200), row-sharded over the ranks (strong scaling).  Rank 0 prints ONE JSON line.
 
 `--impl reference` times the reference's own CPU implementation of the path on the host cores: the UNMODIFIED
-gp.py / vmod.py from the git-ignored copy under baseline/_ref/ (`__graft_entry__.build()` makes it where
-/root/reference is mounted; it travels to the GPU box with the snapshot), falling back to the op-for-op port in
-oracle/gp_oracle.py (`kind: "port"`).  Each step evaluates a fixed 100k-row sample of the workload (BASELINE.md 3).
+gp.py / vmod.py from the git-ignored copy under baseline/_ref/ (`__graft_entry__.build()` makes it where the reference
+checkout named by BASELINE.json's reference_path exists), falling back to the op-for-op port in oracle/gp_oracle.py
+(`kind: "port"`).  Each step evaluates a fixed 100k-row sample of the workload (BASELINE.md 3).
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident leg returned (see dump_outputs), so that
+two builds can be compared output for output: the inputs are generated from fixed seeds.
 
 `--check` (any --gpus): parity of the multi-GPU path on the real collective -- all ranks' all-reduced G, C and W
 bit-identical, sum(nll) / Xb rows against the unsharded evaluation on rank 0; a failure fails the run.
@@ -318,6 +322,33 @@ def run_check(args, gp, vm, pr, cfg, world, rank, dev):
     return report
 
 
+DUMP_XB_ROWS = 1 << 15       # 32 MB of Xb at L = 256; nll is written whole (4 MB at N = 1M)
+
+
+def dump_outputs(out_dir, result, N, off, n, world, rank, dev):
+    """Write what one step returned to its caller, as float32 .npy files in out_dir: nll (N x 1) and vbs whole, and Xb
+    (N x L) on DUMP_XB_ROWS rows drawn with a fixed seed, in ascending row order (all of Xb where N is not larger).
+    Ranks contribute their own rows to zero-filled buffers summed over the ranks, so the files do not depend on --gpus."""
+    import numpy as np
+    Xb, _, vbs, nll = result
+    nll_all = torch.zeros(N, 1, device=dev, dtype=nll.dtype)
+    nll_all[off:off + n] = nll
+    rows = torch.arange(N) if N <= DUMP_XB_ROWS else \
+        torch.randperm(N, generator=torch.Generator().manual_seed(0))[:DUMP_XB_ROWS].sort().values
+    rows = rows.to(dev)
+    mine = (rows >= off) & (rows < off + n)
+    xb_rows = torch.zeros(rows.numel(), Xb.shape[1], device=dev, dtype=Xb.dtype)
+    xb_rows[mine] = Xb[rows[mine] - off]
+    if world > 1:
+        import torch.distributed as dist
+        dist.all_reduce(nll_all)
+        dist.all_reduce(xb_rows)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, t in (("nll", nll_all), ("vbs", vbs), ("Xb", xb_rows)):
+            np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     import gppvae_b200
@@ -376,14 +407,15 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = _lib.launch_count()
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        out = fn()      # only the last step's results are held: earlier ones are freed as in an ordinary loop
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1) / steps], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), _lib.launch_count() - l0
+        return float(ms.item()), _lib.launch_count() - l0, out
 
     # ---- device-resident throughput (inputs already in HBM)
     sampler = ClockSampler(local)
@@ -392,9 +424,12 @@ def run_ours(args):
     barrier()
     sampler.start()
     gp.stage_hook = hook
-    ms, launches = timed(lambda: step(pr.d, pr.w, pr.Z), args.steps, 0)
+    ms, launches, last = timed(lambda: step(pr.d, pr.w, pr.Z), args.steps, 0)
     gp.stage_hook = None
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, N, off, n, world, rank, dev)
+    del last
     stages = {}
     for (na, ea), (nb, eb) in zip(events[:-1], events[1:]):
         if nb.endswith(":end"):
@@ -408,7 +443,7 @@ def run_ours(args):
     if world == 1 and args.workload != "c3":
         from gppvae_b200.graph import CapturedGPTerm
         cap = CapturedGPTerm(vm, gp, pr.d, pr.w, pr.Z)
-        ms_graph, _ = timed(lambda: cap(), args.steps, 3)
+        ms_graph, _ = timed(lambda: cap(), args.steps, 3)[:2]
         del cap
         gp.invalidate_cache()
 
@@ -419,7 +454,7 @@ def run_ours(args):
             return gp.taylor_coeff(pr.Z, [V], need_vb=True)
     ms_full = None
     if not args.skip_full:
-        ms_full, _ = timed(full_step, max(1, min(args.steps, 3)), 1)
+        ms_full, _ = timed(full_step, max(1, min(args.steps, 3)), 1)[:2]
         gp.invalidate_cache()      # drop the cached V / Binv / planes before the next leg
         torch.cuda.empty_cache()
 
@@ -438,7 +473,7 @@ def run_ours(args):
             kr_step()
         events.clear()
         gp.stage_hook = hook
-        ms_kr, launches_kr = timed(kr_step, args.steps, 0)
+        ms_kr, launches_kr = timed(kr_step, args.steps, 0)[:2]
         gp.stage_hook = None
         st_kr = {}
         for (na, ea), (nb, eb) in zip(events[:-1], events[1:]):
@@ -723,7 +758,13 @@ def main():
     ap.add_argument("--skip-structured", action="store_true", help="omit the structured-route leg")
     ap.add_argument("--check", action="store_true",
                     help="run the sharded-vs-unsharded parity check (always on when more than one rank runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (nll, vbs, a seeded row sample of Xb)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours), not those of --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

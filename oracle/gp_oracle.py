@@ -9,10 +9,9 @@ as shipped" behaviour, float64 for the ground truth used to grade quantities
 the fp32 reference itself cannot pin (``Vb``, ``vbs[0]``; BASELINE.md section 2).
 
 Pinning: ``tests/golden/make_golden.py`` imports the *unmodified* reference
-classes from ``/root/reference/pysrc/faceplace`` (under a three-line shim) and
-stores their inputs/outputs in ``tests/golden/*.npz``; ``tests/test_oracle.py``
-checks every function below against those vectors, and -- when
-``/root/reference`` is mounted -- against the live reference classes as well.
+classes from the reference checkout (under a three-line shim) and stores their
+inputs/outputs in ``tests/golden/*.npz``; ``tests/test_oracle.py`` checks every
+function below against those vectors.
 
 Each function cites the reference lines it follows.  Symbols: ``n`` rows,
 ``Q`` columns of V (= p*q), ``L`` latent dimensions, ``vs = [v0, vn]``.

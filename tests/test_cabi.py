@@ -62,7 +62,10 @@ def test_argument_validation_needs_no_device(lib):
 def test_workspace_sizes_are_consistent(lib):
     for n, Q, L in [(4005, 576, 256), (100_000, 1024, 256), (1_000_000, 4096, 256), (1, 4, 4)]:
         g = lib.gpp_gram_workspace_bytes(n, Q, L)
-        assert g > 0 and g % (128 * 128 * 4) == 0
+        # whole 128 x 128 fp32 partial tiles; the tensor-core pass 1, which serves the shape where a CUDA driver is
+        # present, adds 256 bytes of absmax slots to its own workspace
+        tails = (0, 256) if lib.gpp_planes_supported(n, Q, L) else (0,)
+        assert g > 0 and g % (128 * 128 * 4) in tails
         assert g < 2 << 30, "pass-1 split-K workspace must stay bounded"
         assert lib.gpp_factor_state_bytes(Q) >= 3 * ((Q + 63) // 64 * 64) ** 2 * 4
         assert lib.gpp_solve_workspace_bytes(Q, L) > Q * L * 4
