@@ -17,7 +17,26 @@ GPP_PLANES_COLSQ, GPP_PLANES_UNIT_BOUND = 1, 2
 # scalar slots (enum gpp_scalar_slot)
 S_V0, S_VN, S_LOGDETB, S_TRBINV, S_WNORM2, S_ROWCONST, S_XB2, S_QUAD, NSCAL = range(9)
 
+GPP_MAX_DESIGNS = 16
+
 _PF = c_void_p   # device pointers travel as void*
+# HOST arrays (the k-design entries): of device pointers, of int64 leading dimensions, of int32 column counts
+_PH, _I64H, _I32H = ctypes.POINTER(c_void_p), ctypes.POINTER(c_int64), ctypes.POINTER(c_int32)
+
+
+def host_ptrs(ptrs):
+    """HOST array of device pointers (None entries become NULL)."""
+    return (c_void_p * len(ptrs))(*ptrs)
+
+
+def host_i64(vals):
+    return (c_int64 * len(vals))(*[int(v) for v in vals])
+
+
+def host_i32(vals):
+    return (c_int32 * len(vals))(*[int(v) for v in vals])
+
+
 _SIGNATURES = {
     "gpp_version": (c_int, []),
     "gpp_last_error": (c_char_p, []),
@@ -87,6 +106,19 @@ _SIGNATURES = {
                                          c_int32, _PF, _PF, _PF, c_void_p]),
     "gpp_taylor_expansion_bwd": (c_int, [_PF, _PF, c_int64, _PF, c_int64, c_int64, c_int32, c_int32, _PF, _PF, _PF,
                                          c_int64, _PF, c_int64, _PF, c_void_p]),
+    "gpp_split_stacked_workspace_bytes": (c_size_t, [c_int64, c_int32, _I32H]),
+    "gpp_split_planes_stacked": (c_int, [c_int32, _PH, _I64H, _I32H, c_int64, c_uint32, _PF, c_size_t, _PF, c_size_t,
+                                         c_void_p]),
+    "gpp_factor_blocks_state_bytes": (c_size_t, [c_int32, c_int32]),
+    "gpp_factor_blocks": (c_int, [_PF, c_int64, c_int32, _I32H, _PF, c_uint32, _PF, _PF, _PF, _PF, c_size_t, c_void_p]),
+    "gpp_solve_blocks_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "gpp_solve_w_blocks": (c_int, [_PF, c_int64, c_int32, _I32H, c_int32, c_int32, c_int64, _PF, c_int64, _PF, _PF, _PF,
+                                   c_size_t, _PF, c_size_t, c_void_p]),
+    "gpp_vbs_blocks": (c_int, [_PF, _PF, _PF, c_int32, _I32H, c_int64, c_int32, _PF, c_void_p]),
+    "gpp_taylor_expansion_fwd_multi": (c_int, [_PF, c_int64, _PF, c_int64, c_int32, _PH, _I64H, _PH, _I64H, _I32H, c_int64,
+                                               c_int32, _PF, _PF, _PF, c_void_p]),
+    "gpp_taylor_expansion_bwd_multi": (c_int, [_PF, _PF, c_int64, c_int32, _PH, _I64H, _I32H, c_int64, c_int32, _PF, _PF,
+                                               _PF, c_int64, _PH, _I64H, _PF, c_void_p]),
     "gpp_host_ctx_create": (c_int, [ctypes.POINTER(c_void_p)]),
     "gpp_host_ctx_destroy": (c_int, [c_void_p]),
     "gpp_gp_term_host_submit": (c_int, [c_void_p, _PF, c_int64, c_int32, _PF, c_int64, c_int32, _PF, _PF, _PF, c_int64,

@@ -281,6 +281,85 @@ extern "C" int gpp_vbs(const double* scal, int64_t n_total, int32_t Q, int32_t L
   return launch_vbs(scal, n_total, Q, L, vbs, (cudaStream_t)stream);
 }
 
+// ------------------------------------------------------------------ k stacked designs
+// BlockSpec from the caller's host array of block column counts (each a positive multiple of 4)
+static int block_spec(const char* who, int32_t k, const int32_t* cols_host, BlockSpec& bs) {
+  GPP_REQUIRE(k >= 1 && k <= GPP_MAX_DESIGNS, "%s: k = %d designs (1..%d supported)", who, k, GPP_MAX_DESIGNS);
+  GPP_REQUIRE(cols_host, "%s: null column counts", who);
+  bs = BlockSpec{};
+  bs.k = k;
+  int64_t q = 0;
+  for (int i = 0; i < k; ++i) {
+    GPP_REQUIRE(cols_host[i] > 0 && cols_host[i] % 4 == 0,
+                "%s: design %d has %d columns (a positive multiple of 4 is required)", who, i, cols_host[i]);
+    q += cols_host[i];
+    GPP_REQUIRE(q < (1 << 20), "%s: too many stacked columns", who);
+    bs.start[i + 1] = (int)q;
+  }
+  return GPP_OK;
+}
+
+extern "C" size_t gpp_split_stacked_workspace_bytes(int64_t n, int32_t k, const int32_t* cols_host) {
+  if (!cols_host || k < 1 || k > GPP_MAX_DESIGNS) return 0;
+  return split_stacked_workspace_bytes(n, k, cols_host);
+}
+
+extern "C" int gpp_split_planes_stacked(int32_t k, const float* const* X_host, const int64_t* ldx_host,
+                                        const int32_t* cols_host, int64_t n, uint32_t flags, void* planes,
+                                        size_t planes_bytes_, void* workspace, size_t workspace_bytes,
+                                        gpp_stream_t stream) {
+  BlockSpec bs;
+  GPP_TRY(block_spec("split_planes_stacked", k, cols_host, bs));
+  GPP_REQUIRE(n >= 0 && X_host && ldx_host, "split_planes_stacked: bad n / null host array");
+  for (int i = 0; i < k; ++i)
+    GPP_REQUIRE(mat_ok(X_host[i], ldx_host[i], cols_host[i]),
+                "split_planes_stacked: source %d must be 16-byte aligned with ldx >= cols and ldx %% 4 == 0", i);
+  GPP_REQUIRE(planes_ok(planes) && planes_bytes_ >= planes_bytes(n, bs.start[k]),
+              "split_planes_stacked: planes buffer must be 256-byte aligned and gpp_planes_bytes(n, sum cols) long");
+  return launch_split_planes_stacked(k, X_host, ldx_host, cols_host, n, planes, (flags & GPP_PLANES_UNIT_BOUND) != 0,
+                                     (flags & GPP_PLANES_COLSQ) != 0, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" size_t gpp_factor_blocks_state_bytes(int32_t Q, int32_t k) {
+  return Q > 0 && k >= 1 && k <= GPP_MAX_DESIGNS ? factor_blocks_workspace_bytes(Q, k) : 0;
+}
+extern "C" size_t gpp_solve_blocks_workspace_bytes(int32_t Q, int32_t L, int32_t k) {
+  return Q > 0 && L > 0 && k >= 1 && k <= GPP_MAX_DESIGNS ? solve_blocks_workspace_bytes(Q, L, k) : 0;
+}
+
+extern "C" int gpp_factor_blocks(const float* G, int64_t ldg, int32_t k, const int32_t* cols_host, const float* vs,
+                                 uint32_t flags, float* Binv, double* scal, double* blk, void* state, size_t state_bytes,
+                                 gpp_stream_t stream) {
+  BlockSpec bs;
+  GPP_TRY(block_spec("factor_blocks", k, cols_host, bs));
+  const int Q = bs.start[k];
+  GPP_REQUIRE(mat_ok(G, ldg, Q), "factor_blocks: bad G");
+  GPP_REQUIRE(vs && scal && blk, "factor_blocks: null vs / scal / blk");
+  GPP_REQUIRE(!(flags & GPP_WANT_BINV) || (Binv && aligned16(Binv)), "factor_blocks: Binv required with GPP_WANT_BINV");
+  return launch_factor_blocks(G, ldg, bs, vs, flags, Binv, scal, blk, state, state_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int gpp_solve_w_blocks(const float* C, int64_t ldc, int32_t k, const int32_t* cols_host, int32_t L,
+                                  int32_t L_true, int64_t n_total, float* W, int64_t ldw, double* scal, double* blk,
+                                  const void* state, size_t state_bytes, void* workspace, size_t workspace_bytes,
+                                  gpp_stream_t stream) {
+  BlockSpec bs;
+  GPP_TRY(block_spec("solve_w_blocks", k, cols_host, bs));
+  GPP_REQUIRE(L > 0 && L % 4 == 0 && n_total > 0 && L_true > 0 && L_true <= L, "solve_w_blocks: bad shape L=%d L_true=%d",
+              L, L_true);
+  GPP_REQUIRE(mat_ok(C, ldc, L) && mat_ok(W, ldw, L) && scal && blk, "solve_w_blocks: bad C / W / scal / blk");
+  return launch_solve_w_blocks(C, ldc, bs, L, L_true, n_total, W, ldw, scal, blk, state, state_bytes, workspace,
+                               workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int gpp_vbs_blocks(const double* scal, const double* blk, const float* vs, int32_t k, const int32_t* cols_host,
+                              int64_t n_total, int32_t L, float* vbs, gpp_stream_t stream) {
+  BlockSpec bs;
+  GPP_TRY(block_spec("vbs_blocks", k, cols_host, bs));
+  GPP_REQUIRE(scal && blk && vs && vbs && n_total > 0 && L > 0, "vbs_blocks: bad argument");
+  return launch_vbs_blocks(scal, blk, vs, bs, n_total, L, vbs, (cudaStream_t)stream);
+}
+
 // ------------------------------------------------------------------ Vb
 extern "C" size_t gpp_vb_workspace_bytes(int64_t n, int32_t Q, int32_t L) {
   return tc_rows_supported(n, Q + L, Q) ? tc_vb_workspace_bytes(Q, L) : 0;

@@ -841,6 +841,62 @@ int launch_split_planes(const float* X, int64_t ldx, int64_t n, int cols, void* 
   return GPP_OK;
 }
 
+// Planes of the column concatenation [X_0 | ... | X_{k-1}] (every cols[i] a multiple of 4) written straight into one
+// planes buffer of n x sum(cols): no fp32 concatenation.  One common scale: the exact scans of all sources fold into
+// meta[0] before any source is split (or the bound |x| <= 1 when unit_bound).  Source i is split by the single-matrix
+// kernels at its column offset, and its column sums of squares are reduced into its column range -- fixed order, so
+// diag(G) is exact and reproducible.  The sources are processed one after the other on `st`, so the partial sums reuse
+// one workspace of the largest source's size.
+size_t split_stacked_workspace_bytes(int64_t n, int k, const int* cols) {
+  size_t b = 0;
+  for (int i = 0; i < k; ++i) {
+    const size_t s = split_workspace_bytes(n, cols[i]);
+    if (s > b) b = s;
+  }
+  return b;
+}
+
+int launch_split_planes_stacked(int k, const float* const* X, const int64_t* ldx, const int* cols, int64_t n, void* planes,
+                                bool unit_bound, bool want_colsq, void* ws, size_t ws_bytes, cudaStream_t st) {
+  int total = 0;
+  for (int i = 0; i < k; ++i) total += cols[i];
+  PlanesView pv = planes_view(planes, n, total);
+  if (want_colsq && (!ws || ws_bytes < split_stacked_workspace_bytes(n, k, cols))) {
+    set_error("split_planes_stacked: workspace too small (%zu < %zu bytes)", ws_bytes,
+              split_stacked_workspace_bytes(n, k, cols));
+    return GPP_ERR_WORKSPACE;
+  }
+  if (unit_bound) {
+    planes_meta_kernel<<<1, 32, 0, st>>>(pv.meta, (uint32_t)(1 - 1 + 127) << 23, 0u);   // max|x| < 2^1
+    GPP_LAUNCH_CHECK();
+  } else {
+    GPP_CUDA(cudaMemsetAsync(pv.meta, 0, 4, st));
+    for (int i = 0; i < k; ++i) GPP_TRY(tc_absmax_fold(X[i], ldx[i], n, cols[i], pv.meta, st));
+  }
+  if (n <= 0) return GPP_OK;
+  int off = 0;
+  for (int i = 0; i < k; ++i) {
+    dim3 grid;
+    int64_t rpb;
+    split_grid(n, cols[i], grid, rpb);
+    double* part = want_colsq ? static_cast<double*>(ws) : nullptr;
+    split_planes_kernel<<<grid, 256, 0, st>>>(X[i], ldx[i], n, cols[i], pv.hi + off, pv.lo + off, pv.ldp, pv.meta, rpb,
+                                              part);
+    GPP_LAUNCH_CHECK();
+    if (want_colsq) {
+      colsq_reduce_kernel<<<(unsigned)ceil_div(cols[i], 256), 256, 0, st>>>(part, (int)grid.y, cols[i], pv.colsq + off,
+                                                                            pv.meta);
+      GPP_LAUNCH_CHECK();
+    }
+    off += cols[i];
+  }
+  if (!want_colsq) {
+    planes_meta_kernel<<<1, 32, 0, st>>>(pv.meta, 0u, 0u);
+    GPP_LAUNCH_CHECK();
+  }
+  return GPP_OK;
+}
+
 int launch_kr_planes(const float* xn, int64_t P, int p, const float* wn, int64_t nviews, int q, const int64_t* d,
                      const int64_t* w, int64_t n, float* V, int64_t ldv, void* planes, void* ws, size_t ws_bytes,
                      cudaStream_t st) {

@@ -896,8 +896,10 @@ int make_map_2d(CUtensorMap* m, const float* ptr, int64_t rows, int64_t cols, in
 // Record the bit pattern of max|X| over ALL of X in *slot (zeroed here); the kernels derive the power-of-two scales of
 // the fp16 operands from it.  The scan is exact (one streaming read, cheap next to the GEMM it feeds): an operand scaled
 // from a sampled maximum would silently saturate on an outlier row the sample missed.
-int launch_absmax(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st) {
-  GPP_CUDA(cudaMemsetAsync(slot, 0, 4, st));
+// zero_slot = false: fold X into what *slot already holds (one scale shared by several matrices).
+int launch_absmax(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st,
+                  bool zero_slot = true) {
+  if (zero_slot) GPP_CUDA(cudaMemsetAsync(slot, 0, 4, st));
   if (rows <= 0 || cols < 4) return GPP_OK;
   const int64_t want = ceil_div(rows * (int64_t)cols, 256 * 4 * 8);   // >= 8 float4 per thread
   const int cap = 8 * sm_count();                                      // one wave of 256-thread CTAs
@@ -1022,6 +1024,10 @@ extern "C" int gpp_debug_prof(unsigned long long* out /* [512][16] */) {
 
 int tc_absmax(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st) {
   return launch_absmax(X, ld, rows, cols, slot, st);
+}
+
+int tc_absmax_fold(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st) {
+  return launch_absmax(X, ld, rows, cols, slot, st, false);
 }
 
 bool tc_pass1_supported(int64_t n, int Q, int L) { return Q >= 128 && n >= 512 && encode_fn() != nullptr; }

@@ -4,6 +4,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include "../../include/gppvae_b200.h"
+
 namespace gpp {
 
 // ---- gemm_simt.cu ----
@@ -59,6 +61,8 @@ int launch_tc_blockgemm(const float* Amat, int64_t a_rows, int64_t a_cols, int64
 int launch_tc_syrk_sub(float* C, int64_t ldc, const float* A, int64_t lda, const float* At, int64_t ldat, int n, int K,
                        const uint32_t* amax, cudaStream_t st);
 int tc_absmax(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st);
+// the same scan folded into *slot (not zeroed first): one scale for several matrices
+int tc_absmax_fold(const float* X, int64_t ld, int64_t rows, int cols, uint32_t* slot, cudaStream_t st);
 
 bool tc_available();   // cuTensorMapEncodeTiled resolvable from this driver
 
@@ -114,5 +118,27 @@ int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t 
 int launch_solve_w(const float* C, int64_t ldc, int Q, int L, int L_true, int64_t n_total, float* W, int64_t ldw,
                    double* scal, const void* state, size_t state_bytes, void* ws, size_t ws_bytes, cudaStream_t st);
 int launch_vbs(const double* scal, int64_t n_total, int Q, int L, float* vbs, cudaStream_t st);
+
+// k stacked designs V = [V_0 | ... | V_{k-1}]: block i owns columns [start[i], start[i+1]) (start[k] = Q, every width a
+// positive multiple of 4).  Passed to kernels by value.
+constexpr int kMaxBlocks = GPP_MAX_DESIGNS;
+struct BlockSpec {
+  int k;
+  int start[kMaxBlocks + 1];
+};
+size_t factor_blocks_workspace_bytes(int Q, int k);
+size_t solve_blocks_workspace_bytes(int Q, int L, int k);
+int launch_factor_blocks(const float* G, int64_t ldg, const BlockSpec& bs, const float* vs, uint32_t flags, float* Binv,
+                         double* scal, double* blk, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_solve_w_blocks(const float* C, int64_t ldc, const BlockSpec& bs, int L, int L_true, int64_t n_total, float* W,
+                          int64_t ldw, double* scal, double* blk, const void* state, size_t state_bytes, void* ws,
+                          size_t ws_bytes, cudaStream_t st);
+int launch_vbs_blocks(const double* scal, const double* blk, const float* vs, const BlockSpec& bs, int64_t n_total, int L,
+                      float* vbs, cudaStream_t st);
+
+// ---- gemm_planes.cu / gemm_tc.cu: planes of a stacked design
+size_t split_stacked_workspace_bytes(int64_t n, int k, const int* cols);
+int launch_split_planes_stacked(int k, const float* const* X, const int64_t* ldx, const int* cols, int64_t n, void* planes,
+                                bool unit_bound, bool want_colsq, void* ws, size_t ws_bytes, cudaStream_t st);
 
 }  // namespace gpp

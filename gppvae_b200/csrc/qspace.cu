@@ -826,6 +826,143 @@ int launch_vbs(const double* scal, int64_t n_total, int Q, int L, float* vbs, cu
   return GPP_OK;
 }
 
+// ------------------------------------------------------------------ k stacked designs (block form)
+// V = [V_0 | ... | V_{k-1}], v_i = vs[i], vn = vs[k], D = diag(sqrt(v_i) on the columns of block i):
+//   B = I + D G D / vn,  W = D B^-1 D C / vn,  Binv <- D B^-1 D.
+// The factorisation is the single-design one on that B; afterwards Linv's columns are scaled by D (Linv' = Linv D, still
+// lower triangular and |Linv'| <= |Linv| <= 1), so that the unchanged solve computes Linv'^T Linv' C / vn = W and the
+// unchanged Binv product gives D B^-1 D.  With scal[V0] = 1 the N-long kernels (pass 2, Vb) then compute the k-design
+// Xb and Vb as they stand.  Per block (caller-owned blk[2k]): blk[2i] = tr_i B^-1 (column block i of the UNSCALED Linv),
+// blk[2i + 1] = ||W_i||^2 (row block i of W).
+
+// scal[V0] = 1, scal[VN] = vn; dcol[a] = sqrt(v_i) for the columns a of block i, 1 on the padding up to Qp
+__global__ void blocks_init_kernel(const float* __restrict__ vs, BlockSpec bs, int Qp, double* __restrict__ scal,
+                                   float* __restrict__ dcol) {
+  const int a = blockIdx.x * blockDim.x + threadIdx.x;
+  if (a == 0) {
+    scal[GPP_S_V0] = 1.0;
+    scal[GPP_S_VN] = (double)vs[bs.k];
+  }
+  if (a >= Qp) return;
+  float d = 1.f;
+#pragma unroll
+  for (int i = 0; i < kMaxBlocks; ++i)
+    if (i < bs.k && a >= bs.start[i] && a < bs.start[i + 1]) d = sqrtf(vs[i]);
+  dcol[a] = d;
+}
+
+// Bm (Qp x Qp) = I + D G D / vn on the real Q x Q block, identity on the padding.
+__global__ void __launch_bounds__(256) build_b_blocks_kernel(const float* __restrict__ G, int64_t ldg, int Q, int Qp,
+                                                             const float* __restrict__ dcol,
+                                                             const double* __restrict__ scal, float* __restrict__ Bm) {
+  const float rvn = (float)(1.0 / scal[GPP_S_VN]);
+  const int64_t total4 = (int64_t)Qp * (Qp / 4);
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total4; e += (int64_t)gridDim.x * blockDim.x) {
+    const int i = (int)(e / (Qp / 4));
+    const int j4 = (int)(e - (int64_t)i * (Qp / 4)) * 4;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (i < Q && j4 < Q) {
+      const float4 g = *reinterpret_cast<const float4*>(G + (int64_t)i * ldg + j4);
+      const float4 dj = *reinterpret_cast<const float4*>(dcol + j4);
+      const float ri = dcol[i] * rvn;
+      v = make_float4(ri * dj.x * g.x, ri * dj.y * g.y, ri * dj.z * g.z, ri * dj.w * g.w);
+    }
+    if (i == j4 + 0) v.x += 1.f;
+    if (i == j4 + 1) v.y += 1.f;
+    if (i == j4 + 2) v.z += 1.f;
+    if (i == j4 + 3) v.w += 1.f;
+    *reinterpret_cast<float4*>(Bm + (int64_t)i * Qp + j4) = v;
+  }
+}
+
+// A[r][c] *= dcol[c] over the Q x Q block (Linv -> Linv D)
+__global__ void __launch_bounds__(256) scale_cols_kernel(float* __restrict__ A, int64_t ld, int Q,
+                                                         const float* __restrict__ dcol) {
+  const int64_t total4 = (int64_t)Q * (Q / 4);
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total4; e += (int64_t)gridDim.x * blockDim.x) {
+    const int i = (int)(e / (Q / 4));
+    const int j4 = (int)(e - (int64_t)i * (Q / 4)) * 4;
+    float4* p = reinterpret_cast<float4*>(A + (int64_t)i * ld + j4);
+    const float4 d = *reinterpret_cast<const float4*>(dcol + j4);
+    float4 v = *p;
+    v.x *= d.x; v.y *= d.y; v.z *= d.z; v.w *= d.w;
+    *p = v;
+  }
+}
+
+// partials[blockIdx.x * k + i] = sum of squares of block i of A (rows x cols): the column block [start[i], start[i+1])
+// over all rows (by_cols), or the row block over all columns.  Same fixed-order arithmetic as sumsq_partial_kernel.
+__global__ void __launch_bounds__(256) block_sumsq_partial_kernel(const float* __restrict__ A, int64_t ld, int rows,
+                                                                  int cols, BlockSpec bs, int by_cols,
+                                                                  double* __restrict__ partials) {
+  __shared__ double red[8];
+  for (int b = 0; b < bs.k; ++b) {
+    const int r_lo = by_cols ? 0 : bs.start[b], r_hi = by_cols ? rows : bs.start[b + 1];
+    const int c_lo = by_cols ? bs.start[b] : 0, c4n = ((by_cols ? bs.start[b + 1] : cols) - c_lo) >> 2;
+    double s = 0;
+    for (int r = r_lo + blockIdx.x; r < r_hi; r += gridDim.x) {
+      const float4* row = reinterpret_cast<const float4*>(A + (int64_t)r * ld + c_lo);
+      for (int c0 = threadIdx.x; c0 < c4n; c0 += 4 * blockDim.x) {
+        float f = 0.f;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const int c = c0 + u * blockDim.x;
+          if (c < c4n) {
+            const float4 v = row[c];
+            f = fmaf(v.x, v.x, f); f = fmaf(v.y, v.y, f); f = fmaf(v.z, v.z, f); f = fmaf(v.w, v.w, f);
+          }
+        }
+        s += (double)f;
+      }
+    }
+    s = warp_sum(s);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double t = 0;
+      for (int w = 0; w < 8; ++w) t += red[w];
+      partials[(int64_t)blockIdx.x * bs.k + b] = t;
+    }
+    __syncthreads();
+  }
+}
+
+// blk[2i + slot] = sum over the CTAs of partials[c * k + i], in a fixed order
+__global__ void __launch_bounds__(256) block_reduce_kernel(const double* __restrict__ partials, int nparts, int k,
+                                                           int slot, double* __restrict__ blk) {
+  __shared__ double red[8];
+  for (int b = 0; b < k; ++b) {
+    double s = 0;
+    for (int c = threadIdx.x; c < nparts; c += blockDim.x) s += partials[(int64_t)c * k + b];
+    s = block_sum_256(s, red);
+    if (threadIdx.x == 0) blk[2 * b + slot] = s;
+  }
+}
+
+// vbs (k + 1 entries) of the block form:
+//   vbs[i] = -0.5 ||W_i||^2 / v_i^2 + 0.5 L (Q_i - tr_i B^-1) / v_i,   vbs[k] = -0.5 ||Xb||^2 + 0.5 L (N - Q + tr B^-1) / vn
+__global__ void vbs_blocks_kernel(const double* __restrict__ scal, const double* __restrict__ blk,
+                                  const float* __restrict__ vs, BlockSpec bs, int64_t n_total, int L,
+                                  float* __restrict__ vbs) {
+  const int i = threadIdx.x;
+  const int Q = bs.start[bs.k];
+  if (i < bs.k) {
+    const double v = (double)vs[i];
+    const double Qi = (double)(bs.start[i + 1] - bs.start[i]);
+    vbs[i] = (float)(-0.5 * blk[2 * i + 1] / (v * v) + 0.5 * (double)L * (Qi - blk[2 * i]) / v);
+  } else if (i == bs.k) {
+    vbs[i] = (float)(-0.5 * scal[GPP_S_XB2] +
+                     0.5 * (double)L * ((double)n_total - (double)Q + scal[GPP_S_TRBINV]) / scal[GPP_S_VN]);
+  }
+}
+
+int launch_vbs_blocks(const double* scal, const double* blk, const float* vs, const BlockSpec& bs, int64_t n_total, int L,
+                      float* vbs, cudaStream_t st) {
+  vbs_blocks_kernel<<<1, 32, 0, st>>>(scal, blk, vs, bs, n_total, L, vbs);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
 // ------------------------------------------------------------------ driver
 // The factor workspace doubles as the factorisation *state*: after launch_factor() it holds Lc and
 // Linv, which launch_solve_w() reuses for any number of right-hand sides (train_gppvae.py builds the
@@ -1013,11 +1150,22 @@ static int side_stream(SideStream** out) {
 }
 
 
-int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t flags, float* Binv, double* scal,
-                  void* ws, size_t ws_bytes, cudaStream_t st) {
+// Block form (k designs): the per-column scales and the per-block partial sums follow the single-design state.
+static size_t blocks_off_dcol(int Q) { return align_up(factor_layout(Q).total, 256); }
+static size_t blocks_off_part(int Q) {
+  return blocks_off_dcol(Q) + align_up((size_t)factor_layout(Q).Qp * sizeof(float), 256);
+}
+size_t factor_blocks_workspace_bytes(int Q, int k) {
+  return blocks_off_part(Q) + align_up((size_t)kSumsqBlocks * k * sizeof(double), 256);
+}
+
+// bs == nullptr: the single-design factorisation (scal[V0] = v0); otherwise the block form above, blk[2i] = tr_i B^-1.
+static int factor_impl(const float* G, int64_t ldg, int Q, const float* vs, uint32_t flags, float* Binv, double* scal,
+                       const BlockSpec* bs, double* blk, void* ws, size_t ws_bytes, cudaStream_t st) {
   const FactorLayout f = factor_layout(Q);
-  if (!ws || ws_bytes < f.total) {
-    set_error("factor: workspace too small (%zu < %zu bytes)", ws_bytes, f.total);
+  const size_t need = bs ? factor_blocks_workspace_bytes(Q, bs->k) : f.total;
+  if (!ws || ws_bytes < need) {
+    set_error("factor: workspace too small (%zu < %zu bytes)", ws_bytes, need);
     return GPP_ERR_WORKSPACE;
   }
   char* base = static_cast<char*>(ws);
@@ -1030,12 +1178,20 @@ int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t 
   const int Qp = f.Qp;
   const int nb = Qp / NB;
 
-  scal_init_kernel<<<1, 32, 0, st>>>(vs, scal);
-  GPP_LAUNCH_CHECK();
+  float* dcol = bs ? reinterpret_cast<float*>(base + blocks_off_dcol(Q)) : nullptr;
+  double* bpart = bs ? reinterpret_cast<double*>(base + blocks_off_part(Q)) : nullptr;
   {
     const int64_t total4 = (int64_t)Qp * (Qp / 4);
     int blocks = (int)(ceil_div(total4, 256) < 4096 ? ceil_div(total4, 256) : 4096);
-    build_b_kernel<<<blocks, 256, 0, st>>>(G, ldg, Q, Qp, scal, Bm);
+    if (bs) {
+      blocks_init_kernel<<<(unsigned)ceil_div(Qp, 256), 256, 0, st>>>(vs, *bs, Qp, scal, dcol);
+      GPP_LAUNCH_CHECK();
+      build_b_blocks_kernel<<<blocks, 256, 0, st>>>(G, ldg, Q, Qp, dcol, scal, Bm);
+    } else {
+      scal_init_kernel<<<1, 32, 0, st>>>(vs, scal);
+      GPP_LAUNCH_CHECK();
+      build_b_kernel<<<blocks, 256, 0, st>>>(G, ldg, Q, Qp, scal, Bm);
+    }
     GPP_LAUNCH_CHECK();
   }
   GPP_CUDA(cudaMemsetAsync(Linv, 0, (size_t)Qp * Qp * sizeof(float), st));
@@ -1205,7 +1361,17 @@ int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t 
     }
   }
 
-  if (flags & GPP_WANT_BINV) {  // Binv = Linv^T Linv
+  if (bs) {   // tr_i B^-1 from the unscaled Linv, then Linv <- Linv D
+    block_sumsq_partial_kernel<<<kSumsqBlocks, 256, 0, st>>>(Linv, Qp, Q, Q, *bs, 1, bpart);
+    GPP_LAUNCH_CHECK();
+    block_reduce_kernel<<<1, 256, 0, st>>>(bpart, kSumsqBlocks, bs->k, 0, blk);
+    GPP_LAUNCH_CHECK();
+    const int64_t total4 = (int64_t)Q * (Q / 4);
+    scale_cols_kernel<<<(unsigned)(ceil_div(total4, 256) < 4096 ? ceil_div(total4, 256) : 4096), 256, 0, st>>>(Linv, Qp, Q,
+                                                                                                              dcol);
+    GPP_LAUNCH_CHECK();
+  }
+  if (flags & GPP_WANT_BINV) {  // Binv = Linv^T Linv  (block form: D B^-1 D)
     if (!Binv) {
       set_error("factor: GPP_WANT_BINV set but Binv is null");
       return GPP_ERR_INVALID_ARGUMENT;
@@ -1215,11 +1381,26 @@ int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t 
     else
       GPP_TRY(launch_tn(Linv, Qp, Q, Linv, Qp, Q, nullptr, 0, 0, Q, 1, Binv, Q, nullptr, 0, nullptr, tnws, f.tn_bytes, st));
   }
+  if (bs) {   // tr B^-1 = the sum of the per-block partials
+    factor_scalars_kernel<<<1, 256, 0, st>>>(Bm, Qp, Q, bpart, kSumsqBlocks * bs->k, scal);
+    GPP_LAUNCH_CHECK();
+    return GPP_OK;
+  }
   sumsq_partial_kernel<<<kSumsqBlocks, 256, 0, st>>>(Linv, Qp, Q, Q, part);
   GPP_LAUNCH_CHECK();
   factor_scalars_kernel<<<1, 256, 0, st>>>(Bm, Qp, Q, part, kSumsqBlocks, scal);
   GPP_LAUNCH_CHECK();
   return GPP_OK;
+}
+
+int launch_factor(const float* G, int64_t ldg, int Q, const float* vs, uint32_t flags, float* Binv, double* scal,
+                  void* ws, size_t ws_bytes, cudaStream_t st) {
+  return factor_impl(G, ldg, Q, vs, flags, Binv, scal, nullptr, nullptr, ws, ws_bytes, st);
+}
+
+int launch_factor_blocks(const float* G, int64_t ldg, const BlockSpec& bs, const float* vs, uint32_t flags, float* Binv,
+                         double* scal, double* blk, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return factor_impl(G, ldg, bs.start[bs.k], vs, flags, Binv, scal, &bs, blk, ws, ws_bytes, st);
 }
 
 // W = (v0/vn) Linv^T (Linv C) for C (Q x L); `state` is the workspace launch_factor filled for the same Q.
@@ -1274,6 +1455,35 @@ int launch_solve_w(const float* C, int64_t ldc, int Q, int L, int L_true, int64_
   sumsq_partial_kernel<<<kSumsqBlocks, 256, 0, st>>>(W, ldw, Q, L, part);
   GPP_LAUNCH_CHECK();
   solve_scalars_kernel<<<1, 256, 0, st>>>(L_true, n_total, part, kSumsqBlocks, scal);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+size_t solve_blocks_workspace_bytes(int Q, int L, int k) {
+  return align_up(solve_layout(Q, L).total, 256) + align_up((size_t)kSumsqBlocks * k * sizeof(double), 256);
+}
+
+// The state of launch_factor_blocks holds Linv D, so the single-design solve yields W = D B^-1 D C / vn; then
+// blk[2i + 1] = ||W_i||^2 over row block i.
+int launch_solve_w_blocks(const float* C, int64_t ldc, const BlockSpec& bs, int L, int L_true, int64_t n_total, float* W,
+                          int64_t ldw, double* scal, double* blk, const void* state, size_t state_bytes, void* ws,
+                          size_t ws_bytes, cudaStream_t st) {
+  const int Q = bs.start[bs.k];
+  if (!state || state_bytes < factor_blocks_workspace_bytes(Q, bs.k)) {
+    set_error("solve_w_blocks: factorisation state too small (%zu < %zu bytes)", state_bytes,
+              factor_blocks_workspace_bytes(Q, bs.k));
+    return GPP_ERR_WORKSPACE;
+  }
+  if (!ws || ws_bytes < solve_blocks_workspace_bytes(Q, L, bs.k)) {
+    set_error("solve_w_blocks: workspace too small (%zu < %zu bytes)", ws_bytes, solve_blocks_workspace_bytes(Q, L, bs.k));
+    return GPP_ERR_WORKSPACE;
+  }
+  const size_t off = align_up(solve_layout(Q, L).total, 256);
+  GPP_TRY(launch_solve_w(C, ldc, Q, L, L_true, n_total, W, ldw, scal, state, state_bytes, ws, off, st));
+  double* bpart = reinterpret_cast<double*>(static_cast<char*>(ws) + off);
+  block_sumsq_partial_kernel<<<kSumsqBlocks, 256, 0, st>>>(W, ldw, Q, L, bs, 0, bpart);
+  GPP_LAUNCH_CHECK();
+  block_reduce_kernel<<<1, 256, 0, st>>>(bpart, kSumsqBlocks, bs.k, 1, blk);
   GPP_LAUNCH_CHECK();
   return GPP_OK;
 }

@@ -7,6 +7,7 @@
 namespace gpp {
 
 constexpr int kTeWarps = 8;
+constexpr int kMaxDesigns = GPP_MAX_DESIGNS;
 
 __device__ __forceinline__ float row_dot(const float* __restrict__ a, const float* __restrict__ b, int len, int lane) {
   float s = 0.f;
@@ -89,6 +90,92 @@ taylor_bwd_lvs_kernel(const float* __restrict__ gout, int64_t n, const float* __
   }
 }
 
+// ---- k designs (gp.py:127-133 summed over the designs, gp.py:130-131), k + 1 variances: one launch each whatever k is
+struct TeTable {
+  int k;
+  const float* V[kMaxDesigns];
+  const float* Vb[kMaxDesigns];
+  float* gV[kMaxDesigns];
+  int64_t ldv[kMaxDesigns], ldvb[kMaxDesigns], ldgv[kMaxDesigns];
+  int Q[kMaxDesigns];
+};
+
+// softmax(lvs[0..m)) (gp.py:48-50) in double, without a per-thread array: vs_b = exp(lvs_b - mx) / s.
+// Returns <vbs, vs>.
+__device__ __forceinline__ double softmax_dot(const float* __restrict__ lvs, const float* __restrict__ vbs, int m,
+                                              double& mx, double& s) {
+  mx = (double)lvs[0];
+  for (int b = 1; b < m; ++b) mx = fmax(mx, (double)lvs[b]);
+  s = 0;
+  double d = 0;
+  for (int b = 0; b < m; ++b) {
+    const double e = exp((double)lvs[b] - mx);
+    s += e;
+    d += (double)vbs[b] * e;
+  }
+  return d / s;
+}
+
+__global__ void __launch_bounds__(kTeWarps * 32)
+taylor_fwd_multi_kernel(const float* __restrict__ X, int64_t ldx, const float* __restrict__ Xb, int64_t ldxb, TeTable t,
+                        int64_t n, int L, const float* __restrict__ vbs, const float* __restrict__ lvs,
+                        float* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * kTeWarps + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * kTeWarps;
+  double mx, se;
+  const float cterm = (float)(softmax_dot(lvs, vbs, t.k + 1, mx, se) / (double)n);
+  for (int64_t r = warp; r < n; r += nwarps) {
+    float s = row_dot(Xb + r * ldxb, X + r * ldx, L, lane);
+    for (int j = 0; j < t.k; ++j) s += row_dot(t.Vb[j] + r * t.ldvb[j], t.V[j] + r * t.ldv[j], t.Q[j], lane);
+    s = warp_sum(s);
+    if (lane == 0) out[r] = s + cterm;
+  }
+}
+
+__global__ void __launch_bounds__(kTeWarps * 32)
+taylor_bwd_multi_rows_kernel(const float* __restrict__ gout, const float* __restrict__ Xb, int64_t ldxb, TeTable t,
+                             int64_t n, int L, float* __restrict__ gX, int64_t ldgx) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * kTeWarps + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * kTeWarps;
+  auto scale_row = [&](const float* src, float* dst, int len, float g) {
+    const float4* s4 = reinterpret_cast<const float4*>(src);
+    float4* d4 = reinterpret_cast<float4*>(dst);
+    for (int c = lane; c < (len >> 2); c += 32) {
+      const float4 v = s4[c];
+      d4[c] = make_float4(g * v.x, g * v.y, g * v.z, g * v.w);
+    }
+  };
+  for (int64_t r = warp; r < n; r += nwarps) {
+    const float g = gout[r];
+    if (gX) scale_row(Xb + r * ldxb, gX + r * ldgx, L, g);
+    for (int j = 0; j < t.k; ++j)
+      if (t.gV[j]) scale_row(t.Vb[j] + r * t.ldvb[j], t.gV[j] + r * t.ldgv[j], t.Q[j], g);
+  }
+}
+
+// glvs_b = (sum g / n) * vs_b * (vbs_b - <vbs, vs>),  b = 0..m-1
+__global__ void __launch_bounds__(256)
+taylor_bwd_multi_lvs_kernel(const float* __restrict__ gout, int64_t n, int m, const float* __restrict__ vbs,
+                            const float* __restrict__ lvs, float* __restrict__ glvs) {
+  __shared__ double red[8];
+  double s = 0;
+  for (int64_t i = threadIdx.x; i < n; i += blockDim.x) s += (double)gout[i];
+  s = warp_sum(s);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0;
+    for (int w = 0; w < 8; ++w) t += red[w];
+    double mx, se;
+    const double mean = softmax_dot(lvs, vbs, m, mx, se);
+    const double scale = t / (double)n;
+    for (int b = 0; b < m; ++b)
+      glvs[b] = (float)(scale * (exp((double)lvs[b] - mx) / se) * ((double)vbs[b] - mean));
+  }
+}
+
 static int rows_grid(int64_t n) {
   const int64_t want = ceil_div(n, kTeWarps);
   const int64_t cap = (int64_t)sm_count() * 8;
@@ -129,6 +216,76 @@ extern "C" int gpp_taylor_expansion_bwd(const float* gout, const float* Xb, int6
   }
   if (glvs) {
     taylor_bwd_lvs_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(gout, n, vbs, lvs, glvs);
+    GPP_LAUNCH_CHECK();
+  }
+  return GPP_OK;
+}
+
+// Fill the pointer table of the k-design entries from the caller's host arrays.
+static int te_table(const char* who, int32_t k, const float* const* V, const int64_t* ldv, const float* const* Vb,
+                    const int64_t* ldvb, float* const* gV, const int64_t* ldgv, const int32_t* Q, TeTable& t) {
+  GPP_REQUIRE(k >= 1 && k <= kMaxDesigns, "%s: k = %d designs (1..%d supported)", who, k, kMaxDesigns);
+  GPP_REQUIRE(Vb && ldvb && Q, "%s: null host array", who);
+  t = TeTable{};
+  t.k = k;
+  for (int j = 0; j < k; ++j) {
+    GPP_REQUIRE(Q[j] > 0 && Q[j] % 4 == 0, "%s: design %d has %d columns (a positive multiple of 4 is required)", who, j,
+                Q[j]);
+    GPP_REQUIRE(Vb[j] && aligned16(Vb[j]) && ldvb[j] >= Q[j] && ldvb[j] % 4 == 0, "%s: bad Vb of design %d", who, j);
+    t.Vb[j] = Vb[j];
+    t.ldvb[j] = ldvb[j];
+    t.Q[j] = Q[j];
+    if (V) {
+      GPP_REQUIRE(ldv && V[j] && aligned16(V[j]) && ldv[j] >= Q[j] && ldv[j] % 4 == 0, "%s: bad V of design %d", who, j);
+      t.V[j] = V[j];
+      t.ldv[j] = ldv[j];
+    }
+    if (gV && gV[j]) {
+      GPP_REQUIRE(ldgv && aligned16(gV[j]) && ldgv[j] >= Q[j] && ldgv[j] % 4 == 0, "%s: bad gV of design %d", who, j);
+      t.gV[j] = gV[j];
+      t.ldgv[j] = ldgv[j];
+    }
+  }
+  return GPP_OK;
+}
+
+extern "C" int gpp_taylor_expansion_fwd_multi(const float* X, int64_t ldx, const float* Xb, int64_t ldxb, int32_t k,
+                                              const float* const* V_host, const int64_t* ldv_host,
+                                              const float* const* Vb_host, const int64_t* ldvb_host, const int32_t* Q_host,
+                                              int64_t n, int32_t L, const float* vbs, const float* lvs, float* out,
+                                              gpp_stream_t stream) {
+  GPP_REQUIRE(X && Xb && vbs && lvs && out && V_host, "taylor_expansion_fwd_multi: null pointer");
+  GPP_REQUIRE(n > 0 && L > 0 && L % 4 == 0, "taylor_expansion_fwd_multi: bad shape");
+  GPP_REQUIRE(ldx >= L && ldxb >= L && ldx % 4 == 0 && ldxb % 4 == 0 && aligned16(X) && aligned16(Xb),
+              "taylor_expansion_fwd_multi: bad X / Xb");
+  TeTable t;
+  GPP_TRY(te_table("taylor_expansion_fwd_multi", k, V_host, ldv_host, Vb_host, ldvb_host, nullptr, nullptr, Q_host, t));
+  taylor_fwd_multi_kernel<<<rows_grid(n), kTeWarps * 32, 0, (cudaStream_t)stream>>>(X, ldx, Xb, ldxb, t, n, L, vbs, lvs,
+                                                                                    out);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_taylor_expansion_bwd_multi(const float* gout, const float* Xb, int64_t ldxb, int32_t k,
+                                              const float* const* Vb_host, const int64_t* ldvb_host, const int32_t* Q_host,
+                                              int64_t n, int32_t L, const float* vbs, const float* lvs, float* gX,
+                                              int64_t ldgx, float* const* gV_host, const int64_t* ldgv_host, float* glvs,
+                                              gpp_stream_t stream) {
+  GPP_REQUIRE(gout && vbs && lvs, "taylor_expansion_bwd_multi: null pointer");
+  GPP_REQUIRE(n > 0 && L > 0 && L % 4 == 0, "taylor_expansion_bwd_multi: bad shape");
+  GPP_REQUIRE(!gX || (Xb && aligned16(Xb) && aligned16(gX) && ldxb >= L && ldgx >= L && ldxb % 4 == 0 && ldgx % 4 == 0),
+              "taylor_expansion_bwd_multi: bad gX / Xb");
+  TeTable t;
+  GPP_TRY(te_table("taylor_expansion_bwd_multi", k, nullptr, nullptr, Vb_host, ldvb_host, gV_host, ldgv_host, Q_host, t));
+  bool any_gv = false;
+  for (int j = 0; j < k; ++j) any_gv = any_gv || t.gV[j] != nullptr;
+  if (gX || any_gv) {
+    taylor_bwd_multi_rows_kernel<<<rows_grid(n), kTeWarps * 32, 0, (cudaStream_t)stream>>>(gout, Xb, ldxb, t, n, L, gX,
+                                                                                           ldgx);
+    GPP_LAUNCH_CHECK();
+  }
+  if (glvs) {
+    taylor_bwd_multi_lvs_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(gout, n, k + 1, vbs, lvs, glvs);
     GPP_LAUNCH_CHECK();
   }
   return GPP_OK;

@@ -25,7 +25,7 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from ._lib import S_QUAD, S_XB2
+from ._lib import GPP_MAX_DESIGNS, S_QUAD, S_XB2
 from .vmod import KhatriRao
 
 
@@ -53,6 +53,33 @@ class LowRankFactor:
         zeros = torch.zeros(self.n, self.Q, device=self.V.device, dtype=torch.float32)
         VB = ops.x_minus_am(zeros, self.Q, self.V, self.ldv, self.fac.Binv, self.Q, self.n, self.Q, self.Q, -1.0)
         return r * VB[:, : self.Qtrue]
+
+
+class BlocksFactor(LowRankFactor):
+    """`U` / `UBi` of `GP.U_UBi_Shb` for k >= 2 designs: carries the designs, their stacked operand (ops.Stacked) and the
+    block-form factorisation (Binv = D B^-1 D, D = diag(sqrt(v_i)) on block i)."""
+
+    def __init__(self, kind: str, Vs, stk: ops.Stacked, vs: torch.Tensor, fac: ops.Factorisation):
+        self.kind, self.Vs, self.stk, self.vs, self.fac = kind, list(Vs), stk, vs, fac
+        self.Q = stk.Q
+        self.n = stk.n
+        self.shape = torch.Size((self.n, sum(stk.true_widths)))
+
+    def dense(self) -> torch.Tensor:
+        """The reference's U = [sqrt(v_i) V_i] / sqrt(vn) (gp.py:27-28) or UBi = U B^-1 (gp.py:35-36)."""
+        vs = self.vs.detach()
+        sq = torch.sqrt(vs[:-1] / vs[-1])
+        if self.kind == "U":
+            return torch.cat([sq[i] * V.detach() for i, V in enumerate(self.Vs)], 1)
+        if self.fac.Binv is None:
+            raise RuntimeError("UBi.dense() needs B^-1: call GP.U_UBi_Shb(Vs, vs, want_binv=True)")
+        Vc = torch.zeros(self.n, self.Q, device=vs.device, dtype=torch.float32)
+        for o, V in zip(self.stk.offsets, self.Vs):
+            Vc[:, o:o + V.shape[1]] = V.detach()
+        # V (D B^-1 D) D^-1 / sqrt(vn) = U B^-1 on the true columns
+        VB = ops.x_minus_am(torch.zeros_like(Vc), self.Q, Vc, self.Q, self.fac.Binv, self.Q, self.n, self.Q, self.Q, -1.0)
+        return torch.cat([VB[:, o:o + V.shape[1]] / torch.sqrt(vs[i] * vs[-1])
+                          for i, (o, V) in enumerate(zip(self.stk.offsets, self.Vs))], 1)
 
 
 class KhatriRaoFactor:
@@ -106,13 +133,20 @@ class LazySingularValues:
     """`Shb` of gp.py:33 (singular values of B, descending).  The trainer discards it
     (train_gppvae.py:235), so it is only computed if somebody asks -- off the hot path, from G."""
 
-    def __init__(self, G: torch.Tensor, Qtrue: int, vs: torch.Tensor):
-        self._G, self._Q, self._vs, self._val = G, Qtrue, vs, None
+    def __init__(self, G: torch.Tensor, Qtrue: int, vs: torch.Tensor, stk: Optional[ops.Stacked] = None):
+        self._G, self._Q, self._vs, self._stk, self._val = G, Qtrue, vs, stk, None
 
     def value(self) -> torch.Tensor:
         if self._val is None:
             vs = self._vs.detach()
-            B = torch.eye(self._Q, device=self._G.device) + (vs[0] / vs[-1]) * self._G[: self._Q, : self._Q]
+            if self._stk is not None:   # k designs: B = I + D G D / vn on the true columns of every block
+                stk = self._stk
+                cols = torch.cat([torch.arange(o, o + t) for o, t in zip(stk.offsets, stk.true_widths)]).to(self._G.device)
+                d = torch.cat([torch.sqrt(vs[i]).expand(t) for i, t in enumerate(stk.true_widths)])
+                G = self._G[:, : stk.Q][cols][:, cols]
+                B = torch.eye(cols.numel(), device=G.device) + (d[:, None] * d[None, :] / vs[-1]) * G
+            else:
+                B = torch.eye(self._Q, device=self._G.device) + (vs[0] / vs[-1]) * self._G[: self._Q, : self._Q]
             self._val = torch.linalg.eigvalsh(B.double()).flip(0).to(torch.float32)
         return self._val
 
@@ -166,9 +200,8 @@ class GP(nn.Module):
         if not vsum2one:
             # the reference's other branch is broken (gp.py:52 uses an undefined name)
             raise NotImplementedError("vsum2one=False is not implemented (it raises NameError in the reference too)")
-        if n_rand_effs != 1:
-            # the reference trainer only ever builds GP(n_rand_effs=1) (train_gppvae.py:138)
-            raise NotImplementedError("only one random-effect design (n_rand_effs=1) is implemented")
+        if int(n_rand_effs) != n_rand_effs or not 1 <= n_rand_effs <= GPP_MAX_DESIGNS:
+            raise ValueError(f"n_rand_effs must be an integer in 1..{GPP_MAX_DESIGNS} (got {n_rand_effs})")
         self.n_rand_effs = n_rand_effs
         self.vsum2one = vsum2one
         self.lvs = nn.Parameter(torch.zeros([n_rand_effs + 1]))      # gp.py:21-22
@@ -199,6 +232,7 @@ class GP(nn.Module):
         see (`V.data[...] = ...`); in-place tensor operations and optimiser steps are detected."""
         self._cache.clear()
         ops.PLANES.invalidate()
+        ops.STACKED.invalidate()
 
     def _all_reduce(self, t: torch.Tensor, async_op: bool = False):
         """SUM over the row shards.  `async_op=True` returns the collective's work handle (None when not sharded): the
@@ -246,22 +280,52 @@ class GP(nn.Module):
         Vm, ldv = ops.as_matrix(Vs[0], "V")
         return Vm, ldv, Vm.shape[1], Vs[0].shape[1]
 
-    def _factorise(self, Vm, ldv, Q, vs, want_binv: bool, Xm=None, ldx=0, Lk=0, vs_origin=None):
+    def _stack(self, Vs: Sequence[torch.Tensor], Lk: int) -> ops.Stacked:
+        """k >= 2 designs: check them and return their stacked operand (planes at tensor-core shapes)."""
+        k = self.n_rand_effs
+        if len(Vs) != k:
+            raise ValueError(f"GP(n_rand_effs={k}) expects {k} design matrices in Vs, got {len(Vs)}")
+        if any(isinstance(V, KhatriRao) for V in Vs):
+            raise NotImplementedError("the structured route (vmod.KhatriRao) takes a single design; with n_rand_effs > 1 "
+                                      "pass the dense Khatri-Rao matrix (KhatriRao.dense()) instead")
+        n, Q = Vs[0].shape[0], sum(ops.round4(V.shape[1]) for V in Vs)
+        use_planes = ops.planes_supported(n, Q, Lk)
+
+        def before_build():   # new stacked planes are about to be built: a cache entry on the previous ones lets them go
+            if isinstance(self._cache.token, ops.Stacked):
+                self._cache.clear()
+        return ops.stacked(Vs, use_planes, before_build)
+
+    def _factor(self, G, ldg, Q, vs, want_binv, stk):
+        if stk is None:
+            return ops.factor(G, ldg, Q, vs, want_binv)
+        return ops.factor_blocks(G, ldg, stk.widths, vs, want_binv)
+
+    def _factorise(self, Vm, ldv, Q, vs, want_binv: bool, Xm=None, ldx=0, Lk=0, vs_origin=None, stk=None):
         """Pass 1 (+ all-reduce) and the factorisation, through the cache.
         Returns (fac, C, pV) with C = V^T X (Q x Lk, summed over ranks) or None when no X was given, and pV the operand
-        planes of V (None for shapes below the tensor-core tile, which run on the fp32 engine)."""
-        n = Vm.shape[0]
+        planes of V (None for shapes below the tensor-core tile, which run on the fp32 engine).  With `stk` (k >= 2
+        designs) V is the stacked operand and the factorisation is the block form."""
         tok, keep_vs = self._vs_token(vs if vs_origin is None else vs_origin)
-        key = (Vm.untyped_storage().data_ptr(), Vm.storage_offset(), Vm._version, n, Q, ldv, tok)
-        use_planes = ops.planes_supported(n, Q, Lk)
-        pV = ops.planes_of(Vm, ldv) if use_planes else None
+        if stk is None:
+            n = Vm.shape[0]
+            key = (Vm.untyped_storage().data_ptr(), Vm.storage_offset(), Vm._version, n, Q, ldv, tok)
+            use_planes = ops.planes_supported(n, Q, Lk)
+            pV = ops.planes_of(Vm, ldv) if use_planes else None
+            token, keep_v = pV, (None if use_planes else Vm)
+        else:
+            n = stk.n
+            key = ("blocks", stk.key, tok)
+            use_planes = stk.planes is not None
+            pV = stk.planes
+            token, keep_v = stk, None          # the stacked operand (held by the entry's token) pins what it needs
 
         def vtx():
             if use_planes:
                 return ops.atb_planes(pV, ops.split_planes(Xm, ldx, n, Lk), n, Q, Lk)
             return ops.atb(Vm, ldv, Xm, ldx, n, Q, Lk)
 
-        fac = self._cache.lookup(key, want_binv, vs, token=pV)
+        fac = self._cache.lookup(key, want_binv, vs, token=token)
         if fac is not None:
             self.cache_hits += 1
             C = None
@@ -281,10 +345,10 @@ class GP(nn.Module):
             hC = self._all_reduce(C, async_op=True)
             hG.wait()
             self._stage("allreduce:end")
-            fac = ops.factor(G, Q, Q, vs, want_binv)
+            fac = self._factor(G, Q, Q, vs, want_binv, stk)
             hC.wait()
             self._stage("factor:end")
-            self._cache.store(key, (None if use_planes else Vm, keep_vs), G, Q, fac, vs, token=pV)
+            self._cache.store(key, (keep_v, keep_vs), G, Q, fac, vs, token=token)
             self._cache.C = C
             return fac, C, pV
         pX = ops.split_planes(Xm, ldx, n, Lk) if (use_planes and Lk) else None
@@ -293,10 +357,10 @@ class GP(nn.Module):
         self._stage("pass1:end")
         self._all_reduce(GC)
         self._stage("allreduce:end")
-        fac = ops.factor(GC, Q + Lk, Q, vs, want_binv)
+        fac = self._factor(GC, Q + Lk, Q, vs, want_binv, stk)
         self._stage("factor:end")
         # with planes the registry entry pins V (see _FactorCache); without, the cache entry does
-        self._cache.store(key, (None if use_planes else Vm, keep_vs), GC, Q + Lk, fac, vs, token=pV)
+        self._cache.store(key, (keep_v, keep_vs), GC, Q + Lk, fac, vs, token=token)
         self._cache.C = GC[:, Q:] if Lk else None
         return fac, (GC[:, Q:] if Lk else None), pV
 
@@ -349,11 +413,16 @@ class GP(nn.Module):
 
     def U_UBi_Shb(self, Vs: Sequence[torch.Tensor], vs: torch.Tensor, want_binv: bool = False):
         """gp.py:24-38.  Returns handles (see LowRankFactor) that `solve` accepts."""
-        if len(Vs) == 1 and isinstance(Vs[0], KhatriRao):
+        if self.n_rand_effs == 1 and len(Vs) == 1 and isinstance(Vs[0], KhatriRao):
             kr = Vs[0]
             fac, _ = self._kr_factorise(kr, vs, want_binv)
             return (KhatriRaoFactor("U", kr, vs, fac), KhatriRaoFactor("UBi", kr, vs, fac),
                     LazySingularValues(self._cache.G, kr.p * kr.q, vs))
+        if self.n_rand_effs > 1:
+            stk = self._stack(Vs, 0)
+            fac, _, _ = self._factorise(stk.V, stk.Q, stk.Q, vs, want_binv, stk=stk)
+            return (BlocksFactor("U", Vs, stk, vs, fac), BlocksFactor("UBi", Vs, stk, vs, fac),
+                    LazySingularValues(self._cache.G, stk.Q, vs, stk=stk))
         Vm, ldv, Q, Qtrue = self._cat(Vs, vs)
         fac, _, _ = self._factorise(Vm, ldv, Q, vs, want_binv)
         U = LowRankFactor("U", Vm, ldv, Q, Qtrue, vs, fac)
@@ -370,6 +439,21 @@ class GP(nn.Module):
                 raise ValueError(f"X has {n} rows but the factorisation was built for {U.n}")
             C = self._kr_c(U.kr, Xm, ldx, Lk)
             _, _, Xb, _ = self._kr_solve(U.kr, U.fac, C, Xm, ldx, Lk, L, self._n_total(n, X.device))
+        elif isinstance(U, BlocksFactor):
+            if n != U.n:
+                raise ValueError(f"X has {n} rows but the factorisation was built for {U.n}")
+            # the stacked operand in the form this X needs (the factorisation holds for the same designs either way)
+            stk = U.stk if (U.stk.planes is not None) == ops.planes_supported(n, U.Q, Lk) else self._stack(U.Vs, Lk)
+            if stk.planes is not None:
+                C = ops.atb_planes(stk.planes, ops.split_planes(Xm, ldx, n, Lk), n, U.Q, Lk)
+            else:
+                C = ops.atb(stk.V, U.Q, Xm, ldx, n, U.Q, Lk)
+            self._all_reduce(C)
+            W, scal = ops.solve_w(U.fac, C, Lk, Lk, L, self._n_total(n, X.device))
+            if stk.planes is not None:
+                Xb, _ = ops.xb_nll_planes(stk.planes, Xm, ldx, W, n, U.Q, Lk, scal)
+            else:
+                Xb, _ = ops.xb_nll(stk.V, U.Q, Xm, ldx, W, n, U.Q, Lk, scal)
         elif isinstance(U, LowRankFactor):
             if n != U.n:
                 raise ValueError(f"X has {n} rows but the factorisation was built for {U.n}")
@@ -398,7 +482,7 @@ class GP(nn.Module):
         """Shared body of taylor_coeff and nll: returns a dict of everything computed."""
         vs_attached = self.get_vs()
         vs = vs_attached.detach()
-        if len(Vs) == 1 and isinstance(Vs[0], KhatriRao):
+        if self.n_rand_effs == 1 and len(Vs) == 1 and isinstance(Vs[0], KhatriRao):
             kr = Vs[0]
             Xm, ldx = ops.as_matrix(X, "X")
             n, L = X.shape
@@ -412,6 +496,28 @@ class GP(nn.Module):
             W, scal, Xb, nll = self._kr_solve(kr, fac, C, Xm, ldx, Lk, L, n_total)
             return dict(vs=vs, Vm=None, kr=kr, ldv=0, Q=kr.p * kr.q, Qtrue=kr.p_true * kr.q, n=n, L=L, Lk=Lk,
                         n_total=n_total, fac=fac, W=W, scal=scal, Xb=Xb, nll=nll)
+        if self.n_rand_effs > 1:
+            Xm, ldx = ops.as_matrix(X, "X")
+            n, L = X.shape
+            Lk = Xm.shape[1]
+            if any(V.shape[0] != n for V in Vs if torch.is_tensor(V)):
+                raise ValueError(f"X has {n} rows but the designs have {[V.shape[0] for V in Vs]}")
+            self._stage("stack:start")
+            stk = self._stack(Vs, Lk)
+            self._stage("stack:end")
+            if (stk.planes.buf if stk.planes is not None else stk.V).device != Xm.device:
+                raise ValueError("X and V must be on the same device")
+            n_total = self._n_total(n, X.device)
+            fac, C, pV = self._factorise(stk.V, stk.Q, stk.Q, vs, want_vb, Xm, ldx, Lk, vs_origin=vs_attached, stk=stk)
+            W, scal, blk = ops.solve_w_blocks(fac, C, C.stride(0), Lk, L, n_total)
+            self._stage("solve:end")
+            if pV is not None:
+                Xb, nll = ops.xb_nll_planes(pV, Xm, ldx, W, n, stk.Q, Lk, scal)
+            else:
+                Xb, nll = ops.xb_nll(stk.V, stk.Q, Xm, ldx, W, n, stk.Q, Lk, scal)
+            self._stage("pass2:end")
+            return dict(vs=vs, Vm=stk.V, ldv=stk.Q, Q=stk.Q, Qtrue=stk.Q, n=n, L=L, Lk=Lk, n_total=n_total, fac=fac,
+                        W=W, scal=scal, Xb=Xb, nll=nll, pV=pV, stk=stk, blk=blk)
         Vm, ldv, Q, Qtrue = self._cat(Vs, vs)
         Xm, ldx = ops.as_matrix(X, "X")
         n, L = X.shape
@@ -442,8 +548,22 @@ class GP(nn.Module):
         scal, Q, L, Lk = c["scal"], c["Q"], c["L"], c["Lk"]
         if self._sharded:
             self._all_reduce(scal[S_XB2:S_QUAD + 1])
-        vbs = ops.vbs_from_scal(scal, c["n_total"], Q, L)
-        if need_vb and c["Vm"] is None:
+        stk = c.get("stk")
+        if stk is not None:
+            vbs = ops.vbs_blocks(scal, c["blk"], c["vs"], stk.widths, c["n_total"], L)
+        else:
+            vbs = ops.vbs_from_scal(scal, c["n_total"], Q, L)
+        if need_vb and stk is not None:
+            # one N x Q matrix; Vb_i is the view of block i at design i's true width
+            if c["pV"] is not None:
+                Vb = ops.vb_planes(c["pV"], c["Xb"], c["fac"].Binv, c["W"], scal, c["n"], Q, Lk, L)
+            else:
+                Vb = ops.vb(stk.V, Q, c["Xb"], c["fac"].Binv, c["W"], scal, c["n"], Q, Lk, L)
+            Vbs = [Vb[:, o:o + t] for o, t in zip(stk.offsets, stk.true_widths)]
+            self._stage("vb:end")
+        elif stk is not None:
+            Vbs = [None] * len(stk.widths)
+        elif need_vb and c["Vm"] is None:
             Vbs = [LazyVb(c["kr"], c["Xb"], c["fac"], c["W"], scal, Q, Lk, L)]
         elif need_vb:
             if c.get("pV") is not None:
@@ -475,6 +595,14 @@ class GP(nn.Module):
     def taylor_expansion(self, X: torch.Tensor, Vs: Sequence[torch.Tensor], Xb: torch.Tensor,
                          Vbs: Sequence[torch.Tensor], vbs: torch.Tensor) -> torch.Tensor:
         """gp.py:127-133: (n x 1) surrogate with gradients to X, each V and lvs."""
+        if self.n_rand_effs > 1:
+            k = self.n_rand_effs
+            if len(Vs) != k or len(Vbs) != k:
+                raise ValueError(f"GP(n_rand_effs={k}) expects {k} designs in Vs and Vbs, got {len(Vs)} / {len(Vbs)}")
+            if any(isinstance(V, KhatriRao) for V in Vs):
+                raise NotImplementedError("the structured route (vmod.KhatriRao) takes a single design; with "
+                                          "n_rand_effs > 1 pass the dense Khatri-Rao matrix instead")
+            return ops._TaylorExpansionMulti.apply(X, self.lvs, Xb, vbs, *Vs, *Vbs)
         if len(Vs) != 1 or len(Vbs) != 1:
             raise NotImplementedError(f"expected one design matrix in Vs / Vbs, got {len(Vs)} / {len(Vbs)}")
         return ops._TaylorExpansion.apply(X, Vs[0], self.lvs, Xb, Vbs[0], vbs)

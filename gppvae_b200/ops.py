@@ -10,6 +10,7 @@ from typing import Optional, Tuple
 import torch
 
 import collections
+import weakref
 
 from . import _lib
 from ._lib import GPP_PLANES_COLSQ, GPP_PLANES_UNIT_BOUND, GPP_WANT_BINV, NSCAL, check
@@ -200,6 +201,104 @@ def planes_of(V: torch.Tensor, ldv: int) -> Planes:
     return pl
 
 
+class Stacked:
+    """k designs of one evaluation as ONE n x Q operand V = [V_0 | ... | V_{k-1}] (gp.py:27 without the sqrt(v_i)
+    weights, which the block-form factorisation applies): the operand planes of V at tensor-core shapes (`planes`,
+    written from the k fp32 designs without an fp32 copy of V), else a zero-padded fp32 concatenation (`V`).
+    Block i occupies columns [offsets[i], offsets[i] + widths[i]); its first true_widths[i] are design i's columns."""
+
+    def __init__(self, key, n: int, widths, true_widths, planes: Optional[Planes], V: Optional[torch.Tensor]):
+        self.key, self.n, self.widths, self.true_widths, self.planes, self.V = key, n, list(widths), list(true_widths), \
+            planes, V
+        self.offsets = [sum(self.widths[:i]) for i in range(len(self.widths))]
+        self.Q = sum(self.widths)
+
+
+class _StackedRegistry:
+    """The stacked operand of the designs used last (one entry), found again by the designs' storage, layout and version.
+
+    The entry refers to the designs through weak references only and is dropped when the first of them dies, so it
+    never keeps a design alive, and its planes (4 bytes per element of V) go with last epoch's designs instead of
+    staying resident next to the new ones."""
+
+    def __init__(self):
+        self.entry: Optional[Stacked] = None
+        self._refs = ()
+
+    @staticmethod
+    def key(Vs, mats, use_planes: bool):
+        return (use_planes,) + tuple((V.device.index, V.untyped_storage().data_ptr(), V.storage_offset(), tuple(V.shape),
+                                      tuple(V.stride()), V._version, ld) for V, (_, ld) in zip(Vs, mats))
+
+    def get(self, key) -> Optional[Stacked]:
+        e = self.entry
+        return e if e is not None and e.key == key else None
+
+    def put(self, Vs, st: Stacked) -> None:
+        def drop(_ref, st=st):
+            if self.entry is st:
+                self.invalidate()
+        self.entry = st
+        self._refs = tuple(weakref.ref(V, drop) for V in Vs)
+
+    def invalidate(self) -> None:
+        self.entry = None
+        self._refs = ()
+
+
+STACKED = _StackedRegistry()
+
+
+def stacked(Vs, use_planes: bool, before_build=None) -> Stacked:
+    """The Stacked operand of the designs Vs (CUDA float32 n x Q_i each, same n): from the registry, or built now (the
+    previous entry is dropped first, and `before_build()` is called, so that the caller can release what it holds of
+    the previous one: two sets of stacked planes need never coexist)."""
+    mats = [as_matrix(V, f"Vs[{i}]") for i, V in enumerate(Vs)]
+    n = mats[0][0].shape[0]
+    for i, (Vm, _) in enumerate(mats):
+        if Vm.shape[0] != n:
+            raise ValueError(f"Vs[{i}] has {Vm.shape[0]} rows but Vs[0] has {n}")
+        if Vm.device != mats[0][0].device:
+            raise ValueError("all designs must be on the same device")
+    key = STACKED.key(Vs, mats, use_planes)
+    st = STACKED.get(key)
+    if st is not None:
+        return st
+    STACKED.invalidate()
+    if before_build is not None:
+        before_build()
+    widths, true_widths = [Vm.shape[1] for Vm, _ in mats], [V.shape[1] for V in Vs]
+    if use_planes:
+        st = Stacked(key, n, widths, true_widths, split_planes_stacked(mats, n, colsq=True), None)
+    else:
+        Vc = torch.zeros(n, sum(widths), device=mats[0][0].device, dtype=torch.float32)
+        o = 0
+        for V, w in zip(Vs, widths):
+            Vc[:, o:o + V.shape[1]] = V.detach()
+            o += w
+        st = Stacked(key, n, widths, true_widths, None, Vc)
+    STACKED.put(Vs, st)
+    return st
+
+
+def split_planes_stacked(mats, n: int, colsq: bool = False, unit_bound: bool = False) -> Planes:
+    """Operand planes of [M_0 | M_1 | ...] for mats = [(M_i, ld_i)] (fp32, n rows, widths multiples of 4), written
+    directly from the sources with one common scale (gpp_split_planes_stacked)."""
+    lib = _lib.load()
+    dev = mats[0][0].device
+    cols = [M.shape[1] for M, _ in mats]
+    k = len(mats)
+    with torch.cuda.device(dev):
+        buf = _workspace(lib.gpp_planes_bytes(n, sum(cols)), dev)
+        c32 = _lib.host_i32(cols)
+        ws = _workspace(lib.gpp_split_stacked_workspace_bytes(n, k, c32) if colsq else 0, dev)
+        flags = (GPP_PLANES_COLSQ if colsq else 0) | (GPP_PLANES_UNIT_BOUND if unit_bound else 0)
+        check(lib.gpp_split_planes_stacked(k, _lib.host_ptrs([M.data_ptr() for M, _ in mats]),
+                                           _lib.host_i64([ld for _, ld in mats]), c32, n, flags, _p(buf), buf.numel(),
+                                           _p(ws), ws.numel(), _stream(dev)), "split_planes_stacked")
+    return Planes(buf, n, sum(cols), colsq)
+
+
 @_on_device
 def khatri_rao_fwd(xn: torch.Tensor, wn: torch.Tensor, d: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
     """V (n x p*q) from row-normalised tables; returns a view with the reference's shape (columns are
@@ -326,10 +425,12 @@ def atb(A: torch.Tensor, lda: int, B: torch.Tensor, ldb: int, n: int, ka: int, k
 
 
 class Factorisation:
-    """State left by gpp_factor: Lc and Linv inside `state`, the scalar block, optionally Binv."""
+    """State left by gpp_factor: Lc and Linv inside `state`, the scalar block, optionally Binv.  Block form
+    (gpp_factor_blocks): `widths` are the designs' column counts, `blk` the per-block scalars, Binv = D B^-1 D."""
 
-    def __init__(self, Q: int, state: torch.Tensor, scal: torch.Tensor, Binv: Optional[torch.Tensor]):
-        self.Q, self.state, self.scal, self.Binv = Q, state, scal, Binv
+    def __init__(self, Q: int, state: torch.Tensor, scal: torch.Tensor, Binv: Optional[torch.Tensor],
+                 widths=None, blk: Optional[torch.Tensor] = None):
+        self.Q, self.state, self.scal, self.Binv, self.widths, self.blk = Q, state, scal, Binv, widths, blk
 
 
 @_on_device
@@ -356,6 +457,47 @@ def solve_w(f: Factorisation, C: torch.Tensor, ldc: int, L: int, L_true: int, n_
     check(lib.gpp_solve_w(_p(C), ldc, f.Q, L, L_true, n_total, _p(W), L, _p(scal), _p(f.state), f.state.numel(),
                           _p(ws), ws.numel(), _stream()), "solve_w")
     return W, scal
+
+
+@_on_device
+def factor_blocks(G: torch.Tensor, ldg: int, widths, vs: torch.Tensor, want_binv: bool) -> Factorisation:
+    """gpp_factor_blocks: B = I + D G D / vn for the stacked designs of column counts `widths`."""
+    lib = _lib.load()
+    dev = G.device
+    Q, k = sum(widths), len(widths)
+    state = _workspace(lib.gpp_factor_blocks_state_bytes(Q, k), dev)
+    scal = torch.zeros(NSCAL, device=dev, dtype=torch.float64)
+    blk = torch.zeros(2 * k, device=dev, dtype=torch.float64)
+    Binv = torch.empty(Q, Q, device=dev, dtype=torch.float32) if want_binv else None
+    vs32 = vs.detach().to(torch.float32).contiguous()
+    check(lib.gpp_factor_blocks(_p(G), ldg, k, _lib.host_i32(widths), _p(vs32), GPP_WANT_BINV if want_binv else 0,
+                                _p(Binv), _p(scal), _p(blk), _p(state), state.numel(), _stream()), "factor_blocks")
+    return Factorisation(Q, state, scal, Binv, list(widths), blk)
+
+
+@_on_device
+def solve_w_blocks(f: Factorisation, C: torch.Tensor, ldc: int, L: int, L_true: int, n_total: int
+                   ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """W = D B^-1 D C / vn and private copies of the scalar block and of the per-block scalars (||W_i||^2 added)."""
+    lib = _lib.load()
+    k = len(f.widths)
+    W = torch.empty(f.Q, L, device=C.device, dtype=torch.float32)
+    scal, blk = f.scal.clone(), f.blk.clone()
+    ws = _workspace(lib.gpp_solve_blocks_workspace_bytes(f.Q, L, k), C.device)
+    check(lib.gpp_solve_w_blocks(_p(C), ldc, k, _lib.host_i32(f.widths), L, L_true, n_total, _p(W), L, _p(scal), _p(blk),
+                                 _p(f.state), f.state.numel(), _p(ws), ws.numel(), _stream()), "solve_w_blocks")
+    return W, scal, blk
+
+
+@_on_device
+def vbs_blocks(scal: torch.Tensor, blk: torch.Tensor, vs: torch.Tensor, widths, n_total: int, L: int) -> torch.Tensor:
+    """vbs = dNLL/d[v_0 .. v_{k-1}, vn] (k + 1 entries)."""
+    k = len(widths)
+    out = torch.empty(k + 1, device=scal.device, dtype=torch.float32)
+    vs32 = vs.detach().to(torch.float32).contiguous()
+    check(_lib.load().gpp_vbs_blocks(_p(scal), _p(blk), _p(vs32), k, _lib.host_i32(widths), n_total, L, _p(out),
+                                     _stream()), "vbs_blocks")
+    return out
 
 
 @_on_device
@@ -543,6 +685,59 @@ class _TaylorExpansion(torch.autograd.Function):
         check(lib.gpp_taylor_expansion_bwd(_p(g), _p(Xbm), ldxb, _p(Vbm), ldvb, n, Lk, Qk, _p(vbs32), _p(lvs32),
                                            _p(gX), Lk, _p(gV), max(Qk, 4), _p(gl), _stream()), "taylor_expansion_bwd")
         return (gX[:, :L] if need_x and Lk != L else gX, gV[:, :Q] if need_v and Qk != Q else gV, gl, None, None, None)
+
+
+class _TaylorExpansionMulti(torch.autograd.Function):
+    """gp.py:127-133 over k designs (k + 1 variances) as one fused forward and one fused backward launch.
+    apply(X, lvs, Xb, vbs, V_0 .. V_{k-1}, Vb_0 .. Vb_{k-1})."""
+
+    @staticmethod
+    def forward(ctx, X, lvs, Xb, vbs, *VVb):
+        lib = _lib.load()
+        k = len(VVb) // 2
+        Xm, ldx = as_matrix(X, "X")
+        Xbm, ldxb = as_matrix(Xb, "Xb")
+        n, L = X.shape
+        Lk = Xm.shape[1]
+        Vm = [as_matrix(V, f"Vs[{j}]") for j, V in enumerate(VVb[:k])]
+        Vbm = [as_matrix(Vb, f"Vbs[{j}]") for j, Vb in enumerate(VVb[k:])]
+        for j in range(k):
+            if VVb[j].shape != VVb[k + j].shape:
+                raise ValueError(f"Vs[{j}] is {tuple(VVb[j].shape)} but Vbs[{j}] is {tuple(VVb[k + j].shape)}")
+        Qk = [M.shape[1] for M, _ in Vm]
+        vbs32 = vbs.detach().to(torch.float32).contiguous()
+        lvs32 = lvs.detach().to(torch.float32).contiguous()
+        if vbs32.numel() != k + 1 or lvs32.numel() != k + 1:
+            raise ValueError(f"vbs and lvs must have {k + 1} entries for {k} designs")
+        out = torch.empty(n, 1, device=X.device, dtype=torch.float32)
+        check(lib.gpp_taylor_expansion_fwd_multi(_p(Xm), ldx, _p(Xbm), ldxb, k, _lib.host_ptrs([_p(M) for M, _ in Vm]),
+                                                 _lib.host_i64([ld for _, ld in Vm]),
+                                                 _lib.host_ptrs([_p(M) for M, _ in Vbm]),
+                                                 _lib.host_i64([ld for _, ld in Vbm]), _lib.host_i32(Qk), n, Lk, _p(vbs32),
+                                                 _p(lvs32), _p(out), _stream()), "taylor_expansion_fwd_multi")
+        ctx.save_for_backward(Xbm, vbs32, lvs32, *[M for M, _ in Vbm])
+        ctx.dims = (n, L, Lk, ldxb, [V.shape[1] for V in VVb[:k]], Qk, [ld for _, ld in Vbm])
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        lib = _lib.load()
+        Xbm, vbs32, lvs32, *Vbm = ctx.saved_tensors
+        n, L, Lk, ldxb, Qt, Qk, ldvb = ctx.dims
+        k = len(Vbm)
+        g = gout.detach().to(torch.float32).contiguous().view(-1)
+        need_x, need_l = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        need_v = ctx.needs_input_grad[4:4 + k]
+        gX = torch.empty(n, Lk, device=g.device, dtype=torch.float32) if need_x else None
+        gV = [torch.empty(n, Qk[j], device=g.device, dtype=torch.float32) if need_v[j] else None for j in range(k)]
+        gl = torch.empty(k + 1, device=g.device, dtype=torch.float32) if need_l else None
+        check(lib.gpp_taylor_expansion_bwd_multi(_p(g), _p(Xbm), ldxb, k, _lib.host_ptrs([_p(M) for M in Vbm]),
+                                                 _lib.host_i64(ldvb), _lib.host_i32(Qk), n, Lk, _p(vbs32), _p(lvs32),
+                                                 _p(gX), Lk, _lib.host_ptrs([_p(t) for t in gV]),
+                                                 _lib.host_i64(Qk), _p(gl), _stream()), "taylor_expansion_bwd_multi")
+        gX = gX[:, :L] if need_x and Lk != L else gX
+        gV = [t[:, :Qt[j]] if t is not None and Qk[j] != Qt[j] else t for j, t in enumerate(gV)]
+        return (gX, gl, None, None, *gV, *([None] * k))
 
 
 def normalize_rows(x: torch.Tensor) -> torch.Tensor:

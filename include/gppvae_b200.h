@@ -201,6 +201,55 @@ int gpp_atb(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t n,
 int gpp_am(const float* A, int64_t lda, const float* M, int64_t ldm, int64_t n, int32_t k, int32_t m, float alpha,
            float* out, int64_t ldo, void* workspace, size_t workspace_bytes, gpp_stream_t stream);
 
+/* ---------------- several random effects: GP(n_rand_effs = k)  (gp.py:21-22,27,55-95,127-133) ----------------
+ * K = sum_i v_i V_i V_i^T + vn I with vs = softmax(lvs) = [v_0 .. v_{k-1}, vn] (k + 1 entries, DEVICE vector).  The
+ * designs are stacked, V = [V_0 | ... | V_{k-1}] (n x Q, Q = sum Q_i; gp.py:27 concatenates sqrt(v_i) V_i), and with
+ * D = diag(sqrt(v_i) on the columns of block i):
+ *   B = I + D G D / vn (G = V^T V),   W = D B^-1 D C / vn (C = V^T X),   Xb = (X - V W) / vn.
+ * Block column counts travel as a HOST int32 array cols_host[k] (each a positive multiple of 4, k <= GPP_MAX_DESIGNS);
+ * per-block scalars as a caller-owned DEVICE double[2k]: blk[2i] = tr_i B^-1 (the diagonal of B^-1 over block i),
+ * blk[2i + 1] = ||W_i||^2 (row block i of W).
+ *   gpp_split_planes_stacked  planes of the concatenation written directly from the k fp32 sources (X_host: HOST array of
+ *                             k device pointers, ldx_host their leading dimensions): one exact magnitude scan over all
+ *                             sources (skipped with GPP_PLANES_UNIT_BOUND), every source column written once into its
+ *                             column range, the column sums of squares (GPP_PLANES_COLSQ) in a fixed order.  The buffer is
+ *                             what gpp_split_planes makes of the concatenation: every *_planes entry takes it.
+ *   gpp_factor_blocks         gp.py:27-35 for k designs: the Cholesky of B as gpp_factor does it; writes
+ *                             scal[V0] = 1, scal[VN] = vn, LOGDETB, TRBINV (all blocks), blk[2i]; with GPP_WANT_BINV,
+ *                             Binv = D B^-1 D.  With scal[V0] = 1 and this Binv, gpp_xb_nll(_planes) and gpp_vb(_planes)
+ *                             compute the k-design Xb, nll (gp.py:42-44,84-87) and Vb = [Vb_0 | ... ] (gp.py:68-71)
+ *                             unchanged.  The state also serves gpp_solve_w (W without the per-block norms).
+ *   gpp_solve_w_blocks        W = D B^-1 D C / vn, scal[WNORM2, ROWCONST] as gpp_solve_w, and blk[2i + 1].
+ *   gpp_vbs_blocks            vbs (k + 1 entries, gp.py:75-81):  vbs[i] = -||W_i||^2 / (2 v_i^2) + L (Q_i - tr_i B^-1) / (2 v_i),
+ *                             vbs[k] = -sum Xb^2 / 2 + L (n_total - Q + tr B^-1) / (2 vn); sum Xb^2 from scal[XB2]
+ *                             (all-reduced by the caller when rows are sharded). */
+#define GPP_MAX_DESIGNS 16
+size_t gpp_split_stacked_workspace_bytes(int64_t n, int32_t k, const int32_t* cols_host);
+int gpp_split_planes_stacked(int32_t k, const float* const* X_host, const int64_t* ldx_host, const int32_t* cols_host,
+                             int64_t n, uint32_t flags, void* planes, size_t planes_bytes, void* workspace,
+                             size_t workspace_bytes, gpp_stream_t stream);
+size_t gpp_factor_blocks_state_bytes(int32_t Q, int32_t k);
+int gpp_factor_blocks(const float* G, int64_t ldg, int32_t k, const int32_t* cols_host, const float* vs, uint32_t flags,
+                      float* Binv, double* scal, double* blk, void* state, size_t state_bytes, gpp_stream_t stream);
+size_t gpp_solve_blocks_workspace_bytes(int32_t Q, int32_t L, int32_t k);
+int gpp_solve_w_blocks(const float* C, int64_t ldc, int32_t k, const int32_t* cols_host, int32_t L, int32_t L_true,
+                       int64_t n_total, float* W, int64_t ldw, double* scal, double* blk, const void* state,
+                       size_t state_bytes, void* workspace, size_t workspace_bytes, gpp_stream_t stream);
+int gpp_vbs_blocks(const double* scal, const double* blk, const float* vs, int32_t k, const int32_t* cols_host,
+                   int64_t n_total, int32_t L, float* vbs, gpp_stream_t stream);
+/* Taylor surrogate over k designs (gp.py:127-133):  out_i = Xb_i.X_i + sum_j Vb_j,i.V_j,i + <vbs, softmax(lvs)> / n,
+ * vbs and lvs of k + 1 entries; V_host / Vb_host are HOST arrays of k device pointers, Q_host the designs' column counts
+ * (multiples of 4).  Backward: gX = gout_i Xb_i, gV_j = gout_i Vb_j, glvs = J_softmax^T vbs * sum(gout) / n (k + 1
+ * entries); gX, glvs and any gV_host[j] may be NULL when that gradient is not needed.  One launch each whatever k is. */
+int gpp_taylor_expansion_fwd_multi(const float* X, int64_t ldx, const float* Xb, int64_t ldxb, int32_t k,
+                                   const float* const* V_host, const int64_t* ldv_host, const float* const* Vb_host,
+                                   const int64_t* ldvb_host, const int32_t* Q_host, int64_t n, int32_t L,
+                                   const float* vbs, const float* lvs, float* out, gpp_stream_t stream);
+int gpp_taylor_expansion_bwd_multi(const float* gout, const float* Xb, int64_t ldxb, int32_t k,
+                                   const float* const* Vb_host, const int64_t* ldvb_host, const int32_t* Q_host,
+                                   int64_t n, int32_t L, const float* vbs, const float* lvs, float* gX, int64_t ldgx,
+                                   float* const* gV_host, const int64_t* ldgv_host, float* glvs, gpp_stream_t stream);
+
 /* ---------------- structured Khatri-Rao path (V never materialised; SURVEY.md 8(f) row 4) ----------------
  * V[i, j q + k] = xn[d_i, j] wn[w_i, k] (vmod.py:28-35), so V^T V, V^T X and V W (gp.py:30,42-44) factor through the
  * (object, view) slots s = o * nviews + v:
