@@ -4,7 +4,8 @@ Drop-in for the reference's `gp.GP` and `vmod.Vmodel` (ahmerb/GPPVAE, pysrc/face
 All numerics run in libgppvae_b200.so (hand-written CUDA, C ABI in include/gppvae_b200.h); there is no
 CPU path: tensors must live on a CUDA device.
 """
-from .gp import GP, KhatriRaoFactor, LazyVb, LowRankFactor  # noqa: F401
-from .vmod import KhatriRao, Vmodel, normalize_rows  # noqa: F401
+from .gp import GP, EffectsFactor, KhatriRaoFactor, LazyEffectVb, LazyVb, LowRankFactor  # noqa: F401
+from .vmod import KhatriRao, ObjectEffect, ViewEffect, Vmodel, normalize_rows  # noqa: F401
 
-__all__ = ["GP", "Vmodel", "normalize_rows", "LowRankFactor", "KhatriRao", "KhatriRaoFactor", "LazyVb"]
+__all__ = ["GP", "Vmodel", "normalize_rows", "LowRankFactor", "KhatriRao", "KhatriRaoFactor", "LazyVb", "ObjectEffect",
+           "ViewEffect", "EffectsFactor", "LazyEffectVb"]

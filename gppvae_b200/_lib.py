@@ -18,6 +18,8 @@ GPP_PLANES_COLSQ, GPP_PLANES_UNIT_BOUND = 1, 2
 S_V0, S_VN, S_LOGDETB, S_TRBINV, S_WNORM2, S_ROWCONST, S_XB2, S_QUAD, NSCAL = range(9)
 
 GPP_MAX_DESIGNS = 16
+# factored designs over one slot index (enum gpp_effect_kind)
+EFFECT_KINDS = {"kr": 0, "object": 1, "view": 2}
 
 _PF = c_void_p   # device pointers travel as void*
 # HOST arrays (the k-design entries): of device pointers, of int64 leading dimensions, of int32 column counts
@@ -102,6 +104,15 @@ _SIGNATURES = {
     "gpp_kr_xb_workspace_bytes": (c_size_t, [c_int64]),
     "gpp_kr_xb_nll": (c_int, [_PF, c_int64, _PF, c_int64, _PF, _PF, c_int64, c_int64, c_int32, c_int32, _PF, _PF,
                               c_int64, _PF, _PF, c_size_t, c_void_p]),
+    "gpp_kr_view_sums_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32, c_int32, c_int32]),
+    "gpp_kr_view_sums": (c_int, [_PF, c_int64, _PF, _PF, _PF, c_int64, c_int32, c_int32, c_int32, c_int32, _PF, c_int64,
+                                 _PF, c_size_t, c_void_p]),
+    "gpp_kr_assemble_gc_blocks": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int32, c_int32, c_int32, c_int32, c_int32,
+                                          _I32H, c_int32, _PF, c_int64, c_void_p]),
+    "gpp_kr_assemble_m_blocks": (c_int, [_PF, c_int64, _PF, c_int32, c_int32, c_int32, c_int32, c_int32, _I32H, _PF,
+                                         c_int64, _PF, c_int64, c_void_p]),
+    "gpp_kr_xb_nll_views": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, _PF, c_int64, c_int64, c_int32,
+                                    c_int32, _PF, _PF, c_int64, _PF, _PF, c_size_t, c_void_p]),
     "gpp_taylor_expansion_fwd": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, c_int64, c_int64, c_int32,
                                          c_int32, _PF, _PF, _PF, c_void_p]),
     "gpp_taylor_expansion_bwd": (c_int, [_PF, _PF, c_int64, _PF, c_int64, c_int64, c_int32, c_int32, _PF, _PF, _PF,

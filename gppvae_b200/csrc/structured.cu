@@ -153,6 +153,264 @@ __global__ void __launch_bounds__(256) kr_xb_kernel(const float* __restrict__ X,
 
 constexpr int kKrXbBlocks = 1184;   // 8 x 148
 
+// ---------------------------------------------------------------- several factored designs (GP(n_rand_effs = k))
+// Object-only x^[d] and view-only w^[w] designs are slot functions too.  Beside S_v and T_v they need the per-view
+// first moments  z_v = sum_{i: w_i = v} X_i (L),  a_v = x^T cnt_v (p),  n_v = sum_o cnt[o, v]:
+// every block of GC = V^T [V | X] for V = [V_K | V_O | V_W] (any order, each kind at most once) is then a sum over v
+// of (row weight) (column weight) (S_v, a_v or n_v), the weight being wn[v, k] for a K or W index and 1 for an O index.
+struct EffLayout {
+  int k;
+  int kind[3];   // GPP_EFFECT_*
+  int off[4];    // first column of every block, off[k] = Q
+};
+
+// Row or column t of the stacked design: its kind, its object column j (-1 for a W index) and its view column k
+// (-1 for an O index); a W index at or past q is padding (kind = -1: an exactly zero row / column).
+__device__ __forceinline__ void eff_decode(const EffLayout& lay, int t, int q, int& kind, int& j, int& kk) {
+  int b = 0;
+  while (b + 1 < lay.k && t >= lay.off[b + 1]) ++b;
+  const int u = t - lay.off[b];
+  kind = lay.kind[b];
+  if (kind == GPP_EFFECT_KR) { j = u / q; kk = u - j * q; }
+  else if (kind == GPP_EFFECT_OBJECT) { j = u; kk = -1; }
+  else { j = -1; kk = u; if (u >= q) kind = -1; }
+}
+
+// Partials of the per-view moments.  Block (c, v) walks the objects of chunk c in order and, for each, the rows of
+// slot (o, v) in slot order; part[(c nviews + v) ldp + ...] = [z (L) | a (p) | n, 0, 0, 0].  Four rows are loaded
+// before they are added (in row order), so the sums do not depend on the launch.
+__global__ void __launch_bounds__(256) kr_view_sums_partial_kernel(const float* __restrict__ X, int64_t ldx,
+                                                                    const int64_t* __restrict__ order,
+                                                                    const int64_t* __restrict__ slot_start,
+                                                                    const float* __restrict__ xn, int64_t P, int p,
+                                                                    int nviews, int L, int with_x, int64_t chunk,
+                                                                    float* __restrict__ part, int64_t ldp) {
+  const int v = blockIdx.y;
+  const int64_t o0 = (int64_t)blockIdx.x * chunk, o1 = (o0 + chunk < P) ? o0 + chunk : P;
+  float* out = part + ((int64_t)blockIdx.x * nviews + v) * ldp;
+  for (int c = threadIdx.x * 4; c < L; c += blockDim.x * 4) {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int64_t o = o0; o < o1; ++o) {
+      const int64_t s = o * nviews + v;
+      int64_t t = slot_start[s];
+      const int64_t e = slot_start[s + 1];
+      for (; t + 4 <= e; t += 4) {
+        float4 x[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) x[u] = *reinterpret_cast<const float4*>(X + order[t + u] * ldx + c);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) { acc.x += x[u].x; acc.y += x[u].y; acc.z += x[u].z; acc.w += x[u].w; }
+      }
+      for (; t < e; ++t) {
+        const float4 x = *reinterpret_cast<const float4*>(X + order[t] * ldx + c);
+        acc.x += x.x; acc.y += x.y; acc.z += x.z; acc.w += x.w;
+      }
+    }
+    *reinterpret_cast<float4*>(out + c) = acc;
+  }
+  if (!with_x) return;
+  for (int c = threadIdx.x * 4; c < p; c += blockDim.x * 4) {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int64_t o = o0; o < o1; ++o) {
+      const int64_t s = o * nviews + v;
+      const float cnt = (float)(slot_start[s + 1] - slot_start[s]);
+      const float4 x = *reinterpret_cast<const float4*>(xn + o * p + c);
+      acc.x = fmaf(cnt, x.x, acc.x); acc.y = fmaf(cnt, x.y, acc.y); acc.z = fmaf(cnt, x.z, acc.z); acc.w = fmaf(cnt, x.w, acc.w);
+    }
+    *reinterpret_cast<float4*>(out + L + c) = acc;
+  }
+  if (threadIdx.x == 0) {
+    int64_t n = 0;
+    for (int64_t o = o0; o < o1; ++o) n += slot_start[o * nviews + v + 1] - slot_start[o * nviews + v];
+    *reinterpret_cast<float4*>(out + L + p) = make_float4((float)n, 0.f, 0.f, 0.f);
+  }
+}
+
+// VM[v, c] = sum over the chunks, in chunk order, of the partials (n_v in double: an exact count).
+__global__ void __launch_bounds__(256) kr_view_sums_reduce_kernel(const float* __restrict__ part, int64_t ldp,
+                                                                   int nchunks, int nviews, int width, int ncnt,
+                                                                   float* __restrict__ VM, int64_t ldvm) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= (int64_t)nviews * width) return;
+  const int v = (int)(e / width), c = (int)(e - (int64_t)v * width);
+  if (c == ncnt) {
+    double n = 0;
+    for (int ch = 0; ch < nchunks; ++ch) n += (double)part[((int64_t)ch * nviews + v) * ldp + c];
+    VM[(int64_t)v * ldvm + c] = (float)n;
+    return;
+  }
+  float s = 0.f;
+  for (int ch = 0; ch < nchunks; ++ch) s += part[((int64_t)ch * nviews + v) * ldp + c];
+  VM[(int64_t)v * ldvm + c] = s;
+}
+
+// The stacked GC (Q x ((with_g ? Q : 0) + L)) of the layout from ST (as kr_assemble_gc reads it) and VM
+// (nviews rows [z_v | a_v | n_v]).  One block per GC row; wn in shared memory.
+__global__ void __launch_bounds__(256) kr_assemble_gc_blocks_kernel(const float* __restrict__ ST, int64_t ldst,
+                                                                    const float* __restrict__ VM, int64_t ldvm,
+                                                                    const float* __restrict__ wn, int p, int q,
+                                                                    int nviews, int L, int with_g, EffLayout lay,
+                                                                    float* __restrict__ GC, int64_t ldgc) {
+  extern __shared__ float wsm[];   // wn, nviews x q
+  for (int e = threadIdx.x; e < nviews * q; e += blockDim.x) wsm[e] = wn[e];
+  __syncthreads();
+  const int Q = lay.off[lay.k];
+  const int Qg = with_g ? Q : 0;
+  const int zcol0 = with_g ? nviews * p : 0;
+  const int r = blockIdx.x;
+  int rkind, rj, rk;
+  eff_decode(lay, r, q, rkind, rj, rk);
+  const int ncol4 = (Qg + L) >> 2;
+  for (int c4 = threadIdx.x; c4 < ncol4; c4 += blockDim.x) {
+    const int c = c4 << 2;
+    float o[4] = {0.f, 0.f, 0.f, 0.f};
+    if (rkind < 0) {
+      // padding row of the view block: exactly zero
+    } else if (c < Qg) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        int ckind, cj, ck;
+        eff_decode(lay, c + e, q, ckind, cj, ck);
+        if (ckind < 0) continue;
+        float s = 0.f;
+        for (int v = 0; v < nviews; ++v) {
+          const float wr = rk >= 0 ? wsm[v * q + rk] : 1.f;
+          const float wc = ck >= 0 ? wsm[v * q + ck] : 1.f;
+          float base;
+          if (rj >= 0 && cj >= 0) base = ST[(int64_t)rj * ldst + v * p + cj];
+          else if (rj >= 0) base = VM[(int64_t)v * ldvm + L + rj];
+          else if (cj >= 0) base = VM[(int64_t)v * ldvm + L + cj];
+          else base = VM[(int64_t)v * ldvm + L + p];
+          s = fmaf(wr * wc, base, s);
+        }
+        o[e] = s;
+      }
+    } else {
+      const int l = c - Qg;
+      for (int v = 0; v < nviews; ++v) {
+        const float4 t = rj >= 0 ? *reinterpret_cast<const float4*>(ST + (int64_t)rj * ldst + zcol0 + (int64_t)v * L + l)
+                                 : *reinterpret_cast<const float4*>(VM + (int64_t)v * ldvm + l);
+        const float wk = rk >= 0 ? wsm[v * q + rk] : 1.f;
+        o[0] = fmaf(wk, t.x, o[0]); o[1] = fmaf(wk, t.y, o[1]); o[2] = fmaf(wk, t.z, o[2]); o[3] = fmaf(wk, t.w, o[3]);
+      }
+    }
+    *reinterpret_cast<float4*>(GC + (int64_t)r * ldgc + c) = make_float4(o[0], o[1], o[2], o[3]);
+  }
+}
+
+// Blocks 0 .. p-1: M[j, v L + l] = sum_k wn[v,k] W_K[(j,k), l] + W_O[j, l];  blocks p .. p + nviews - 1:
+// R[v, l] = sum_k wn[v,k] W_W[k, l].  offK / offO / offW: the row of W where the block starts, -1 when absent.
+__global__ void __launch_bounds__(256) kr_assemble_m_blocks_kernel(const float* __restrict__ W, int64_t ldw,
+                                                                   const float* __restrict__ wn, int p, int q,
+                                                                   int nviews, int L, int offK, int offO, int offW,
+                                                                   float* __restrict__ M, int64_t ldm,
+                                                                   float* __restrict__ R, int64_t ldr) {
+  const int L4 = L >> 2;
+  if ((int)blockIdx.x >= p) {
+    const int v = blockIdx.x - p;
+    for (int c4 = threadIdx.x; c4 < L4; c4 += blockDim.x) {
+      const int l = c4 << 2;
+      float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int k = 0; k < q; ++k) {
+        const float wk = wn[v * q + k];
+        const float4 x = *reinterpret_cast<const float4*>(W + (int64_t)(offW + k) * ldw + l);
+        acc.x = fmaf(wk, x.x, acc.x); acc.y = fmaf(wk, x.y, acc.y); acc.z = fmaf(wk, x.z, acc.z); acc.w = fmaf(wk, x.w, acc.w);
+      }
+      *reinterpret_cast<float4*>(R + (int64_t)v * ldr + l) = acc;
+    }
+    return;
+  }
+  const int j = blockIdx.x;
+  for (int c4 = threadIdx.x; c4 < nviews * L4; c4 += blockDim.x) {
+    const int c = c4 << 2, v = c / L, l = c - v * L;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (offK >= 0) {
+      for (int k = 0; k < q; ++k) {
+        const float wk = wn[v * q + k];
+        const float4 x = *reinterpret_cast<const float4*>(W + (int64_t)(offK + j * q + k) * ldw + l);
+        acc.x = fmaf(wk, x.x, acc.x); acc.y = fmaf(wk, x.y, acc.y); acc.z = fmaf(wk, x.z, acc.z); acc.w = fmaf(wk, x.w, acc.w);
+      }
+    }
+    if (offO >= 0) {
+      const float4 x = *reinterpret_cast<const float4*>(W + (int64_t)(offO + j) * ldw + l);
+      acc.x += x.x; acc.y += x.y; acc.z += x.z; acc.w += x.w;
+    }
+    *reinterpret_cast<float4*>(M + (int64_t)j * ldm + c) = acc;
+  }
+}
+
+// kr_xb_kernel with the per-view row: Xb_i = (X_i - Y[d_i, w_i L ..] - R[w_i]) / vn.
+__global__ void __launch_bounds__(256) kr_xb_views_kernel(const float* __restrict__ X, int64_t ldx,
+                                                          const float* __restrict__ Y, int64_t ldy,
+                                                          const float* __restrict__ R, int64_t ldr,
+                                                          const int64_t* __restrict__ d, const int64_t* __restrict__ w,
+                                                          int64_t n, int64_t P, int nviews, int L,
+                                                          const double* __restrict__ scal, float* __restrict__ Xb,
+                                                          int64_t ldxb, float* __restrict__ quad,
+                                                          double* __restrict__ xb2_part) {
+  __shared__ double red[8];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int64_t warp = (int64_t)blockIdx.x * 8 + wib, nwarps = (int64_t)gridDim.x * 8;
+  const float inv_vn = (float)(1.0 / scal[GPP_S_VN]);
+  const float qnan = __int_as_float(0x7fc00000);
+  double xb2 = 0;
+  for (int64_t i = warp; i < n; i += nwarps) {
+    const int64_t di = d[i], wi = w[i];
+    const bool ok = (di >= 0) & (di < P) & (wi >= 0) & (wi < nviews);
+    const float* y = Y + (ok ? di * ldy + wi * L : 0);
+    const float* rr = R + (ok ? wi * ldr : 0);
+    float qs = 0.f, x2 = 0.f;
+    for (int c = lane * 4; c < L; c += 128) {
+      const float4 x = *reinterpret_cast<const float4*>(X + i * ldx + c);
+      const float4 yy = *reinterpret_cast<const float4*>(y + c);
+      const float4 r4 = *reinterpret_cast<const float4*>(rr + c);
+      float4 o;
+      o.x = ok ? (x.x - (yy.x + r4.x)) * inv_vn : qnan; o.y = ok ? (x.y - (yy.y + r4.y)) * inv_vn : qnan;
+      o.z = ok ? (x.z - (yy.z + r4.z)) * inv_vn : qnan; o.w = ok ? (x.w - (yy.w + r4.w)) * inv_vn : qnan;
+      *reinterpret_cast<float4*>(Xb + i * ldxb + c) = o;
+      qs = fmaf(x.x, o.x, qs); qs = fmaf(x.y, o.y, qs); qs = fmaf(x.z, o.z, qs); qs = fmaf(x.w, o.w, qs);
+      x2 = fmaf(o.x, o.x, x2); x2 = fmaf(o.y, o.y, x2); x2 = fmaf(o.z, o.z, x2); x2 = fmaf(o.w, o.w, x2);
+    }
+    qs = warp_sum(qs);
+    x2 = warp_sum(x2);
+    if (lane == 0) quad[i] = qs;
+    xb2 += (double)x2;
+  }
+  if (lane == 0) red[wib] = xb2;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0;
+    for (int k = 0; k < 8; ++k) t += red[k];
+    xb2_part[blockIdx.x] = t;
+  }
+}
+
+// Chunks of objects per view for the moments: about 8 blocks per SM over all views, a function of the shape alone.
+inline int64_t view_sums_chunks(int64_t P, int nviews) {
+  const int64_t target = (1184 + nviews - 1) / nviews;
+  return target < P ? target : P;
+}
+
+inline int view_sums_width(int p, int L, int with_x) { return L + (with_x ? p + 4 : 0); }
+
+// Checks the kinds list and fills the layout (block widths p q, p, round4(q)).
+inline int eff_layout(int32_t k, const int32_t* kinds_host, int p, int q, EffLayout& lay, int& has) {
+  if (!(k >= 1 && k <= 3 && kinds_host)) return 0;
+  lay.k = k;
+  has = 0;
+  int off = 0;
+  for (int b = 0; b < k; ++b) {
+    const int kd = kinds_host[b];
+    if (kd < GPP_EFFECT_KR || kd > GPP_EFFECT_VIEW || (has & (1 << kd))) return 0;
+    has |= 1 << kd;
+    lay.kind[b] = kd;
+    lay.off[b] = off;
+    off += kd == GPP_EFFECT_KR ? p * q : kd == GPP_EFFECT_OBJECT ? p : (q + 3) / 4 * 4;
+  }
+  lay.off[k] = off;
+  return 1;
+}
+
 }  // namespace gpp
 
 using namespace gpp;
@@ -225,6 +483,121 @@ extern "C" int gpp_kr_xb_nll(const float* X, int64_t ldx, const float* Y, int64_
   double* fin = part + align_up((size_t)kKrXbBlocks * sizeof(double), 256) / sizeof(double);
   cudaStream_t st = (cudaStream_t)stream;
   kr_xb_kernel<<<kKrXbBlocks, 256, 0, st>>>(X, ldx, Y, ldy, d, w, n, P, nviews, L, scal, Xb, ldxb, quad, part);
+  GPP_LAUNCH_CHECK();
+  return launch_xb_finalize(quad, 1, n, part, kKrXbBlocks, fin, scal, nll, st);
+}
+
+extern "C" size_t gpp_kr_view_sums_workspace_bytes(int64_t P, int32_t p, int32_t nviews, int32_t L, int32_t with_x) {
+  if (P <= 0 || p <= 0 || nviews <= 0 || L <= 0) return 0;
+  return align_up((size_t)view_sums_chunks(P, nviews) * nviews * view_sums_width(p, L, with_x) * sizeof(float), 256);
+}
+
+extern "C" int gpp_kr_view_sums(const float* X, int64_t ldx, const int64_t* order, const int64_t* slot_start,
+                                const float* xn, int64_t P, int32_t p, int32_t nviews, int32_t L, int32_t with_x,
+                                float* VM, int64_t ldvm, void* workspace, size_t workspace_bytes, gpp_stream_t stream) {
+  GPP_REQUIRE(X && order && slot_start && VM && (xn || !with_x), "kr_view_sums: null pointer");
+  GPP_REQUIRE(P > 0 && p > 0 && nviews > 0 && L > 0 && p % 4 == 0 && L % 4 == 0,
+              "kr_view_sums: p and L must be positive multiples of 4");
+  const int width = view_sums_width(p, L, with_x);
+  GPP_REQUIRE(ldx >= L && ldx % 4 == 0 && ldvm >= width && ldvm % 4 == 0 && aligned16(X) && aligned16(VM) &&
+                  (!with_x || aligned16(xn)),
+              "kr_view_sums: bad leading dimension / alignment");
+  const size_t need = gpp_kr_view_sums_workspace_bytes(P, p, nviews, L, with_x);
+  if (!workspace || workspace_bytes < need) {
+    set_error("kr_view_sums: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    return GPP_ERR_WORKSPACE;
+  }
+  const int64_t nch = view_sums_chunks(P, nviews);
+  const int64_t chunk = ceil_div(P, nch);
+  const int cols = (with_x && p > L) ? p : L;
+  int threads = (int)ceil_div((int64_t)cols / 4, 32) * 32;
+  threads = threads > 256 ? 256 : threads;
+  float* part = static_cast<float*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  kr_view_sums_partial_kernel<<<dim3((unsigned)nch, (unsigned)nviews), threads, 0, st>>>(
+      X, ldx, order, slot_start, xn, P, p, nviews, L, with_x, chunk, part, width);
+  GPP_LAUNCH_CHECK();
+  const int64_t total = (int64_t)nviews * width;
+  kr_view_sums_reduce_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(part, width, (int)nch, nviews, width,
+                                                                            with_x ? L + p : -1, VM, ldvm);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_kr_assemble_gc_blocks(const float* ST, int64_t ldst, const float* VM, int64_t ldvm, const float* wn,
+                                         int32_t p, int32_t q, int32_t nviews, int32_t L, int32_t k,
+                                         const int32_t* kinds_host, int32_t with_g, float* GC, int64_t ldgc,
+                                         gpp_stream_t stream) {
+  EffLayout lay;
+  int has = 0;
+  GPP_REQUIRE(p > 0 && q > 0 && nviews > 0 && L >= 0 && p % 4 == 0 && L % 4 == 0 && (L > 0 || with_g),
+              "kr_assemble_gc_blocks: p and L must be multiples of 4");
+  GPP_REQUIRE(eff_layout(k, kinds_host, p, q, lay, has),
+              "kr_assemble_gc_blocks: kinds must list 1..3 distinct GPP_EFFECT_* values");
+  const bool need_st = has & ((1 << GPP_EFFECT_KR) | (1 << GPP_EFFECT_OBJECT));
+  const bool need_vm = has & (1 << GPP_EFFECT_VIEW);
+  GPP_REQUIRE(wn && GC && (ST || !need_st) && (VM || !need_vm), "kr_assemble_gc_blocks: null pointer");
+  const int64_t Q = lay.off[k];
+  GPP_REQUIRE((!need_st || (ldst >= (int64_t)nviews * ((with_g ? p : 0) + L) && ldst % 4 == 0 && aligned16(ST))) &&
+                  (!need_vm || (ldvm >= L + (with_g ? p + 4 : 0) && ldvm % 4 == 0 && aligned16(VM))) &&
+                  ldgc >= (with_g ? Q : 0) + L && ldgc % 4 == 0 && aligned16(GC),
+              "kr_assemble_gc_blocks: bad leading dimension / alignment");
+  const size_t smem = (size_t)nviews * q * sizeof(float);
+  GPP_REQUIRE(smem <= 48 * 1024, "kr_assemble_gc_blocks: view table too large");
+  kr_assemble_gc_blocks_kernel<<<(unsigned)Q, 256, smem, (cudaStream_t)stream>>>(ST, ldst, VM, ldvm, wn, p, q, nviews, L,
+                                                                                 with_g, lay, GC, ldgc);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_kr_assemble_m_blocks(const float* W, int64_t ldw, const float* wn, int32_t p, int32_t q,
+                                        int32_t nviews, int32_t L, int32_t k, const int32_t* kinds_host, float* M,
+                                        int64_t ldm, float* R, int64_t ldr, gpp_stream_t stream) {
+  EffLayout lay;
+  int has = 0;
+  GPP_REQUIRE(p > 0 && q > 0 && nviews > 0 && L > 0 && p % 4 == 0 && L % 4 == 0,
+              "kr_assemble_m_blocks: p and L must be positive multiples of 4");
+  GPP_REQUIRE(eff_layout(k, kinds_host, p, q, lay, has),
+              "kr_assemble_m_blocks: kinds must list 1..3 distinct GPP_EFFECT_* values");
+  const bool need_m = has & ((1 << GPP_EFFECT_KR) | (1 << GPP_EFFECT_OBJECT));
+  const bool need_r = has & (1 << GPP_EFFECT_VIEW);
+  GPP_REQUIRE(W && wn && (M || !need_m) && (R || !need_r), "kr_assemble_m_blocks: null pointer");
+  GPP_REQUIRE(ldw >= L && ldw % 4 == 0 && aligned16(W) &&
+                  (!need_m || (ldm >= (int64_t)nviews * L && ldm % 4 == 0 && aligned16(M))) &&
+                  (!need_r || (ldr >= L && ldr % 4 == 0 && aligned16(R))),
+              "kr_assemble_m_blocks: bad leading dimension / alignment");
+  int off[3] = {-1, -1, -1};
+  for (int b = 0; b < k; ++b) off[lay.kind[b]] = lay.off[b];
+  const unsigned grid = (unsigned)((need_m ? p : 0) + (need_r ? nviews : 0));
+  // without M the R blocks start at 0: shift them by passing p = 0
+  kr_assemble_m_blocks_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(W, ldw, wn, need_m ? p : 0, q, nviews, L,
+                                                                      off[GPP_EFFECT_KR], off[GPP_EFFECT_OBJECT],
+                                                                      off[GPP_EFFECT_VIEW], M, ldm, R, ldr);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_kr_xb_nll_views(const float* X, int64_t ldx, const float* Y, int64_t ldy, const float* R, int64_t ldr,
+                                   const int64_t* d, const int64_t* w, int64_t n, int64_t P, int32_t nviews, int32_t L,
+                                   double* scal, float* Xb, int64_t ldxb, float* nll, void* workspace,
+                                   size_t workspace_bytes, gpp_stream_t stream) {
+  GPP_REQUIRE(X && Y && R && d && w && scal && Xb && nll, "kr_xb_nll_views: null pointer");
+  GPP_REQUIRE(n >= 0 && P > 0 && nviews > 0 && L > 0 && L % 4 == 0, "kr_xb_nll_views: bad shape");
+  GPP_REQUIRE(ldx >= L && ldx % 4 == 0 && ldxb >= L && ldxb % 4 == 0 && ldy >= (int64_t)nviews * L && ldy % 4 == 0 &&
+                  ldr >= L && ldr % 4 == 0 && aligned16(X) && aligned16(Y) && aligned16(R) && aligned16(Xb),
+              "kr_xb_nll_views: bad leading dimension / alignment");
+  const size_t need = gpp_kr_xb_workspace_bytes(n);
+  if (!workspace || workspace_bytes < need) {
+    set_error("kr_xb_nll_views: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    return GPP_ERR_WORKSPACE;
+  }
+  char* ws = static_cast<char*>(workspace);
+  float* quad = reinterpret_cast<float*>(ws);
+  double* part = reinterpret_cast<double*>(ws + align_up((size_t)(n > 0 ? n : 1) * sizeof(float), 256));
+  double* fin = part + align_up((size_t)kKrXbBlocks * sizeof(double), 256) / sizeof(double);
+  cudaStream_t st = (cudaStream_t)stream;
+  kr_xb_views_kernel<<<kKrXbBlocks, 256, 0, st>>>(X, ldx, Y, ldy, R, ldr, d, w, n, P, nviews, L, scal, Xb, ldxb, quad,
+                                                  part);
   GPP_LAUNCH_CHECK();
   return launch_xb_finalize(quad, 1, n, part, kKrXbBlocks, fin, scal, nll, st);
 }

@@ -26,7 +26,7 @@ from torch import nn
 
 from . import ops
 from ._lib import GPP_MAX_DESIGNS, S_QUAD, S_XB2
-from .vmod import KhatriRao
+from .vmod import KhatriRao, _FactoredEffect, effect_base, effect_kind, effects_c, effects_st_vm
 
 
 class LowRankFactor:
@@ -82,6 +82,15 @@ class BlocksFactor(LowRankFactor):
                           for i, (o, V) in enumerate(zip(self.stk.offsets, self.Vs))], 1)
 
 
+class EffectsFactor(BlocksFactor):
+    """`U` / `UBi` of `GP.U_UBi_Shb` for k factored designs (Vmodel.lazy_effects): carries the designs, their block
+    layout (an ops.Stacked without operand) and the block-form factorisation; `GP.solve` takes the structured route with
+    it.  `dense()` goes through the designs' dense()."""
+
+    def dense(self) -> torch.Tensor:
+        return BlocksFactor(self.kind, [V.dense() for V in self.Vs], self.stk, self.vs, self.fac).dense()
+
+
 class KhatriRaoFactor:
     """`U` / `UBi` of `GP.U_UBi_Shb` when V was given in factored form (vmod.KhatriRao): carries the factors and the
     factorisation; `GP.solve` takes the structured route with it.  `dense()` goes through the dense handle."""
@@ -125,6 +134,55 @@ class LazyVb:
         out = torch.empty(n, self.shape[1], device=self.kr.device, dtype=torch.float32)
         for a in range(0, n, chunk):
             idx = torch.arange(a, min(n, a + chunk), device=self.kr.device)
+            out[a:a + idx.numel()] = self[idx]
+        return out
+
+
+class _EffectsVbRows:
+    """Rows of the stacked Vb = (L/vn) V (D B^-1 D) - Xb W^T of k factored designs: the trainer gathers every Vbs[i][idx]
+    with the same idx, so the m x Q product is formed once per index set and sliced per design."""
+
+    def __init__(self, Vs, lay: ops.Stacked, Xb, fac, W, scal, Lk, L):
+        self.Vs, self.lay, self.Xb, self.fac, self.W, self.scal, self.Lk, self.L = list(Vs), lay, Xb, fac, W, scal, Lk, L
+        self.device = Xb.device
+        self._key = self._idx = self._rows = None
+
+    def rows(self, key) -> torch.Tensor:
+        if self._key is not None and key is self._key:
+            return self._rows
+        idx = key if torch.is_tensor(key) else torch.as_tensor(key, device=self.device)
+        idx = idx.to(self.device).reshape(-1)
+        if self._idx is not None and idx.shape == self._idx.shape and torch.equal(idx, self._idx):
+            self._key = key
+            return self._rows
+        lay = self.lay
+        m = idx.numel()
+        Vr = torch.zeros(m, lay.Q, device=self.device, dtype=torch.float32)
+        for V, o, t in zip(self.Vs, lay.offsets, lay.true_widths):
+            Vr[:, o:o + t] = V[idx]
+        Xbr = self.Xb[idx].contiguous()
+        self._rows = ops.vb(Vr, lay.Q, Xbr, self.fac.Binv, self.W, self.scal, m, lay.Q, self.Lk, self.L)
+        self._key, self._idx = key, idx
+        return self._rows
+
+
+class LazyEffectVb:
+    """`Vbs[i]` of a structured evaluation with k factored designs: `[idx]` returns design i's columns of the rows idx
+    of the stacked Vb (see _EffectsVbRows)."""
+
+    def __init__(self, rows: _EffectsVbRows, i: int):
+        self._r, self.i = rows, i
+        self.shape = rows.Vs[i].shape
+
+    def __getitem__(self, idx) -> torch.Tensor:
+        o = self._r.lay.offsets[self.i]
+        return self._r.rows(idx)[:, o:o + self.shape[1]]
+
+    def dense(self, chunk: int = 65536) -> torch.Tensor:
+        n, dev = self.shape[0], self._r.device
+        out = torch.empty(n, self.shape[1], device=dev, dtype=torch.float32)
+        for a in range(0, n, chunk):
+            idx = torch.arange(a, min(n, a + chunk), device=dev)
             out[a:a + idx.numel()] = self[idx]
         return out
 
@@ -285,9 +343,6 @@ class GP(nn.Module):
         k = self.n_rand_effs
         if len(Vs) != k:
             raise ValueError(f"GP(n_rand_effs={k}) expects {k} design matrices in Vs, got {len(Vs)}")
-        if any(isinstance(V, KhatriRao) for V in Vs):
-            raise NotImplementedError("the structured route (vmod.KhatriRao) takes a single design; with n_rand_effs > 1 "
-                                      "pass the dense Khatri-Rao matrix (KhatriRao.dense()) instead")
         n, Q = Vs[0].shape[0], sum(ops.round4(V.shape[1]) for V in Vs)
         use_planes = ops.planes_supported(n, Q, Lk)
 
@@ -397,19 +452,125 @@ class GP(nn.Module):
         self._cache.store(key, (kr, keep_vs), GC, Q + Lx, fac, vs)
         return fac, (GC[:, Q:] if Lk else None)
 
+    @staticmethod
+    def _kr_y(kr: KhatriRao, M: torch.Tensor) -> torch.Tensor:
+        """Y = xn [M_0 | M_1 | ...], the P-long product of the structured pass 2."""
+        if ops.planes_supported(kr.P, kr.p, 0):
+            pM = ops.split_planes(M, M.stride(0), kr.p, M.shape[1])
+            return ops.am_planes(kr.xn_planes(), pM, kr.P, kr.p, M.shape[1])
+        return ops.am(kr.xn, kr.p, M, M.stride(0), kr.P, kr.p, M.shape[1])
+
     def _kr_solve(self, kr: KhatriRao, fac, C, Xm, ldx, Lk, L, n_total):
         """W, the scalar block, Xb = (X - V W)/vn and nll for the rows of X, V in factored form."""
         W, scal = ops.solve_w(fac, C, C.stride(0), Lk, L, n_total)
         self._stage("solve:end")
         M = ops.kr_assemble_m(W, kr.wn, kr.p, Lk)
-        if ops.planes_supported(kr.P, kr.p, 0):
-            pM = ops.split_planes(M, M.stride(0), kr.p, M.shape[1])
-            Y = ops.am_planes(kr.xn_planes(), pM, kr.P, kr.p, M.shape[1])
-        else:
-            Y = ops.am(kr.xn, kr.p, M, M.stride(0), kr.P, kr.p, M.shape[1])
+        Y = self._kr_y(kr, M)
         Xb, nll = ops.kr_xb_nll(Xm, ldx, Y, kr.d, kr.w, kr.P, kr.nviews, Lk, scal)
         self._stage("pass2:end")
         return W, scal, Xb, nll
+
+    # ------------------------------------------------------------------ structured route, k factored designs
+    def _effects(self, Vs) -> Optional[KhatriRao]:
+        """k >= 2 designs: the KhatriRao whose slot index and tables the designs share when they are all factored
+        (Vmodel.lazy_effects), None when they are all dense."""
+        k = self.n_rand_effs
+        if len(Vs) != k:
+            raise ValueError(f"GP(n_rand_effs={k}) expects {k} design matrices in Vs, got {len(Vs)}")
+        factored = [isinstance(V, (KhatriRao, _FactoredEffect)) for V in Vs]
+        if not any(factored):
+            return None
+        if not all(factored):
+            raise NotImplementedError("factored designs (vmod.KhatriRao, ObjectEffect, ViewEffect) and dense designs "
+                                      "cannot be mixed: pass every design factored (Vmodel.lazy_effects) or every one "
+                                      "dense (.dense())")
+        base = effect_base(Vs[0])
+        if any(effect_base(V) is not base for V in Vs):
+            raise ValueError("the factored designs are built over different d, w or tables: make them with one "
+                             "Vmodel.lazy_effects call")
+        kinds = [effect_kind(V) for V in Vs]
+        if len(set(kinds)) != k:
+            raise ValueError(f"each kind of factored design may appear once, got {kinds}")
+        return base
+
+    @staticmethod
+    def _effects_layout(base: KhatriRao, kinds) -> ops.Stacked:
+        """Block layout of the stacked factored designs: widths p q, p, round4(q) (p already padded to 4)."""
+        true = [base.p_true * base.q if k == "kr" else base.p_true if k == "object" else base.q for k in kinds]
+        return ops.Stacked(None, base.n, ops.effect_widths(kinds, base.p, base.q), true, None, None)
+
+    def _all_reduce_pair(self, ST, VM):
+        """SUM of the slot-sum products and the per-view moments over the row shards, in one collective."""
+        if not self._sharded:
+            return ST, VM
+        parts = [t for t in (ST, VM) if t is not None]
+        flat = torch.cat([t.reshape(-1) for t in parts])
+        self._all_reduce(flat)
+        out, o = [], 0
+        for t in (ST, VM):
+            if t is None:
+                out.append(None)
+            else:
+                out.append(flat[o:o + t.numel()].view(t.shape))
+                o += t.numel()
+        return tuple(out)
+
+    def _effects_factorise(self, Vs, base: KhatriRao, kinds, lay, vs, want_binv: bool, Xm=None, ldx=0, Lk=0,
+                           vs_origin=None):
+        """Structured pass 1 of the stacked factored designs (+ one all-reduce of ST and the moments instead of GC) and
+        the block-form factorisation, through the cache (keyed on the designs and the variances)."""
+        tok, keep_vs = self._vs_token(vs if vs_origin is None else vs_origin)
+        key = ("effects", tuple(id(V) for V in Vs), tok)
+        fac = self._cache.lookup(key, want_binv, vs)
+        if fac is not None:
+            self.cache_hits += 1
+            return fac, (effects_c(base, kinds, Xm, ldx, Lk, self._all_reduce_pair) if Lk else None)
+        if not Lk:      # factorisation alone (U_UBi_Shb): the slot sums still need a right-hand side to walk
+            Xm = torch.zeros(base.n, 4, device=base.device, dtype=torch.float32)
+            ldx, Lx = 4, 4
+        else:
+            Lx = Lk
+        base.index()
+        self._stage("pass1:start")
+        ST, VM = effects_st_vm(base, kinds, Xm, ldx, Lx, True)
+        self._stage("pass1:end")
+        ST, VM = self._all_reduce_pair(ST, VM)
+        self._stage("allreduce:end")
+        GC = ops.kr_assemble_gc_blocks(ST, VM, base.wn, base.p, kinds, Lx, True)
+        fac = ops.factor_blocks(GC, lay.Q + Lx, lay.widths, vs, want_binv)
+        self._stage("factor:end")
+        self._cache.store(key, (tuple(Vs), keep_vs), GC, lay.Q + Lx, fac, vs)
+        return fac, (GC[:, lay.Q:] if Lk else None)
+
+    def _effects_solve(self, base: KhatriRao, kinds, fac, C, Xm, ldx, Lk, L, n_total):
+        """W, the scalar blocks, Xb = (X - V W)/vn and nll for the rows of X, the k designs in factored form:
+        (V W)_i = Y[d_i, w_i] + R[w_i]."""
+        W, scal, blk = ops.solve_w_blocks(fac, C, C.stride(0), Lk, L, n_total)
+        self._stage("solve:end")
+        M, R = ops.kr_assemble_m_blocks(W, base.wn, base.p, kinds, Lk)
+        Y = self._kr_y(base, M)
+        if R is None:
+            Xb, nll = ops.kr_xb_nll(Xm, ldx, Y, base.d, base.w, base.P, base.nviews, Lk, scal)
+        else:
+            Xb, nll = ops.kr_xb_nll_views(Xm, ldx, Y, R, base.d, base.w, base.P, base.nviews, Lk, scal)
+        self._stage("pass2:end")
+        return W, scal, blk, Xb, nll
+
+    def _effects_coefficients(self, X, Vs, base: KhatriRao, vs, vs_attached, want_vb: bool):
+        Xm, ldx = ops.as_matrix(X, "X")
+        n, L = X.shape
+        if base.n != n:
+            raise ValueError(f"X has {n} rows but the designs have {base.n}")
+        if base.device != Xm.device:
+            raise ValueError("X and V must be on the same device")
+        Lk = Xm.shape[1]
+        kinds = [effect_kind(V) for V in Vs]
+        lay = self._effects_layout(base, kinds)
+        n_total = self._n_total(n, X.device)
+        fac, C = self._effects_factorise(Vs, base, kinds, lay, vs, want_vb, Xm, ldx, Lk, vs_origin=vs_attached)
+        W, scal, blk, Xb, nll = self._effects_solve(base, kinds, fac, C, Xm, ldx, Lk, L, n_total)
+        return dict(vs=vs, Vm=None, effects=list(Vs), Q=lay.Q, Qtrue=lay.Q, n=n, L=L, Lk=Lk, n_total=n_total, fac=fac,
+                    W=W, scal=scal, Xb=Xb, nll=nll, pV=None, stk=lay, blk=blk)
 
     def U_UBi_Shb(self, Vs: Sequence[torch.Tensor], vs: torch.Tensor, want_binv: bool = False):
         """gp.py:24-38.  Returns handles (see LowRankFactor) that `solve` accepts."""
@@ -419,6 +580,13 @@ class GP(nn.Module):
             return (KhatriRaoFactor("U", kr, vs, fac), KhatriRaoFactor("UBi", kr, vs, fac),
                     LazySingularValues(self._cache.G, kr.p * kr.q, vs))
         if self.n_rand_effs > 1:
+            base = self._effects(Vs)
+            if base is not None:
+                kinds = [effect_kind(V) for V in Vs]
+                lay = self._effects_layout(base, kinds)
+                fac, _ = self._effects_factorise(Vs, base, kinds, lay, vs, want_binv)
+                return (EffectsFactor("U", Vs, lay, vs, fac), EffectsFactor("UBi", Vs, lay, vs, fac),
+                        LazySingularValues(self._cache.G, lay.Q, vs, stk=lay))
             stk = self._stack(Vs, 0)
             fac, _, _ = self._factorise(stk.V, stk.Q, stk.Q, vs, want_binv, stk=stk)
             return (BlocksFactor("U", Vs, stk, vs, fac), BlocksFactor("UBi", Vs, stk, vs, fac),
@@ -434,7 +602,13 @@ class GP(nn.Module):
         Xm, ldx = ops.as_matrix(X, "X")
         n, L = X.shape
         Lk = Xm.shape[1]
-        if isinstance(U, KhatriRaoFactor):
+        if isinstance(U, EffectsFactor):
+            if n != U.n:
+                raise ValueError(f"X has {n} rows but the factorisation was built for {U.n}")
+            base, kinds = effect_base(U.Vs[0]), [effect_kind(V) for V in U.Vs]
+            C = effects_c(base, kinds, Xm, ldx, Lk, self._all_reduce_pair)
+            _, _, _, Xb, _ = self._effects_solve(base, kinds, U.fac, C, Xm, ldx, Lk, L, self._n_total(n, X.device))
+        elif isinstance(U, KhatriRaoFactor):
             if n != U.n:
                 raise ValueError(f"X has {n} rows but the factorisation was built for {U.n}")
             C = self._kr_c(U.kr, Xm, ldx, Lk)
@@ -497,6 +671,9 @@ class GP(nn.Module):
             return dict(vs=vs, Vm=None, kr=kr, ldv=0, Q=kr.p * kr.q, Qtrue=kr.p_true * kr.q, n=n, L=L, Lk=Lk,
                         n_total=n_total, fac=fac, W=W, scal=scal, Xb=Xb, nll=nll)
         if self.n_rand_effs > 1:
+            base = self._effects(Vs)
+            if base is not None:
+                return self._effects_coefficients(X, Vs, base, vs, vs_attached, want_vb)
             Xm, ldx = ops.as_matrix(X, "X")
             n, L = X.shape
             Lk = Xm.shape[1]
@@ -553,7 +730,10 @@ class GP(nn.Module):
             vbs = ops.vbs_blocks(scal, c["blk"], c["vs"], stk.widths, c["n_total"], L)
         else:
             vbs = ops.vbs_from_scal(scal, c["n_total"], Q, L)
-        if need_vb and stk is not None:
+        if need_vb and c.get("effects") is not None:
+            rows = _EffectsVbRows(c["effects"], stk, c["Xb"], c["fac"], c["W"], scal, Lk, L)
+            Vbs = [LazyEffectVb(rows, i) for i in range(len(stk.widths))]
+        elif need_vb and stk is not None:
             # one N x Q matrix; Vb_i is the view of block i at design i's true width
             if c["pV"] is not None:
                 Vb = ops.vb_planes(c["pV"], c["Xb"], c["fac"].Binv, c["W"], scal, c["n"], Q, Lk, L)
@@ -599,9 +779,9 @@ class GP(nn.Module):
             k = self.n_rand_effs
             if len(Vs) != k or len(Vbs) != k:
                 raise ValueError(f"GP(n_rand_effs={k}) expects {k} designs in Vs and Vbs, got {len(Vs)} / {len(Vbs)}")
-            if any(isinstance(V, KhatriRao) for V in Vs):
-                raise NotImplementedError("the structured route (vmod.KhatriRao) takes a single design; with "
-                                          "n_rand_effs > 1 pass the dense Khatri-Rao matrix instead")
+            if any(isinstance(V, (KhatriRao, _FactoredEffect)) for V in Vs):
+                raise NotImplementedError("taylor_expansion takes dense designs: pass the minibatch rows (V[idx]) of "
+                                          "each factored design")
             return ops._TaylorExpansionMulti.apply(X, self.lvs, Xb, vbs, *Vs, *Vbs)
         if len(Vs) != 1 or len(Vbs) != 1:
             raise NotImplementedError(f"expected one design matrix in Vs / Vbs, got {len(Vs)} / {len(Vbs)}")

@@ -13,7 +13,7 @@ import collections
 import weakref
 
 from . import _lib
-from ._lib import GPP_PLANES_COLSQ, GPP_PLANES_UNIT_BOUND, GPP_WANT_BINV, NSCAL, check
+from ._lib import EFFECT_KINDS, GPP_PLANES_COLSQ, GPP_PLANES_UNIT_BOUND, GPP_WANT_BINV, NSCAL, check
 
 
 def _stream(device=None) -> int:
@@ -615,6 +615,67 @@ def kr_xb_nll(X: torch.Tensor, ldx: int, Y: torch.Tensor, d: torch.Tensor, w: to
     ws = _workspace(lib.gpp_kr_xb_workspace_bytes(n), X.device)
     check(lib.gpp_kr_xb_nll(_p(X), ldx, _p(Y), Y.stride(0), _p(d), _p(w), n, P, nviews, L, _p(scal), _p(Xb), L, _p(nll),
                             _p(ws), ws.numel(), _stream()), "kr_xb_nll")
+    return Xb, nll
+
+
+# ----------------------------------------------------------------------------- several factored designs
+@_on_device
+def kr_view_sums(X: torch.Tensor, ldx: int, order: torch.Tensor, slot_start: torch.Tensor, xn: torch.Tensor,
+                 nviews: int, L: int, with_x: bool) -> torch.Tensor:
+    """VM (nviews x (L + (p + 4 if with_x))): rows [z_v | a_v | n_v, 0, 0, 0], the per-view first moments."""
+    lib = _lib.load()
+    P, p = xn.shape
+    VM = torch.empty(nviews, L + (p + 4 if with_x else 0), device=X.device, dtype=torch.float32)
+    ws = _workspace(lib.gpp_kr_view_sums_workspace_bytes(P, p, nviews, L, int(with_x)), X.device)
+    check(lib.gpp_kr_view_sums(_p(X), ldx, _p(order), _p(slot_start), _p(xn), P, p, nviews, L, int(with_x), _p(VM),
+                               VM.stride(0), _p(ws), ws.numel(), _stream()), "kr_view_sums")
+    return VM
+
+
+def effect_widths(kinds, p: int, q: int):
+    """Block widths of the stacked factored designs (p already a multiple of 4)."""
+    return [p * q if k == "kr" else p if k == "object" else round4(q) for k in kinds]
+
+
+@_on_device
+def kr_assemble_gc_blocks(ST: Optional[torch.Tensor], VM: Optional[torch.Tensor], wn: torch.Tensor, p: int, kinds,
+                          L: int, with_g: bool) -> torch.Tensor:
+    """The stacked GC = V^T [V | X] (with_g) or C = V^T X of the factored designs `kinds`, from ST and VM."""
+    nv, q = wn.shape
+    Q = sum(effect_widths(kinds, p, q))
+    dev = wn.device
+    GC = torch.empty(Q, (Q if with_g else 0) + L, device=dev, dtype=torch.float32)
+    check(_lib.load().gpp_kr_assemble_gc_blocks(_p(ST), ST.stride(0) if ST is not None else 0, _p(VM),
+                                                VM.stride(0) if VM is not None else 0, _p(wn), p, q, nv, L, len(kinds),
+                                                _lib.host_i32([EFFECT_KINDS[k] for k in kinds]), int(with_g), _p(GC),
+                                                GC.stride(0), _stream()), "kr_assemble_gc_blocks")
+    return GC
+
+
+@_on_device
+def kr_assemble_m_blocks(W: torch.Tensor, wn: torch.Tensor, p: int, kinds, L: int
+                         ) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """(M, R): M (p x nviews L) with W_O folded in, None without K and O; R (nviews x L), None without W."""
+    nv, q = wn.shape
+    M = torch.empty(p, nv * L, device=W.device, dtype=torch.float32) if ("kr" in kinds or "object" in kinds) else None
+    R = torch.empty(nv, L, device=W.device, dtype=torch.float32) if "view" in kinds else None
+    check(_lib.load().gpp_kr_assemble_m_blocks(_p(W), W.stride(0), _p(wn), p, q, nv, L, len(kinds),
+                                               _lib.host_i32([EFFECT_KINDS[k] for k in kinds]), _p(M),
+                                               M.stride(0) if M is not None else 0, _p(R),
+                                               R.stride(0) if R is not None else 0, _stream()), "kr_assemble_m_blocks")
+    return M, R
+
+
+@_on_device
+def kr_xb_nll_views(X: torch.Tensor, ldx: int, Y: torch.Tensor, R: torch.Tensor, d: torch.Tensor, w: torch.Tensor,
+                    P: int, nviews: int, L: int, scal: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    lib = _lib.load()
+    n = X.shape[0]
+    Xb = torch.empty(n, L, device=X.device, dtype=torch.float32)
+    nll = torch.empty(n, 1, device=X.device, dtype=torch.float32)
+    ws = _workspace(lib.gpp_kr_xb_workspace_bytes(n), X.device)
+    check(lib.gpp_kr_xb_nll_views(_p(X), ldx, _p(Y), Y.stride(0), _p(R), R.stride(0), _p(d), _p(w), n, P, nviews, L,
+                                  _p(scal), _p(Xb), L, _p(nll), _p(ws), ws.numel(), _stream()), "kr_xb_nll_views")
     return Xb, nll
 
 

@@ -117,7 +117,7 @@ class KhatriRao:
 
 
 class _KhatriRaoT:
-    def __init__(self, kr: KhatriRao):
+    def __init__(self, kr):
         self.kr = kr
         self.shape = torch.Size((kr.shape[1], kr.shape[0]))
 
@@ -125,6 +125,92 @@ class _KhatriRaoT:
         return self.kr.vtx(X)
 
     __matmul__ = mm
+
+
+class _FactoredEffect:
+    """A design over the tables and slot index of a KhatriRao `kr` (Vmodel.lazy_effects): the same tensor-like surface
+    as KhatriRao.  Several of them, with `kr` itself, are the designs of GP(n_rand_effs=k) on the structured route."""
+
+    kind = ""
+
+    def __init__(self, kr: KhatriRao, width: int):
+        self.kr = kr
+        self.n = kr.n
+        self.device = kr.device
+        self.shape = torch.Size((kr.n, width))
+
+    def detach(self) -> "_FactoredEffect":
+        return self
+
+    def dense(self) -> torch.Tensor:
+        return self._rows(self.kr.d, self.kr.w)
+
+    def __getitem__(self, idx) -> torch.Tensor:
+        return self._rows(self.kr.d[idx].contiguous(), self.kr.w[idx].contiguous())
+
+    def vtx(self, X: torch.Tensor) -> torch.Tensor:
+        """V^T X (width x m) through the slot sums (object) or the per-view sums (view): no N-long GEMM."""
+        Xm, ldx = ops.as_matrix(X, "X")
+        if Xm.shape[0] != self.n:
+            raise ValueError(f"X has {Xm.shape[0]} rows but V has {self.n}")
+        return effects_c(self.kr, [self.kind], Xm, ldx, Xm.shape[1])[: self.shape[1], : X.shape[1]]
+
+    def t(self) -> "_KhatriRaoT":
+        return _KhatriRaoT(self)
+
+
+class ObjectEffect(_FactoredEffect):
+    """The object-only design V[i, j] = x()[d_i, j] (n x p), held as the factors of `kr`."""
+
+    kind = "object"
+
+    def __init__(self, kr: KhatriRao):
+        super().__init__(kr, kr.p_true)
+
+    def _rows(self, d, w):
+        kr = self.kr   # xn (x) a one-column view table of ones is xn[d]
+        return ops.khatri_rao_fwd(kr.xn[:, : kr.p_true], torch.ones(kr.nviews, 1, device=kr.device), d, w)
+
+
+class ViewEffect(_FactoredEffect):
+    """The view-only design V[i, k] = v()[w_i, k] (n x q), held as the factors of `kr`."""
+
+    kind = "view"
+
+    def __init__(self, kr: KhatriRao):
+        super().__init__(kr, kr.q)
+
+    def _rows(self, d, w):
+        kr = self.kr   # a one-column object table of ones (x) wn is wn[w]
+        return ops.khatri_rao_fwd(torch.ones(kr.P, 1, device=kr.device), kr.wn, d, w)
+
+
+def effect_kind(V) -> str:
+    return "kr" if isinstance(V, KhatriRao) else V.kind
+
+
+def effect_base(V) -> KhatriRao:
+    return V if isinstance(V, KhatriRao) else V.kr
+
+
+def effects_st_vm(kr: KhatriRao, kinds, Xm: torch.Tensor, ldx: int, Lx: int, with_g: bool):
+    """The per-rank partial sums the stacked designs `kinds` need: ST (slot sums through x^T, None without K and O) and
+    VM (per-view moments, None without W)."""
+    ST = kr.st(Xm, ldx, Lx, with_g) if ("kr" in kinds or "object" in kinds) else None
+    VM = None
+    if "view" in kinds:
+        order, slot_start = kr.index()
+        VM = ops.kr_view_sums(Xm, ldx, order, slot_start, kr.xn, kr.nviews, Lx, with_g)
+    return ST, VM
+
+
+def effects_c(kr: KhatriRao, kinds, Xm: torch.Tensor, ldx: int, Lk: int, reduce=None) -> torch.Tensor:
+    """C = V^T X of the stacked designs `kinds` (padded block widths); `reduce(ST, VM)` sums the partials over row
+    shards (GP._all_reduce_pair)."""
+    ST, VM = effects_st_vm(kr, kinds, Xm, ldx, Lk, False)
+    if reduce is not None:
+        ST, VM = reduce(ST, VM)
+    return ops.kr_assemble_gc_blocks(ST, VM, kr.wn, kr.p, kinds, Lk, False)
 
 
 class Vmodel(nn.Module):
@@ -160,6 +246,15 @@ class Vmodel(nn.Module):
         else:
             self._lazy_index = (key, kr.index(), (kr.d, kr.w), kr.max_count())   # keeps d, w alive so the addresses stay theirs
         return kr
+
+    def lazy_effects(self, d: torch.Tensor, w: torch.Tensor, kinds=("kr", "object", "view")) -> list:
+        """Factored designs of GP(n_rand_effs=len(kinds)) for the rows (d, w): "kr" is `lazy(d, w)`, "object" the
+        object-only design x()[d] (ObjectEffect), "view" the view-only design v()[w] (ViewEffect).  They share one slot
+        index and one snapshot of the normalised tables, so GP takes the structured route with all of them."""
+        if not kinds or len(set(kinds)) != len(kinds) or any(k not in ("kr", "object", "view") for k in kinds):
+            raise ValueError(f"kinds must be distinct values of 'kr', 'object', 'view' (got {kinds})")
+        kr = self.lazy(d, w)
+        return [kr if k == "kr" else ObjectEffect(kr) if k == "object" else ViewEffect(kr) for k in kinds]
 
     def _init_params(self) -> None:
         """vmod.py:37-40: objects start at e_0 (+1e-3 noise), views at the identity (+1e-3 noise)."""

@@ -289,6 +289,37 @@ int gpp_kr_xb_nll(const float* X, int64_t ldx, const float* Y, int64_t ldy, cons
                   int64_t n, int64_t P, int32_t nviews, int32_t L, double* scal, float* Xb, int64_t ldxb, float* nll,
                   void* workspace, size_t workspace_bytes, gpp_stream_t stream);
 
+/* ---------------- several factored designs over one slot index (GP(n_rand_effs = k), k <= 3) ----------------
+ * The Khatri-Rao design V_K = xn[d] (x) wn[w], the object-only design V_O = xn[d] and the view-only design V_W = wn[w],
+ * stacked in the order of a HOST int32 list kinds_host[k] of distinct GPP_EFFECT_* values.  Block widths: p q (K),
+ * p (O), round4(q) (W; its padding rows and columns are exactly zero).  With the per-view first moments
+ *   z_v = sum_{i: w_i = v} X_i (L),   a_v = xn^T cnt[:, v] (p),   n_v = sum_o cnt[o, v]
+ * every block of GC = V^T [V | X] is a sum over v:  KK = wn_vk wn_vk' S_v,  KO = wn_vk S_v,  KW = wn_vk wn_vk' a_v,
+ * OO = S_v,  OW = a_v wn_vk',  WW = n_v wn_vk wn_vk';  C_K = wn_vk T_v,  C_O = T_v,  C_W = wn_vk z_v.
+ *   gpp_kr_view_sums         VM (nviews rows):  VM[v, 0 .. L) = z_v;  with_x: VM[v, L .. L + p) = a_v, VM[v, L + p] = n_v
+ *                            (exact up to 2^24 rows per view), VM[v, L + p + 1 .. L + p + 4) = 0.  Partials per block of
+ *                            objects (rows in slot order), then summed in a fixed order: no atomics.
+ *   gpp_kr_assemble_gc_blocks  the stacked GC (with_g) or C alone from ST (as gpp_kr_assemble_gc reads it; unused and
+ *                            may be NULL without K and O) and VM (unused and may be NULL without W).
+ *   gpp_kr_assemble_m_blocks  M (p x nviews L): M[j, v L + l] = sum_k wn[v,k] W_K[(j,k), l] + W_O[j, l] (needed with K or O)
+ *                            and R (nviews x L): R[v, l] = sum_k wn[v,k] W_W[k, l] (needed with W); then Y = xn M.
+ *   gpp_kr_xb_nll_views      gpp_kr_xb_nll with the per-view row:  Xb_i = (X_i - Y[d_i, w_i L ..] - R[w_i]) / vn. */
+enum gpp_effect_kind { GPP_EFFECT_KR = 0, GPP_EFFECT_OBJECT = 1, GPP_EFFECT_VIEW = 2 };
+size_t gpp_kr_view_sums_workspace_bytes(int64_t P, int32_t p, int32_t nviews, int32_t L, int32_t with_x);
+int gpp_kr_view_sums(const float* X, int64_t ldx, const int64_t* order, const int64_t* slot_start, const float* xn,
+                     int64_t P, int32_t p, int32_t nviews, int32_t L, int32_t with_x, float* VM, int64_t ldvm,
+                     void* workspace, size_t workspace_bytes, gpp_stream_t stream);
+int gpp_kr_assemble_gc_blocks(const float* ST, int64_t ldst, const float* VM, int64_t ldvm, const float* wn, int32_t p,
+                              int32_t q, int32_t nviews, int32_t L, int32_t k, const int32_t* kinds_host, int32_t with_g,
+                              float* GC, int64_t ldgc, gpp_stream_t stream);
+int gpp_kr_assemble_m_blocks(const float* W, int64_t ldw, const float* wn, int32_t p, int32_t q, int32_t nviews,
+                             int32_t L, int32_t k, const int32_t* kinds_host, float* M, int64_t ldm, float* R,
+                             int64_t ldr, gpp_stream_t stream);
+int gpp_kr_xb_nll_views(const float* X, int64_t ldx, const float* Y, int64_t ldy, const float* R, int64_t ldr,
+                        const int64_t* d, const int64_t* w, int64_t n, int64_t P, int32_t nviews, int32_t L,
+                        double* scal, float* Xb, int64_t ldxb, float* nll, void* workspace, size_t workspace_bytes,
+                        gpp_stream_t stream);
+
 /* Taylor surrogate (gp.py:127-133): out_i = Xb_i.X_i + Vb_i.V_i + <vbs, softmax(lvs)> / n      */
 int gpp_taylor_expansion_fwd(const float* X, int64_t ldx, const float* Xb, int64_t ldxb, const float* V,
                              int64_t ldv, const float* Vb, int64_t ldvb, int64_t n, int32_t L, int32_t Q,
