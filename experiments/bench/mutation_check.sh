@@ -1,0 +1,43 @@
+#!/bin/bash
+# Check that tests/test_gpu_kernel_edges.py bites: build three deliberately wrong variants of the library in throw-away
+# copies of the tree and run the tests that must catch each one.  Every mutation writes or reads LESS than the original
+# or changes a value; none widens a range or changes a trip count that producer and consumer warps must agree on.
+#   last_column_group  pass-2 epilogue of tc_rows_kernel skips its last float4 column group  -> section A (sentinels)
+#   last_split         tc_reduce_kernel sums splits - 1 partials                              -> section B (split knob)
+#   diagonal           the exact diagonal that colsq installs is scaled by 1 + 2^-20          -> colsq cases of pass 1
+# usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
+set -u
+OUT=$(mkdir -p "$1" && cd "$1" && pwd)
+ROOT=$(cd "$(dirname "$0")/../.." && pwd)
+TMP=$(mktemp -d)
+trap 'rm -rf "$TMP"' EXIT
+status=0
+run() {   # name file python-replacement pytest-selection...
+  local name=$1 file=$2 repl=$3
+  shift 3
+  local dst=$TMP/$name
+  mkdir -p "$dst"
+  (cd "$ROOT" && tar --exclude=./.git --exclude="./${OUT#"$ROOT"/}" --exclude=./gppvae_b200/build -cf - .) | tar -xf - -C "$dst"
+  python - "$dst/$file" "$repl" <<'EOF' || { echo "$name: mutation does not apply"; status=1; return; }
+import sys
+path, repl = sys.argv[1], sys.argv[2]
+old, new, count = repl.split("|||")
+src = open(path).read()
+assert src.count(old) == int(count), f"expected {count} occurrence(s) of {old!r}, found {src.count(old)}"
+open(path, "w").write(src.replace(old, new))
+EOF
+  (cd "$dst" && python -m gppvae_b200.build --force > "$OUT/$name.build.txt" 2>&1) || { echo "$name: build failed"; status=1; return; }
+  (cd "$dst" && python -m pytest -m gpu -x -q -p no:cacheprovider "$@" > "$OUT/$name.txt" 2>&1)
+  if [ $? -eq 0 ]; then
+    echo "$name: NOT caught"; status=1
+  else
+    echo "$name: caught"; grep -E "^(E |FAILED)" "$OUT/$name.txt" | head -8
+  fi
+}
+run last_column_group gppvae_b200/csrc/gemm_tc.cu "if (col0 + i < p.ncols) {|||if (col0 + i + 4 < p.ncols) {|||1" \
+  tests/test_gpu_kernel_edges.py -k "tc and (test_row_product_entries or test_xb_nll_entries)"
+run last_split gppvae_b200/csrc/gemm_tc.cu "for (int s = 0; s < p.splits; ++s) {|||for (int s = 0; s < p.splits - 1; ++s) {|||1" \
+  tests/test_gpu_kernel_edges.py -k test_split_rows_knob
+run diagonal gppvae_b200/csrc/gemm_tc.cu "= p.diag[row0 + r];|||= p.diag[row0 + r] * (1.0 + 0x1p-20);|||4" \
+  tests/test_gpu_kernel_edges.py -k "test_pass1_gram_entries and tc"
+exit $status
