@@ -1,10 +1,15 @@
 #!/bin/bash
-# Check that tests/test_gpu_kernel_edges.py bites: build three deliberately wrong variants of the library in throw-away
-# copies of the tree and run the tests that must catch each one.  Every mutation writes or reads LESS than the original
-# or changes a value; none widens a range or changes a trip count that producer and consumer warps must agree on.
+# Check that tests/test_gpu_kernel_edges.py and tests/test_gpu_structured_kernel_edges.py bite: build deliberately wrong
+# variants of the library in throw-away copies of the tree and run the tests that must catch each one.  Every mutation
+# writes or reads LESS than the original or changes a value; none widens a range or changes a trip count that producer
+# and consumer warps must agree on.
 #   last_column_group  pass-2 epilogue of tc_rows_kernel skips its last float4 column group  -> section A (sentinels)
 #   last_split         tc_reduce_kernel sums splits - 1 partials                              -> section B (split knob)
 #   diagonal           the exact diagonal that colsq installs is scaled by 1 + 2^-20          -> colsq cases of pass 1
+#   slot_last_row      kr_slot_sum_kernel drops the last row of each slot                     -> structured A
+#   view_last_chunk    kr_view_sums_reduce_kernel sums nchunks - 1 partials                   -> structured D
+#   views_r_w          kr_xb_views_kernel leaves R out of the .w component                    -> structured E
+#   shared_slot_scale  KhatriRao.st writes cnt (x) xn under the scale shared with the sums    -> structured B
 # usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
 set -u
 OUT=$(mkdir -p "$1" && cd "$1" && pwd)
@@ -40,4 +45,12 @@ run last_split gppvae_b200/csrc/gemm_tc.cu "for (int s = 0; s < p.splits; ++s) {
   tests/test_gpu_kernel_edges.py -k test_split_rows_knob
 run diagonal gppvae_b200/csrc/gemm_tc.cu "= p.diag[row0 + r];|||= p.diag[row0 + r] * (1.0 + 0x1p-20);|||4" \
   tests/test_gpu_kernel_edges.py -k "test_pass1_gram_entries and tc"
+run slot_last_row gppvae_b200/csrc/structured.cu "for (int64_t t = b; t < e; ++t) {|||for (int64_t t = b; t < e - 1; ++t) {|||1" \
+  tests/test_gpu_structured_kernel_edges.py -k test_kr_slot_sums
+run view_last_chunk gppvae_b200/csrc/structured.cu "for (int ch = 0; ch < nchunks; ++ch) s +=|||for (int ch = 0; ch < nchunks - 1; ++ch) s +=|||1" \
+  tests/test_gpu_structured_kernel_edges.py -k test_kr_view_sums
+run views_r_w gppvae_b200/csrc/structured.cu "(yy.w + r4.w)|||yy.w|||1" \
+  tests/test_gpu_structured_kernel_edges.py -k "test_kr_xb_nll_entries and views"
+run shared_slot_scale gppvae_b200/vmod.py "Lx, 2, self.max_count())|||Lx, 1, self.max_count())|||1" \
+  tests/test_gpu_structured_kernel_edges.py -k test_kr_st_per_range_floor
 exit $status

@@ -382,11 +382,14 @@ extern "C" int gpp_kr_slot_sums_planes(const float* X, int64_t ldx, int64_t n, c
                                        const int64_t* slot_start, const float* xn, int64_t P, int32_t p, int32_t nviews,
                                        int32_t L, int32_t with_x, int32_t max_count, void* planes, size_t planes_bytes_,
                                        gpp_stream_t stream) {
-  GPP_REQUIRE(X && order && slot_start && xn && planes, "kr_slot_sums_planes: null pointer");
-  GPP_REQUIRE(n > 0 && P > 0 && p > 0 && nviews > 0 && L > 0 && p % 4 == 0 && L % 4 == 0 && max_count >= 0,
+  GPP_REQUIRE(with_x >= 0 && with_x <= 2, "kr_slot_sums_planes: with_x must be 0, 1 or 2");
+  const bool reads_x = with_x != 2;
+  GPP_REQUIRE((X || !reads_x) && order && slot_start && xn && planes, "kr_slot_sums_planes: null pointer");
+  GPP_REQUIRE(n > 0 && P > 0 && p > 0 && nviews > 0 && p % 4 == 0 && (!reads_x || (L > 0 && L % 4 == 0)) && max_count >= 0,
               "kr_slot_sums_planes: p and L must be multiples of 4");
-  GPP_REQUIRE(mat_ok(X, ldx, L) && aligned16(xn) && planes_ok(planes), "kr_slot_sums_planes: bad leading dimension / alignment");
-  const int64_t cols = (int64_t)nviews * ((with_x ? p : 0) + L);
+  GPP_REQUIRE((!reads_x || mat_ok(X, ldx, L)) && aligned16(xn) && planes_ok(planes),
+              "kr_slot_sums_planes: bad leading dimension / alignment");
+  const int64_t cols = (int64_t)nviews * (with_x == 2 ? p : (with_x ? p : 0) + L);
   GPP_REQUIRE(cols < (1ll << 31) && planes_bytes_ >= planes_bytes(P, (int)cols), "kr_slot_sums_planes: planes buffer too small");
   return launch_kr_slot_sums_planes(X, ldx, n, order, slot_start, xn, P, p, nviews, L, with_x, max_count, planes,
                                     (cudaStream_t)stream);

@@ -681,11 +681,13 @@ __global__ void copy_u32_kernel(uint32_t* dst, const uint32_t* src) {
 // rows of slot s = o nviews + v (added in the order of `order`: deterministic).  The scale comes from a BOUND instead of a
 // scan of the result: |cnt xn| <= max_count (unit rows), |slot sum| <= max_count max|X| -- meta[0] is set by
 // slot_scale_kernel from the exact max|X| (one read of X) and the largest slot count (known to the caller from the
-// index).  One warp per slot.
-__global__ void slot_scale_kernel(uint32_t* __restrict__ meta, int max_count, int with_x) {
+// index).  One warp per slot.  mode (the entry's with_x): 0 the slot sums alone, bound max_count max|X|;  2 cnt (x) xn
+// alone, bound max_count;  1 both ranges in one buffer under ONE scale, max_count max(1, max|X|) -- the range whose
+// magnitude is far below that bound keeps fewer bits (DESIGN 5.4), so the route splits the two (modes 2 and 0).
+__global__ void slot_scale_kernel(uint32_t* __restrict__ meta, int max_count, int mode) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
-    float xmax = __uint_as_float(meta[2]);            // bits of max|X| (tc_absmax wrote them there)
-    if (with_x) xmax = fmaxf(xmax, 1.f);
+    float xmax = mode == 2 ? 1.f : __uint_as_float(meta[2]);   // bits of max|X| (tc_absmax wrote them there)
+    if (mode == 1) xmax = fmaxf(xmax, 1.f);
     meta[0] = __float_as_uint((float)max_count * xmax);
     meta[1] = 0u;
   }
@@ -1104,19 +1106,21 @@ int launch_pl_vb(const void* planesV, const float* Xb, int64_t ldxb, const float
 }
 
 // ---------------------------------------------------------------- structured route on planes
-// planes (P x nviews ((with_x ? p : 0) + L)) <- [cnt (x) xn | slot sums of X]; n = rows of X.
+// planes (P x nviews ((with_x ? p : 0) + L)) <- [cnt (x) xn | slot sums of X]; n = rows of X.  with_x = 2: the
+// cnt (x) xn part alone (P x nviews p, X is not read).
 int launch_kr_slot_sums_planes(const float* X, int64_t ldx, int64_t n, const int64_t* order, const int64_t* slot_start,
                                const float* xn, int64_t P, int p, int nviews, int L, int with_x, int max_count,
                                void* planes, cudaStream_t st) {
-  const int cols = nviews * ((with_x ? p : 0) + L);
+  const int Lz = with_x == 2 ? 0 : L;
+  const int cols = nviews * ((with_x ? p : 0) + Lz);
   PlanesView pv = planes_view(planes, P, cols);
-  GPP_TRY(tc_absmax(X, ldx, n, L, pv.meta + 2, st));
+  if (Lz) GPP_TRY(tc_absmax(X, ldx, n, L, pv.meta + 2, st));
   slot_scale_kernel<<<1, 32, 0, st>>>(pv.meta, max_count > 0 ? max_count : 1, with_x);
   GPP_LAUNCH_CHECK();
   const int64_t slots = P * nviews;
   const int grid = (int)(ceil_div(slots, 8) < 8192 ? ceil_div(slots, 8) : 8192);
-  kr_slot_sum_planes_kernel<<<grid, 256, 0, st>>>(X, ldx, order, slot_start, xn, P, p, nviews, L, with_x, pv.hi, pv.lo,
-                                                  pv.ldp, pv.meta);
+  kr_slot_sum_planes_kernel<<<grid, 256, 0, st>>>(X, ldx, order, slot_start, xn, P, p, nviews, Lz, with_x != 0, pv.hi,
+                                                  pv.lo, pv.ldp, pv.meta);
   GPP_LAUNCH_CHECK();
   return GPP_OK;
 }

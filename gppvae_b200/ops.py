@@ -382,13 +382,16 @@ def gram_vtz_planes(pV: Planes, pX: Optional[Planes], n: int, Q: int, L: int) ->
 
 
 @_on_device
-def atb_planes(pA: Planes, pB: Planes, n: int, ka: int, kb: int) -> torch.Tensor:
+def atb_planes(pA: Planes, pB: Planes, n: int, ka: int, kb: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """A^T B (ka x kb) from operand planes, into `out` when given (a ka x kb view; its row stride is the ld)."""
     lib = _lib.load()
     dev = pA.buf.device
     with torch.cuda.device(dev):
-        out = torch.empty(ka, kb, device=dev, dtype=torch.float32)
+        if out is None:
+            out = torch.empty(ka, kb, device=dev, dtype=torch.float32)
         ws = _workspace(lib.gpp_gram_planes_workspace_bytes(n, ka, kb), dev)
-        check(lib.gpp_atb_planes(pA.ptr, pB.ptr, n, ka, kb, _p(out), kb, _p(ws), ws.numel(), _stream(dev)), "atb_planes")
+        check(lib.gpp_atb_planes(pA.ptr, pB.ptr, n, ka, kb, _p(out), out.stride(0), _p(ws), ws.numel(), _stream(dev)),
+              "atb_planes")
     return out
 
 
@@ -560,11 +563,12 @@ def kr_slot_sums(X: torch.Tensor, ldx: int, order: torch.Tensor, slot_start: tor
 
 @_on_device
 def kr_slot_sums_planes(X: torch.Tensor, ldx: int, order: torch.Tensor, slot_start: torch.Tensor, xn: torch.Tensor,
-                        nviews: int, L: int, with_x: bool, max_count: int) -> Planes:
-    """The matrix of `kr_slot_sums` written directly as operand planes (no fp32 copy, no scan of it)."""
+                        nviews: int, L: int, with_x: int, max_count: int) -> Planes:
+    """The matrix of `kr_slot_sums` written directly as operand planes (no fp32 copy, no scan of it).  with_x = 2:
+    the cnt (x) xn part alone, under its own scale (include/gppvae_b200.h)."""
     lib = _lib.load()
     P, p = xn.shape
-    cols = nviews * ((p if with_x else 0) + L)
+    cols = nviews * (p if with_x == 2 else (p if with_x else 0) + L)
     with _guard(X):
         buf = _workspace(lib.gpp_planes_bytes(P, cols), X.device)
         check(lib.gpp_kr_slot_sums_planes(_p(X), ldx, X.shape[0], _p(order), _p(slot_start), _p(xn), P, p, nviews, L,

@@ -75,11 +75,19 @@ class KhatriRao:
     def st(self, Xm: torch.Tensor, ldx: int, Lx: int, with_x: bool) -> torch.Tensor:
         """ST = xn^T [cnt (x) xn | slot sums of X]  (p x nviews ((with_x ? p : 0) + Lx)).  From the tensor-core tile up
         (P >= 512, p >= 128) the slot sums are written as operand planes and the P-long product runs on the planes
-        kernel; below that, an fp32 matrix and the kernel that splits its operands itself."""
+        kernel; below that, an fp32 matrix and the kernel that splits its operands itself.  The two column ranges get
+        planes of their own, each with the scale of its own bound (max_count for cnt (x) xn, max_count max|X| for the
+        slot sums), as V and X have in the dense pass 1: under one shared scale the smaller range would lose bits."""
         order, slot_start = self.index()
         if ops.planes_supported(self.P, self.p, 0):
-            pXZ = ops.kr_slot_sums_planes(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, with_x, self.max_count())
-            return ops.atb_planes(self.xn_planes(), pXZ, self.P, self.p, pXZ.cols)
+            ncnt = self.nviews * self.p if with_x else 0
+            ST = torch.empty(self.p, ncnt + self.nviews * Lx, device=self.device, dtype=torch.float32)
+            if with_x:
+                pS = ops.kr_slot_sums_planes(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, 2, self.max_count())
+                ops.atb_planes(self.xn_planes(), pS, self.P, self.p, pS.cols, out=ST[:, : pS.cols])
+            pZ = ops.kr_slot_sums_planes(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, 0, self.max_count())
+            ops.atb_planes(self.xn_planes(), pZ, self.P, self.p, pZ.cols, out=ST[:, ncnt:])
+            return ST
         XZ = ops.kr_slot_sums(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, with_x)
         return ops.atb(self.xn, self.p, XZ, XZ.stride(0), self.P, self.p, XZ.shape[1])
 

@@ -269,10 +269,17 @@ int gpp_kr_slot_sums(const float* X, int64_t ldx, const int64_t* order, const in
                      int64_t P, int32_t p, int32_t nviews, int32_t L, int32_t with_x, float* XZ, int64_t ldxz,
                      gpp_stream_t stream);
 /* The same two products on operand planes (shapes from the tensor-core tile up: P >= 512, p >= 128):
- *   gpp_kr_slot_sums_planes  XZ written directly as planes (gpp_planes_bytes(P, nviews ((with_x ? p : 0) + L))): no fp32
- *                            copy, and no scan of it -- the scale comes from the bound max_count * max(1, max|X|), with
- *                            max_count = the largest number of rows in one slot (the caller knows it from the index)
- *                            and max|X| from one read of X (n rows);  ST = xn^T XZ is then gpp_atb_planes.
+ *   gpp_kr_slot_sums_planes  XZ written directly as planes (gpp_planes_bytes(P, cols)): no fp32 copy, and no scan of
+ *                            it -- the scale comes from a bound, with max_count = the largest number of rows in one slot
+ *                            (the caller knows it from the index) and max|X| from one read of X (n rows):
+ *                              with_x = 0  the slot sums alone, cols = nviews L, scale bound max_count max|X|;
+ *                              with_x = 2  cnt (x) xn alone, cols = nviews p, scale bound max_count (X is not read and
+ *                                          may be NULL; L is ignored);
+ *                              with_x = 1  both, cols = nviews (p + L), ONE scale for both, max_count max(1, max|X|):
+ *                                          the range far below that bound keeps fewer bits (|X| >> 1 costs cnt (x) xn
+ *                                          its precision, |X| << 1 or one crowded slot the slot sums).
+ *                            ST = xn^T XZ is then gpp_atb_planes; the route writes ST as two products (with_x = 2 and
+ *                            0, each into its column range of ST through ldo), so that each range keeps its own scale.
  *   gpp_am_planes            out = alpha A M from the planes of A (n x k) and M (k x m): Y = xn [M_0 | M_1 | ...];
  *                            workspace: 256 bytes. */
 int gpp_kr_slot_sums_planes(const float* X, int64_t ldx, int64_t n, const int64_t* order, const int64_t* slot_start,

@@ -59,6 +59,25 @@ def test_argument_validation_needs_no_device(lib):
     assert lib.gpp_gram_vtz(16, 8, 16, 8, 8, 6, 4, 16, 12, 16, 1 << 20, None) == -1
 
 
+def test_kr_slot_sums_planes_modes_need_no_device(lib):
+    """with_x selects the part of [cnt (x) xn | slot sums] the planes hold: 0, 1 or 2, nothing else; with_x = 2 (cnt (x) xn
+    alone) does not read X, so X may be NULL, and the planes it needs are P x nviews p."""
+    P, p, nviews, L = 512, 128, 3, 64
+    ok_ptr = 1 << 20      # 16-byte aligned, never dereferenced: every call below is rejected before a launch
+    need = lib.gpp_planes_bytes(P, nviews * p)
+    assert need < lib.gpp_planes_bytes(P, nviews * (p + L))
+    args = lambda X, with_x, nbytes: (X, L, 1000, ok_ptr, ok_ptr, ok_ptr, P, p, nviews, L, with_x, 10, ok_ptr, nbytes,
+                                      None)
+    assert lib.gpp_kr_slot_sums_planes(*args(ok_ptr, 3, need)) == -1
+    assert b"with_x must be 0, 1 or 2" in lib.gpp_last_error()
+    assert lib.gpp_kr_slot_sums_planes(*args(None, 1, need)) == -1
+    assert b"null pointer" in lib.gpp_last_error()
+    assert lib.gpp_kr_slot_sums_planes(*args(None, 2, need - 1)) == -1          # X NULL passes, the size does not
+    assert b"planes buffer too small" in lib.gpp_last_error()
+    assert lib.gpp_kr_slot_sums_planes(*args(ok_ptr, 0, lib.gpp_planes_bytes(P, nviews * L) - 1)) == -1
+    assert b"planes buffer too small" in lib.gpp_last_error()
+
+
 def test_workspace_sizes_are_consistent(lib):
     for n, Q, L in [(4005, 576, 256), (100_000, 1024, 256), (1_000_000, 4096, 256), (1, 4, 4)]:
         g = lib.gpp_gram_workspace_bytes(n, Q, L)
