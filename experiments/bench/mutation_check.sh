@@ -10,6 +10,8 @@
 #   view_last_chunk    kr_view_sums_reduce_kernel sums nchunks - 1 partials                   -> structured D
 #   views_r_w          kr_xb_views_kernel leaves R out of the .w component                    -> structured E
 #   shared_slot_scale  KhatriRao.st writes cnt (x) xn under the scale shared with the sums    -> structured B
+#   grad_rhs_last_h    kr_grad_rhs drops the last view's alpha H block from R (writes zero)     -> grad edges, table grad
+#   grad_rhs_m_sign    kr_grad_rhs writes +M_v^T instead of -M_v^T                             -> grad edges, table grad
 # usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
 set -u
 OUT=$(mkdir -p "$1" && cd "$1" && pwd)
@@ -53,4 +55,8 @@ run views_r_w gppvae_b200/csrc/structured.cu "(yy.w + r4.w)|||yy.w|||1" \
   tests/test_gpu_structured_kernel_edges.py -k "test_kr_xb_nll_entries and views"
 run shared_slot_scale gppvae_b200/vmod.py "Lx, 2, self.max_count())|||Lx, 1, self.max_count())|||1" \
   tests/test_gpu_structured_kernel_edges.py -k test_kr_st_per_range_floor
+run grad_rhs_last_h gppvae_b200/csrc/structured.cu "+ j0 + jj] = (float)(alpha * (double)s);|||+ j0 + jj] = v == nviews - 1 ? 0.f : (float)(alpha * (double)s);|||1" \
+  tests/test_gpu_structured_grad_kernel_edges.py tests/test_gpu_structured_table_grad.py -k "grad_rhs or c1"
+run grad_rhs_m_sign gppvae_b200/csrc/structured.cu "* ldr + j] = -s;|||* ldr + j] = s;|||1" \
+  tests/test_gpu_structured_grad_kernel_edges.py tests/test_gpu_structured_table_grad.py -k "grad_rhs or c1"
 exit $status

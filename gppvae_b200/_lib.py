@@ -104,6 +104,11 @@ _SIGNATURES = {
     "gpp_kr_xb_workspace_bytes": (c_size_t, [c_int64]),
     "gpp_kr_xb_nll": (c_int, [_PF, c_int64, _PF, c_int64, _PF, _PF, c_int64, c_int64, c_int32, c_int32, _PF, _PF,
                               c_int64, _PF, _PF, c_size_t, c_void_p]),
+    "gpp_kr_grad_rhs": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int32, c_int32, c_int32, c_int32, c_double, _PF,
+                                c_int64, c_void_p]),
+    "gpp_kr_grad_views_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "gpp_kr_grad_views": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, c_int32, c_int32, c_int32, c_int32,
+                                  c_double, _PF, c_int64, _PF, c_size_t, c_void_p]),
     "gpp_kr_view_sums_workspace_bytes": (c_size_t, [c_int64, c_int32, c_int32, c_int32, c_int32]),
     "gpp_kr_view_sums": (c_int, [_PF, c_int64, _PF, _PF, _PF, c_int64, c_int32, c_int32, c_int32, c_int32, _PF, c_int64,
                                  _PF, c_size_t, c_void_p]),

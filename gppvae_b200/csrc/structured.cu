@@ -385,6 +385,132 @@ __global__ void __launch_bounds__(256) kr_xb_views_kernel(const float* __restric
   }
 }
 
+// ---------------------------------------------------------------- NLL gradient to the tables (DESIGN 5.8)
+// Both entries walk B^-1 in tiles of q rows (j', .) by jc q columns (j0 .. j0 + jc, .): a tile is staged in shared memory
+// once (row stride jc q + 1, so that lanes walking k' hit distinct banks) and every view is served from it.
+inline int grad_tile_jc(int p, int q) {
+  const int jc = 4096 / (q * q);
+  return jc < 1 ? 1 : (jc > p ? p : jc);
+}
+inline size_t grad_smem_bytes(int p, int q, int nviews) {
+  const int jc = grad_tile_jc(p, q);
+  return ((size_t)nviews * q + (size_t)q * (jc * q + 1)) * sizeof(float);
+}
+constexpr size_t kGradSmemMax = 160 * 1024;
+
+__device__ __forceinline__ void grad_stage_tile(const float* __restrict__ Binv, int64_t ldb, int jp, int j0, int nj, int q,
+                                                float* tile, int ts) {
+  const int tw = nj * q;
+  for (int e = threadIdx.x; e < q * tw; e += blockDim.x) {
+    const int kk = e / tw, c = e - kk * tw;
+    tile[kk * ts + c] = Binv[(int64_t)(jp * q + kk) * ldb + (int64_t)j0 * q + c];
+  }
+}
+
+// R[v p + j', j] = alpha sum_{k', k} wn[v,k'] Binv[(j',k'), (j,k)] wn[v,k]  (alpha H_v).  Block (j', chunk of jc j's);
+// one warp per (view, j), lanes over the q x q entries of the tile, fixed-order warp sum.
+__global__ void __launch_bounds__(256) kr_grad_rhs_h_kernel(const float* __restrict__ Binv, int64_t ldb,
+                                                            const float* __restrict__ wn, int p, int q, int nviews,
+                                                            int jc, double alpha, float* __restrict__ R, int64_t ldr) {
+  extern __shared__ float gsm[];
+  float* wsm = gsm;                     // wn, nviews x q
+  float* tile = gsm + nviews * q;       // q x (jc q + 1)
+  const int jp = blockIdx.x, j0 = blockIdx.y * jc, nj = (p - j0 < jc) ? p - j0 : jc;
+  const int ts = jc * q + 1;
+  for (int e = threadIdx.x; e < nviews * q; e += blockDim.x) wsm[e] = wn[e];
+  grad_stage_tile(Binv, ldb, jp, j0, nj, q, tile, ts);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  for (int pr = warp; pr < nviews * nj; pr += nw) {
+    const int v = pr / nj, jj = pr - v * nj;
+    const float* wv = wsm + v * q;
+    float s = 0.f;
+    for (int e = lane; e < q * q; e += 32) {
+      const int kk = e / q, k = e - kk * q;
+      s = fmaf(wv[kk] * wv[k], tile[kk * ts + jj * q + k], s);
+    }
+    s = warp_sum(s);
+    if (lane == 0) R[(int64_t)(v * p + jp) * ldr + j0 + jj] = (float)(alpha * (double)s);
+  }
+}
+
+// R[nviews p + v L + l, j] = -sum_k wn[v,k] W[(j,k), l]  (-M_v^T; the sum of kr_assemble_m_kernel, in its order).
+__global__ void __launch_bounds__(256) kr_grad_rhs_m_kernel(const float* __restrict__ W, int64_t ldw,
+                                                            const float* __restrict__ wn, int p, int q, int nviews, int L,
+                                                            float* __restrict__ R, int64_t ldr) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= (int64_t)nviews * L * p) return;
+  const int64_t row = e / p;
+  const int j = (int)(e - row * p), v = (int)(row / L), l = (int)(row - (int64_t)v * L);
+  float s = 0.f;
+  for (int k = 0; k < q; ++k) s = fmaf(wn[v * q + k], W[(int64_t)(j * q + k) * ldw + l], s);
+  R[((int64_t)nviews * p + row) * ldr + j] = -s;
+}
+
+// part[j' nviews q + v q + k] = alpha sum_{j, k'} S_v[j, j'] wn[v,k'] Binv[(j',k'), (j,k)] - sum_l T_v[j',l] W[(j',k), l]
+// with S_v[j, j'] = ST[j, v p + j'] and T_v[j', l] = ST[j', nviews p + v L + l].  Block j' walks its q rows of B^-1 in
+// tiles; one warp per (view, k), lanes over (j, k') of the tile; a pair's sums over the tiles add in tile order.
+__global__ void __launch_bounds__(256) kr_grad_views_part_kernel(const float* __restrict__ ST, int64_t ldst,
+                                                                 const float* __restrict__ Binv, int64_t ldb,
+                                                                 const float* __restrict__ W, int64_t ldw,
+                                                                 const float* __restrict__ wn, int p, int q, int nviews,
+                                                                 int L, int jc, double alpha, float* __restrict__ part) {
+  extern __shared__ float gsm[];
+  float* wsm = gsm;                     // wn, nviews x q
+  float* tile = gsm + nviews * q;       // q x (jc q + 1)
+  const int jp = blockIdx.x, ts = jc * q + 1;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int npairs = nviews * q;
+  float* out = part + (int64_t)jp * npairs;
+  for (int e = threadIdx.x; e < nviews * q; e += blockDim.x) wsm[e] = wn[e];
+  for (int j0 = 0; j0 < p; j0 += jc) {
+    const int nj = (p - j0 < jc) ? p - j0 : jc;
+    __syncthreads();                    // the previous tile is consumed
+    grad_stage_tile(Binv, ldb, jp, j0, nj, q, tile, ts);
+    __syncthreads();
+    for (int pr = warp; pr < npairs; pr += nw) {
+      const int v = pr / q, k = pr - v * q;
+      const float* wv = wsm + v * q;
+      float s = 0.f;
+      for (int e = lane; e < nj * q; e += 32) {
+        const int jj = e / q, kk = e - jj * q;
+        s = fmaf(ST[(int64_t)(j0 + jj) * ldst + v * p + jp] * wv[kk], tile[kk * ts + jj * q + k], s);
+      }
+      s = warp_sum(s);
+      if (lane == 0) out[pr] = (j0 == 0 ? 0.f : out[pr]) + s;   // only this lane of this block touches out[pr]
+    }
+  }
+  for (int pr = warp; pr < npairs; pr += nw) {
+    const int v = pr / q, k = pr - v * q;
+    const float* t = ST + (int64_t)jp * ldst + (int64_t)nviews * p + (int64_t)v * L;
+    const float* wr = W + (int64_t)(jp * q + k) * ldw;
+    float s = 0.f;
+    for (int l = lane; l < L; l += 32) s = fmaf(t[l], wr[l], s);
+    s = warp_sum(s);
+    if (lane == 0) out[pr] = (float)(alpha * (double)out[pr]) - s;
+  }
+}
+
+// gw[v, k] = sum over j' of part[j'][v, k]: one warp per (v, k), lanes over j', fixed-order warp sum.
+__global__ void __launch_bounds__(256) kr_grad_views_reduce_kernel(const float* __restrict__ part, int p, int npairs,
+                                                                   int q, float* __restrict__ gw, int64_t ldgw) {
+  const int lane = threadIdx.x & 31;
+  const int pr = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (pr >= npairs) return;
+  float s = 0.f;
+  for (int jp = lane; jp < p; jp += 32) s += part[(int64_t)jp * npairs + pr];
+  s = warp_sum(s);
+  if (lane == 0) {
+    const int v = pr / q, k = pr - v * q;
+    gw[(int64_t)v * ldgw + k] = s;
+  }
+}
+
+inline int grad_set_smem(const void* kernel, size_t smem) {
+  if (smem > 48 * 1024) GPP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  return GPP_OK;
+}
+
 // Chunks of objects per view for the moments: about 8 blocks per SM over all views, a function of the shape alone.
 inline int64_t view_sums_chunks(int64_t P, int nviews) {
   const int64_t target = (1184 + nviews - 1) / nviews;
@@ -600,4 +726,61 @@ extern "C" int gpp_kr_xb_nll_views(const float* X, int64_t ldx, const float* Y, 
                                                   part);
   GPP_LAUNCH_CHECK();
   return launch_xb_finalize(quad, 1, n, part, kKrXbBlocks, fin, scal, nll, st);
+}
+
+extern "C" int gpp_kr_grad_rhs(const float* Binv, int64_t ldb, const float* W, int64_t ldw, const float* wn, int32_t p,
+                               int32_t q, int32_t nviews, int32_t L, double alpha, float* R, int64_t ldr,
+                               gpp_stream_t stream) {
+  GPP_REQUIRE(Binv && W && wn && R, "kr_grad_rhs: null pointer");
+  GPP_REQUIRE(p > 0 && q > 0 && nviews > 0 && L > 0 && p % 4 == 0 && L % 4 == 0,
+              "kr_grad_rhs: p and L must be positive multiples of 4");
+  GPP_REQUIRE(ldb >= (int64_t)p * q && ldw >= L && ldr >= p, "kr_grad_rhs: bad leading dimension");
+  GPP_REQUIRE((size_t)nviews * q * sizeof(float) <= 48 * 1024 && grad_smem_bytes(p, q, nviews) <= kGradSmemMax,
+              "kr_grad_rhs: view table or q too large for one tile of B^-1 in shared memory");
+  const int jc = grad_tile_jc(p, q);
+  const size_t smem = grad_smem_bytes(p, q, nviews);
+  GPP_TRY(grad_set_smem((const void*)kr_grad_rhs_h_kernel, smem));
+  cudaStream_t st = (cudaStream_t)stream;
+  kr_grad_rhs_h_kernel<<<dim3((unsigned)p, (unsigned)ceil_div(p, jc)), 256, smem, st>>>(Binv, ldb, wn, p, q, nviews, jc,
+                                                                                       alpha, R, ldr);
+  GPP_LAUNCH_CHECK();
+  const int64_t total = (int64_t)nviews * L * p;
+  kr_grad_rhs_m_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, st>>>(W, ldw, wn, p, q, nviews, L, R, ldr);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" size_t gpp_kr_grad_views_workspace_bytes(int32_t p, int32_t q, int32_t nviews) {
+  if (p <= 0 || q <= 0 || nviews <= 0) return 0;
+  return align_up((size_t)p * nviews * q * sizeof(float), 256);
+}
+
+extern "C" int gpp_kr_grad_views(const float* ST, int64_t ldst, const float* Binv, int64_t ldb, const float* W,
+                                 int64_t ldw, const float* wn, int32_t p, int32_t q, int32_t nviews, int32_t L,
+                                 double alpha, float* gw, int64_t ldgw, void* workspace, size_t workspace_bytes,
+                                 gpp_stream_t stream) {
+  GPP_REQUIRE(ST && Binv && W && wn && gw, "kr_grad_views: null pointer");
+  GPP_REQUIRE(p > 0 && q > 0 && nviews > 0 && L > 0 && p % 4 == 0 && L % 4 == 0,
+              "kr_grad_views: p and L must be positive multiples of 4");
+  GPP_REQUIRE(ldst >= (int64_t)nviews * (p + L) && ldb >= (int64_t)p * q && ldw >= L && ldgw >= q,
+              "kr_grad_views: bad leading dimension");
+  GPP_REQUIRE((size_t)nviews * q * sizeof(float) <= 48 * 1024 && grad_smem_bytes(p, q, nviews) <= kGradSmemMax,
+              "kr_grad_views: view table or q too large for one tile of B^-1 in shared memory");
+  const size_t need = gpp_kr_grad_views_workspace_bytes(p, q, nviews);
+  if (!workspace || workspace_bytes < need) {
+    set_error("kr_grad_views: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    return GPP_ERR_WORKSPACE;
+  }
+  const int jc = grad_tile_jc(p, q);
+  const size_t smem = grad_smem_bytes(p, q, nviews);
+  GPP_TRY(grad_set_smem((const void*)kr_grad_views_part_kernel, smem));
+  float* part = static_cast<float*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  kr_grad_views_part_kernel<<<(unsigned)p, 256, smem, st>>>(ST, ldst, Binv, ldb, W, ldw, wn, p, q, nviews, L, jc, alpha,
+                                                            part);
+  GPP_LAUNCH_CHECK();
+  const int npairs = nviews * q;
+  kr_grad_views_reduce_kernel<<<(unsigned)ceil_div(npairs, 8), 256, 0, st>>>(part, p, npairs, q, gw, ldgw);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
 }

@@ -25,7 +25,7 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from ._lib import GPP_MAX_DESIGNS, S_QUAD, S_XB2
+from ._lib import GPP_MAX_DESIGNS, S_QUAD, S_V0, S_VN, S_XB2
 from .vmod import KhatriRao, _FactoredEffect, effect_base, effect_kind, effects_c, effects_st_vm
 
 
@@ -128,6 +128,35 @@ class LazyVb:
         Xbr = self.Xb[idx].contiguous()
         Vb = ops.vb(Vp, self.Q, Xbr, self.fac.Binv, self.W, self.scal, m, self.Q, self.Lk, self.L)
         return Vb[:, : self.shape[1]]
+
+    def table_grads(self) -> Tuple[torch.Tensor, torch.Tensor]:
+        """The Khatri-Rao backward of this Vb (the contract of khatri_rao_bwd) through the slots, without forming Vb:
+        (gxn (P x p), gwn (nviews x q)), the gradients of sum(nll) to the normalised tables (DESIGN 5.8).
+
+            gxn = [cnt (x) xn | slot sums of Xb] R      R from kr_grad_rhs (alpha H_v over -M_v^T)
+            gwn = kr_grad_views(ST)                     ST = xn^T [cnt (x) xn | slot sums of Xb]
+
+        Only the rows of X this object was built from take part (a row shard's partial gradient), and rows with an
+        index outside the tables sit in no slot, so they add nothing.  Their rows of Xb are NaN, and the slot-sum
+        planes take their scale from max|Xb| over all rows, so those rows are zeroed first (a copy of Xb, made only
+        when such rows exist)."""
+        kr, Lk = self.kr, self.Lk
+        alpha = float(self.scal[S_V0] / self.scal[S_VN]) * self.L
+        Xb = self.Xb
+        n_in = kr.rows_in_table()
+        if n_in < kr.n:
+            Xb = Xb.index_fill(0, kr.index()[0][n_in:], 0.0)
+        ST, ops_left = kr.st_operands(Xb, Xb.stride(0), Lk, True)
+        R = ops.kr_grad_rhs(self.fac.Binv, self.W, kr.wn, kr.p, Lk, alpha)
+        ncnt = kr.nviews * kr.p
+        if isinstance(ops_left, tuple):     # operand planes: each range of the left operand keeps its own scale
+            pS, pZ = ops_left
+            gx = ops.am_planes(pS, ops.split_planes(R[:ncnt], kr.p, ncnt, kr.p), kr.P, ncnt, kr.p)
+            gx += ops.am_planes(pZ, ops.split_planes(R[ncnt:], kr.p, R.shape[0] - ncnt, kr.p), kr.P, pZ.cols, kr.p)
+        else:
+            gx = ops.am(ops_left, ops_left.stride(0), R, kr.p, kr.P, ops_left.shape[1], kr.p)
+        gw = ops.kr_grad_views(ST, self.fac.Binv, self.W, kr.wn, kr.p, Lk, alpha)
+        return gx[:, : kr.p_true], gw
 
     def dense(self, chunk: int = 65536) -> torch.Tensor:
         n = self.kr.n
@@ -761,8 +790,13 @@ class GP(nn.Module):
     def nll(self, X: torch.Tensor, Vs: Sequence[torch.Tensor]) -> torch.Tensor:
         """gp.py:97-110.  Differentiable: backward applies the Taylor coefficients (the exact gradients
         of sum(nll), gp.py:185-221), i.e. it is exact for a uniform upstream gradient (`.sum()`,
-        `.mean()`) -- the only way the reference ever differentiates it; any other upstream gradient raises."""
-        return _NllFunction.apply(self, X, self.lvs, *Vs)
+        `.mean()`) -- the only way the reference ever differentiates it; any other upstream gradient raises.  With a
+        KhatriRao from `Vmodel.lazy(d, w, requires_grad=True)` the gradient also reaches the tables (LazyVb.table_grads).
+        """
+        tables = ()
+        if self.n_rand_effs == 1 and len(Vs) == 1 and isinstance(Vs[0], KhatriRao) and Vs[0].tables is not None:
+            tables = Vs[0].tables     # Vmodel.lazy(..., requires_grad=True): the gradient reaches x0 and v0
+        return _NllFunction.apply(self, X, self.lvs, len(Vs), *Vs, *tables)
 
     def nll_ineff(self, X: torch.Tensor, Vs: Sequence[torch.Tensor]) -> torch.Tensor:
         """gp.py:112-125: O(N^3) cross-check through the dense N x N covariance.  Test utility, stock torch."""
@@ -797,17 +831,24 @@ class _NllFunction(torch.autograd.Function):
     every way the reference ever differentiates nll -- are exact."""
 
     @staticmethod
-    def forward(ctx, gp: GP, X, lvs, *Vs):
+    def forward(ctx, gp: GP, X, lvs, nV, *Vs_tables):
+        Vs, tables = Vs_tables[:nV], Vs_tables[nV:]
         want_grad = any(ctx.needs_input_grad[1:])
         dense = [torch.is_tensor(V) for V in Vs]
         ctx.dense = dense
+        ctx.nV = nV
+        ctx.lazy_vb = None
         with torch.no_grad():
             if want_grad:
-                # a factored V (vmod.KhatriRao) is a detached snapshot: no gradient flows to it, its Vb is never formed
-                need_vb = any(d and ng for d, ng in zip(dense, ctx.needs_input_grad[3:]))
+                # a factored V (vmod.KhatriRao) has no Vb to form: its tables (given after Vs when they are attached)
+                # get theirs through the slots, which needs B^-1 as the dense Vb does
+                want_tables = any(ctx.needs_input_grad[4 + nV:])
+                need_vb = want_tables or any(d and ng for d, ng in zip(dense, ctx.needs_input_grad[4:4 + nV]))
                 Xb, Vbs, vbs, nll = gp.taylor_coeff(X, list(Vs), need_vb=need_vb)
                 saved = [Vb for Vb, d in zip(Vbs, dense) if d and torch.is_tensor(Vb)]
                 ctx.n_vb = len(saved)
+                if want_tables:
+                    ctx.lazy_vb = Vbs[0]
                 ctx.save_for_backward(Xb, vbs, gp.get_vs().detach(), *saved)
             else:
                 nll = gp._coefficients(X, list(Vs), False)["nll"]
@@ -826,7 +867,13 @@ class _NllFunction(torch.autograd.Function):
         glvs = gbar * vs * (vbs - (vbs * vs).sum()) if ctx.needs_input_grad[2] else None
         it = iter(Vbs)
         gVs = []
-        for d, need in zip(ctx.dense, ctx.needs_input_grad[3:]):
+        for d, need in zip(ctx.dense, ctx.needs_input_grad[4:4 + ctx.nV]):
             Vb = next(it) if (d and ctx.n_vb) else None
             gVs.append(gbar * Vb if (need and Vb is not None) else None)
-        return (None, gX, glvs, *gVs)
+        n_tables = len(ctx.needs_input_grad) - 4 - ctx.nV
+        gtables = [None] * n_tables
+        if ctx.lazy_vb is not None:
+            gx, gw = ctx.lazy_vb.table_grads()
+            gtables = [gbar * gx if ctx.needs_input_grad[4 + ctx.nV] else None,
+                       gbar * gw if ctx.needs_input_grad[5 + ctx.nV] else None]
+        return (None, gX, glvs, None, *gVs, *gtables)

@@ -622,6 +622,29 @@ def kr_xb_nll(X: torch.Tensor, ldx: int, Y: torch.Tensor, d: torch.Tensor, w: to
     return Xb, nll
 
 
+@_on_device
+def kr_grad_rhs(Binv: torch.Tensor, W: torch.Tensor, wn: torch.Tensor, p: int, L: int, alpha: float) -> torch.Tensor:
+    """R (nviews (p + L) x p) = [alpha H_0; ..; alpha H_{nv-1}; -M_0^T; ..; -M_{nv-1}^T]: gxn = [cnt (x) xn | Xb sums] R."""
+    nv, q = wn.shape
+    R = torch.empty(nv * (p + L), p, device=W.device, dtype=torch.float32)
+    check(_lib.load().gpp_kr_grad_rhs(_p(Binv), Binv.stride(0), _p(W), W.stride(0), _p(wn), p, q, nv, L, float(alpha),
+                                      _p(R), R.stride(0), _stream()), "kr_grad_rhs")
+    return R
+
+
+@_on_device
+def kr_grad_views(ST: torch.Tensor, Binv: torch.Tensor, W: torch.Tensor, wn: torch.Tensor, p: int, L: int,
+                  alpha: float) -> torch.Tensor:
+    """The NLL gradient to the normalised view table (nviews x q) from ST = xn^T [cnt (x) xn | slot sums of Xb]."""
+    lib = _lib.load()
+    nv, q = wn.shape
+    gw = torch.empty(nv, q, device=W.device, dtype=torch.float32)
+    ws = _workspace(lib.gpp_kr_grad_views_workspace_bytes(p, q, nv), W.device)
+    check(lib.gpp_kr_grad_views(_p(ST), ST.stride(0), _p(Binv), Binv.stride(0), _p(W), W.stride(0), _p(wn), p, q, nv, L,
+                                float(alpha), _p(gw), gw.stride(0), _p(ws), ws.numel(), _stream()), "kr_grad_views")
+    return gw
+
+
 # ----------------------------------------------------------------------------- several factored designs
 @_on_device
 def kr_view_sums(X: torch.Tensor, ldx: int, order: torch.Tensor, slot_start: torch.Tensor, xn: torch.Tensor,

@@ -20,6 +20,8 @@ class KhatriRao:
     the structured route of csrc/structured.cu: V is never written and the N-long GEMMs shrink to P-long ones.
     It is a detached snapshot of the normalised tables (what `vm(Dt, Wt).detach()` is in train_gppvae.py:161);
     `dense()` materialises the reference tensor, `t().mm(X)` is V^T X (train_gppvae.py:237), `[idx]` the dense rows.
+    Made by `Vmodel.lazy(d, w, requires_grad=True)` it also keeps the attached tables (`tables`), and `GP.nll(X, [kr])`
+    then sends the exact NLL gradient to x0 and v0 through the slots (DESIGN 5.8), without the N x Q matrix dNLL/dV.
     """
 
     def __init__(self, xn: torch.Tensor, wn: torch.Tensor, d: torch.Tensor, w: torch.Tensor):
@@ -48,6 +50,8 @@ class KhatriRao:
         self._index = None
         self._max_count = None
         self._xn_planes = None
+        self._rows_in_table = None
+        self.tables = None       # (x(), v()) still attached to autograd: Vmodel.lazy(..., requires_grad=True)
 
     # -- index preparation (once per (d, w): the data set does not change between epochs) ------------------
     def index(self):
@@ -72,24 +76,38 @@ class KhatriRao:
             self.index()
         return self._max_count
 
+    def rows_in_table(self) -> int:
+        """Rows whose (d, w) lies inside the tables: the first rows_in_table() entries of `order` (the rest are the
+        trailing dummy slot).  One host read per KhatriRao, on first use."""
+        if self._rows_in_table is None:
+            self._rows_in_table = int(self.index()[1][-1])
+        return self._rows_in_table
+
     def st(self, Xm: torch.Tensor, ldx: int, Lx: int, with_x: bool) -> torch.Tensor:
         """ST = xn^T [cnt (x) xn | slot sums of X]  (p x nviews ((with_x ? p : 0) + Lx)).  From the tensor-core tile up
         (P >= 512, p >= 128) the slot sums are written as operand planes and the P-long product runs on the planes
         kernel; below that, an fp32 matrix and the kernel that splits its operands itself.  The two column ranges get
         planes of their own, each with the scale of its own bound (max_count for cnt (x) xn, max_count max|X| for the
         slot sums), as V and X have in the dense pass 1: under one shared scale the smaller range would lose bits."""
+        return self.st_operands(Xm, ldx, Lx, with_x)[0]
+
+    def st_operands(self, Xm: torch.Tensor, ldx: int, Lx: int, with_x: bool):
+        """(ST, left operand) of `st`: the left operand [cnt (x) xn | slot sums of X] is the pair of planes (pS, pZ)
+        (pS None without with_x) from the tensor-core tile up, else the fp32 matrix; the table gradient multiplies it
+        once more (LazyVb.table_grads)."""
         order, slot_start = self.index()
         if ops.planes_supported(self.P, self.p, 0):
             ncnt = self.nviews * self.p if with_x else 0
             ST = torch.empty(self.p, ncnt + self.nviews * Lx, device=self.device, dtype=torch.float32)
+            pS = None
             if with_x:
                 pS = ops.kr_slot_sums_planes(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, 2, self.max_count())
                 ops.atb_planes(self.xn_planes(), pS, self.P, self.p, pS.cols, out=ST[:, : pS.cols])
             pZ = ops.kr_slot_sums_planes(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, 0, self.max_count())
             ops.atb_planes(self.xn_planes(), pZ, self.P, self.p, pZ.cols, out=ST[:, ncnt:])
-            return ST
+            return ST, (pS, pZ)
         XZ = ops.kr_slot_sums(Xm, ldx, order, slot_start, self.xn, self.nviews, Lx, with_x)
-        return ops.atb(self.xn, self.p, XZ, XZ.stride(0), self.P, self.p, XZ.shape[1])
+        return ops.atb(self.xn, self.p, XZ, XZ.stride(0), self.P, self.p, XZ.shape[1]), XZ
 
     def xn_planes(self):
         """Operand planes of the normalised object table (the left operand of both P-long products), split once."""
@@ -240,11 +258,17 @@ class Vmodel(nn.Module):
         """V[i, j*q + k] = x()[d_i, j] * v()[w_i, k]  (vmod.py:28-35), differentiable w.r.t. x0 and v0."""
         return ops._KhatriRao.apply(self.x(), self.v(), d, w)
 
-    def lazy(self, d: torch.Tensor, w: torch.Tensor) -> KhatriRao:
+    def lazy(self, d: torch.Tensor, w: torch.Tensor, requires_grad: bool = False) -> KhatriRao:
         """The same V as `forward(d, w).detach()`, kept in factored form (see KhatriRao): the epoch-level call of
-        train_gppvae.py:161 when the GP term should take the structured route."""
-        with torch.no_grad():
-            kr = KhatriRao(self.x(), self.v(), d, w)
+        train_gppvae.py:161 when the GP term should take the structured route.  With `requires_grad=True` the KhatriRao
+        also keeps x() and v() attached, and `GP.nll(X, [kr])` sends the exact NLL gradient back to x0 and v0."""
+        if requires_grad:
+            xa, va = self.x(), self.v()
+            kr = KhatriRao(xa, va, d, w)
+            kr.tables = (xa, va)
+        else:
+            with torch.no_grad():
+                kr = KhatriRao(self.x(), self.v(), d, w)
         # the sort of the rows by (object, view) slot depends on (d, w) alone: the trainer passes the same index
         # tensors every epoch (train_gppvae.py:123-126, 161), so keep the last one
         key = (kr.d.data_ptr(), kr.d._version, kr.w.data_ptr(), kr.w._version, kr.n, kr.P, kr.nviews)

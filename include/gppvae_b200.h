@@ -295,6 +295,28 @@ size_t gpp_kr_xb_workspace_bytes(int64_t n);
 int gpp_kr_xb_nll(const float* X, int64_t ldx, const float* Y, int64_t ldy, const int64_t* d, const int64_t* w,
                   int64_t n, int64_t P, int32_t nviews, int32_t L, double* scal, float* Xb, int64_t ldxb, float* nll,
                   void* workspace, size_t workspace_bytes, gpp_stream_t stream);
+/* NLL gradient to the tables (DESIGN 5.8): the Khatri-Rao backward of Vb = alpha V B^-1 - Xb W^T, alpha = (v0/vn) L_true,
+ * through the slots.  With H_v = (I_p (x) wn_v)^T B^-1 (I_p (x) wn_v) (p x p) and M_v as in gpp_kr_assemble_m:
+ *   gpp_kr_grad_rhs    R (nviews (p + L) x p, ld = ldr):  R[v p + j', j] = alpha H_v[j', j],
+ *                      R[nviews p + v L + l, j] = -M_v[j, l], so that
+ *                      gxn = [cnt (x) xn | slot sums of Xb] R  (gpp_kr_slot_sums with_x = 1 and gpp_am, or the two
+ *                      ranges as planes, with_x = 2 and 0, and two gpp_am_planes summed).
+ *   gpp_kr_grad_views  gw (nviews x q, ld = ldgw) from ST = xn^T [cnt (x) xn | slot sums of Xb] (p x nviews (p + L), as
+ *                      gpp_atb writes it: S_v[j, j'] = ST[j, v p + j'], T_v[j, l] = ST[j, nviews p + v L + l]):
+ *                      gw[v, k] = alpha sum_{j,j',k'} S_v[j,j'] wn[v,k'] B^-1[(j',k'),(j,k)] - sum_{j,l} T_v[j,l] W[(j,k),l];
+ *                      workspace: gpp_kr_grad_views_workspace_bytes (p nviews q floats).
+ * Padding: the rows of R for zero (padded) columns of W are exactly zero.  The alpha H_v rows and columns of padded
+ * object features (p rounded up to 4) are NOT zero: there B^-1 is the identity, so R[v p + j, j] = alpha |wn_v|^2.  They
+ * meet zero columns of cnt (x) xn, so gxn's padded columns come out zero, and the caller drops them.
+ * Both read B^-1 (ld = ldb >= p q) once, in tiles of q rows shared by all views, and reduce in a fixed order without
+ * atomics: repeats are bit-identical.  p and L must be multiples of 4; nviews q floats must fit 48 KB, and one tile of
+ * B^-1 with the view table, (q (q + 1) + nviews q) floats, must fit 160 KB of shared memory (q up to about 200). */
+int gpp_kr_grad_rhs(const float* Binv, int64_t ldb, const float* W, int64_t ldw, const float* wn, int32_t p, int32_t q,
+                    int32_t nviews, int32_t L, double alpha, float* R, int64_t ldr, gpp_stream_t stream);
+size_t gpp_kr_grad_views_workspace_bytes(int32_t p, int32_t q, int32_t nviews);
+int gpp_kr_grad_views(const float* ST, int64_t ldst, const float* Binv, int64_t ldb, const float* W, int64_t ldw,
+                      const float* wn, int32_t p, int32_t q, int32_t nviews, int32_t L, double alpha, float* gw,
+                      int64_t ldgw, void* workspace, size_t workspace_bytes, gpp_stream_t stream);
 
 /* ---------------- several factored designs over one slot index (GP(n_rand_effs = k), k <= 3) ----------------
  * The Khatri-Rao design V_K = xn[d] (x) wn[w], the object-only design V_O = xn[d] and the view-only design V_W = wn[w],
