@@ -12,6 +12,9 @@
 #   shared_slot_scale  KhatriRao.st writes cnt (x) xn under the scale shared with the sums    -> structured B
 #   grad_rhs_last_h    kr_grad_rhs drops the last view's alpha H block from R (writes zero)     -> grad edges, table grad
 #   grad_rhs_m_sign    kr_grad_rhs writes +M_v^T instead of -M_v^T                             -> grad edges, table grad
+#   predict_no_h       kr_predict_rows drops the 2 x^T h_v term of the variance                -> predict edges, predict
+#   predict_last_h     kr_predict_views writes zero for the last view's H_v block               -> predict edges, predict
+#   predict_yh_at_l    kr_predict_rows reads YH at w_i L instead of w_i p                      -> predict edges, predict
 # usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
 set -u
 OUT=$(mkdir -p "$1" && cd "$1" && pwd)
@@ -59,4 +62,10 @@ run grad_rhs_last_h gppvae_b200/csrc/structured.cu "+ j0 + jj] = (float)(alpha *
   tests/test_gpu_structured_grad_kernel_edges.py tests/test_gpu_structured_table_grad.py -k "grad_rhs or c1"
 run grad_rhs_m_sign gppvae_b200/csrc/structured.cu "* ldr + j] = -s;|||* ldr + j] = s;|||1" \
   tests/test_gpu_structured_grad_kernel_edges.py tests/test_gpu_structured_table_grad.py -k "grad_rhs or c1"
+run predict_no_h gppvae_b200/csrc/structured.cu "(double)(a + 2.f * b + |||(double)(a + |||1" \
+  tests/test_gpu_predict_kernel_edges.py tests/test_gpu_predict.py -k "test_kr_predict_rows or k_designs"
+run predict_last_h gppvae_b200/csrc/structured.cu "H[(int64_t)jp * ldh + (int64_t)v * p + j] = s;|||H[(int64_t)jp * ldh + (int64_t)v * p + j] = v == nviews - 1 ? 0.f : s;|||1" \
+  tests/test_gpu_predict_kernel_edges.py tests/test_gpu_predict.py -k "test_kr_predict_views or trained"
+run predict_yh_at_l gppvae_b200/csrc/structured.cu "YH + di * ldyh + wi * p;|||YH + di * ldyh + wi * L;|||1" \
+  tests/test_gpu_predict_kernel_edges.py tests/test_gpu_predict.py -k "test_kr_predict_rows or trained"
 exit $status

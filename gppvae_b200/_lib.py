@@ -118,6 +118,11 @@ _SIGNATURES = {
                                          c_int64, _PF, c_int64, c_void_p]),
     "gpp_kr_xb_nll_views": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, _PF, c_int64, c_int64, c_int32,
                                     c_int32, _PF, _PF, c_int64, _PF, _PF, c_size_t, c_void_p]),
+    "gpp_kr_predict_views": (c_int, [_PF, c_int64, _PF, c_int32, c_int32, c_int32, c_int32, _I32H, _PF, c_int64, _PF,
+                                     _PF, c_void_p]),
+    "gpp_kr_predict_rows": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, _PF, _PF, _PF, _PF, c_int64, c_int64,
+                                    c_int32, c_int32, c_int32, _PF, _PF, c_int64, _PF, c_void_p]),
+    "gpp_rows_dot": (c_int, [_PF, c_int64, _PF, c_int64, c_int64, c_int32, _PF, _PF, c_void_p]),
     "gpp_taylor_expansion_fwd": (c_int, [_PF, c_int64, _PF, c_int64, _PF, c_int64, _PF, c_int64, c_int64, c_int32,
                                          c_int32, _PF, _PF, _PF, c_void_p]),
     "gpp_taylor_expansion_bwd": (c_int, [_PF, _PF, c_int64, _PF, c_int64, c_int64, c_int32, c_int32, _PF, _PF, _PF,

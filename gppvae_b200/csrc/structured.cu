@@ -506,6 +506,169 @@ __global__ void __launch_bounds__(256) kr_grad_views_reduce_kernel(const float* 
   }
 }
 
+// ---------------------------------------------------------------- posterior prediction at new rows (DESIGN 5.9)
+// The stacked new row is u = A_v x + b_v (x = xn[o], v its view), so var* = scal[V0] (x^T H_v x + 2 x^T h_v + c_v) with
+// H_v = A_v^T Binv A_v, h_v = A_v^T Binv b_v, c_v = b_v^T Binv b_v.  offK / offO / offW: first row of the K / O / W block
+// in Binv, -1 when the kind is absent.  Only the q true columns of the view block are read (wn has q columns).
+
+// H[j', v p + j] = sum_{k',k} wn[v,k'] wn[v,k] Binv[K(j',k'), K(j,k)] + sum_k' wn[v,k'] Binv[K(j',k'), O j]
+//                + sum_k wn[v,k] Binv[O j', K(j,k)] + Binv[O j', O j].
+// Block (j', chunk of jc j's): the KK tile is staged as in kr_grad_rhs_h_kernel and serves every view; one warp per
+// (view, j), lanes over the tile and the q KO / OK terms, fixed-order warp sum, then the OO entry.
+__global__ void __launch_bounds__(256) kr_predict_h_kernel(const float* __restrict__ Binv, int64_t ldb,
+                                                           const float* __restrict__ wn, int p, int q, int nviews,
+                                                           int jc, int offK, int offO, float* __restrict__ H,
+                                                           int64_t ldh) {
+  extern __shared__ float gsm[];
+  float* wsm = gsm;                     // wn, nviews x q
+  float* tile = gsm + nviews * q;       // q x (jc q + 1), with K only
+  const int jp = blockIdx.x, j0 = blockIdx.y * jc, nj = (p - j0 < jc) ? p - j0 : jc;
+  const int ts = jc * q + 1;
+  for (int e = threadIdx.x; e < nviews * q; e += blockDim.x) wsm[e] = wn[e];
+  if (offK >= 0) grad_stage_tile(Binv + (int64_t)offK * ldb + offK, ldb, jp, j0, nj, q, tile, ts);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  for (int pr = warp; pr < nviews * nj; pr += nw) {
+    const int v = pr / nj, jj = pr - v * nj, j = j0 + jj;
+    const float* wv = wsm + v * q;
+    float s = 0.f;
+    if (offK >= 0) {
+      for (int e = lane; e < q * q; e += 32) {
+        const int kk = e / q, k = e - kk * q;
+        s = fmaf(wv[kk] * wv[k], tile[kk * ts + jj * q + k], s);
+      }
+      if (offO >= 0) {
+        for (int k = lane; k < q; k += 32) {
+          s = fmaf(wv[k], Binv[(int64_t)(offK + jp * q + k) * ldb + offO + j], s);
+          s = fmaf(wv[k], Binv[(int64_t)(offO + jp) * ldb + offK + j * q + k], s);
+        }
+      }
+    }
+    s = warp_sum(s);
+    if (lane == 0) {
+      if (offO >= 0) s += Binv[(int64_t)(offO + jp) * ldb + offO + j];
+      H[(int64_t)jp * ldh + (int64_t)v * p + j] = s;
+    }
+  }
+}
+
+// Blocks j < p:  h[v p + j] = sum_{k,k'} wn[v,k] Binv[K(j,k), W k'] wn[v,k'] + sum_k' Binv[O j, W k'] wn[v,k'];
+// block p:       c[v] = sum_{k,k'} wn[v,k] Binv[W k, W k'] wn[v,k'].
+// The block stages its q x q tile of Binv (and the O row) once; one warp per view, fixed-order warp sum.
+__global__ void __launch_bounds__(256) kr_predict_hc_kernel(const float* __restrict__ Binv, int64_t ldb,
+                                                            const float* __restrict__ wn, int p, int q, int nviews,
+                                                            int offK, int offO, int offW, float* __restrict__ h,
+                                                            float* __restrict__ c) {
+  extern __shared__ float gsm[];
+  float* wsm = gsm;                     // wn, nviews x q
+  float* tile = gsm + nviews * q;       // q x (q + 1)
+  float* orow = tile + q * (q + 1);     // q
+  const int j = blockIdx.x, ts = q + 1;
+  const bool is_c = j == p;
+  const bool with_tile = is_c || offK >= 0, with_o = !is_c && offO >= 0;
+  for (int e = threadIdx.x; e < nviews * q; e += blockDim.x) wsm[e] = wn[e];
+  if (is_c) grad_stage_tile(Binv + (int64_t)offW * ldb + offW, ldb, 0, 0, 1, q, tile, ts);
+  else if (offK >= 0) grad_stage_tile(Binv + (int64_t)offK * ldb + offW, ldb, j, 0, 1, q, tile, ts);
+  if (with_o)
+    for (int e = threadIdx.x; e < q; e += blockDim.x) orow[e] = Binv[(int64_t)(offO + j) * ldb + offW + e];
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  for (int v = warp; v < nviews; v += nw) {
+    const float* wv = wsm + v * q;
+    float s = 0.f;
+    if (with_tile) {
+      for (int e = lane; e < q * q; e += 32) {
+        const int kk = e / q, k = e - kk * q;
+        s = fmaf(wv[kk] * wv[k], tile[kk * ts + k], s);
+      }
+    }
+    if (with_o)
+      for (int k = lane; k < q; k += 32) s = fmaf(orow[k], wv[k], s);
+    s = warp_sum(s);
+    if (lane == 0) {
+      if (is_c) c[v] = s;
+      else h[(int64_t)v * p + j] = s;
+    }
+  }
+}
+
+// One warp per new row i (o = d_i, v = w_i):  mean_i = Y[o, v L ..] (+ R[v]),
+// var_i = scal[V0] (xn[o] . YH[o, v p ..] + 2 xn[o] . h[v] + c[v]).  Rows with an index outside the tables are NaN.
+__global__ void __launch_bounds__(256) kr_predict_rows_kernel(const float* __restrict__ Y, int64_t ldy,
+                                                              const float* __restrict__ R, int64_t ldr,
+                                                              const float* __restrict__ YH, int64_t ldyh,
+                                                              const float* __restrict__ xn,
+                                                              const float* __restrict__ h, const float* __restrict__ c,
+                                                              const int64_t* __restrict__ d,
+                                                              const int64_t* __restrict__ w, int64_t m, int64_t P,
+                                                              int p, int nviews, int L, const double* __restrict__ scal,
+                                                              float* __restrict__ mean, int64_t ldmean,
+                                                              float* __restrict__ var) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const float qnan = __int_as_float(0x7fc00000);
+  const double v0 = scal[GPP_S_V0];
+  for (int64_t i = warp; i < m; i += nwarps) {
+    const int64_t di = d[i], wi = w[i];
+    const bool ok = (di >= 0) & (di < P) & (wi >= 0) & (wi < nviews);
+    float* out = mean + i * ldmean;
+    if (!ok) {
+      for (int cc = lane * 4; cc < L; cc += 128) *reinterpret_cast<float4*>(out + cc) = make_float4(qnan, qnan, qnan, qnan);
+      if (lane == 0) var[i] = qnan;
+      continue;
+    }
+    for (int cc = lane * 4; cc < L; cc += 128) {
+      float4 o;
+      if (Y) {
+        o = *reinterpret_cast<const float4*>(Y + di * ldy + wi * L + cc);
+        if (R) {
+          const float4 r4 = *reinterpret_cast<const float4*>(R + wi * ldr + cc);
+          o.x += r4.x; o.y += r4.y; o.z += r4.z; o.w += r4.w;
+        }
+      } else {
+        o = *reinterpret_cast<const float4*>(R + wi * ldr + cc);
+      }
+      *reinterpret_cast<float4*>(out + cc) = o;
+    }
+    float a = 0.f, b = 0.f;
+    if (YH) {
+      const float* x = xn + di * p;
+      const float* yh = YH + di * ldyh + wi * p;
+      for (int j = lane; j < p; j += 32) a = fmaf(x[j], yh[j], a);
+      if (h)
+        for (int j = lane; j < p; j += 32) b = fmaf(x[j], h[wi * p + j], b);
+    }
+    a = warp_sum(a);
+    b = warp_sum(b);
+    if (lane == 0) var[i] = (float)(v0 * (double)(a + 2.f * b + (c ? c[wi] : 0.f)));
+  }
+}
+
+// out_i = scal[V0] sum_c A[i, c] B[i, c]: one warp per row, float4 lanes, fixed-order warp sum.
+__global__ void __launch_bounds__(256) rows_dot_kernel(const float* __restrict__ A, int64_t lda,
+                                                       const float* __restrict__ B, int64_t ldb, int64_t m, int cols,
+                                                       const double* __restrict__ scal, float* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const double v0 = scal[GPP_S_V0];
+  for (int64_t i = warp; i < m; i += nwarps) {
+    float s = 0.f;
+    for (int cc = lane * 4; cc < cols; cc += 128) {
+      const float4 a = *reinterpret_cast<const float4*>(A + i * lda + cc);
+      const float4 b = *reinterpret_cast<const float4*>(B + i * ldb + cc);
+      s = fmaf(a.x, b.x, s); s = fmaf(a.y, b.y, s); s = fmaf(a.z, b.z, s); s = fmaf(a.w, b.w, s);
+    }
+    s = warp_sum(s);
+    if (lane == 0) out[i] = (float)(v0 * (double)s);
+  }
+}
+
+inline size_t predict_hc_smem_bytes(int q, int nviews) {
+  return ((size_t)nviews * q + (size_t)q * (q + 1) + q) * sizeof(float);
+}
+
 inline int grad_set_smem(const void* kernel, size_t smem) {
   if (smem > 48 * 1024) GPP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   return GPP_OK;
@@ -781,6 +944,73 @@ extern "C" int gpp_kr_grad_views(const float* ST, int64_t ldst, const float* Bin
   GPP_LAUNCH_CHECK();
   const int npairs = nviews * q;
   kr_grad_views_reduce_kernel<<<(unsigned)ceil_div(npairs, 8), 256, 0, st>>>(part, p, npairs, q, gw, ldgw);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_kr_predict_views(const float* Binv, int64_t ldb, const float* wn, int32_t p, int32_t q,
+                                    int32_t nviews, int32_t k, const int32_t* kinds_host, float* H, int64_t ldh,
+                                    float* h, float* c, gpp_stream_t stream) {
+  EffLayout lay;
+  int has = 0;
+  GPP_REQUIRE(p > 0 && q > 0 && nviews > 0 && p % 4 == 0, "kr_predict_views: p must be a positive multiple of 4");
+  GPP_REQUIRE(eff_layout(k, kinds_host, p, q, lay, has),
+              "kr_predict_views: kinds must list 1..3 distinct GPP_EFFECT_* values");
+  const bool with_k = has & (1 << GPP_EFFECT_KR), with_o = has & (1 << GPP_EFFECT_OBJECT);
+  const bool need_h = with_k || with_o, need_hc = has & (1 << GPP_EFFECT_VIEW);
+  GPP_REQUIRE(Binv && wn && (H || !need_h) && ((h && c) || !need_hc), "kr_predict_views: null pointer");
+  GPP_REQUIRE(ldb >= lay.off[k] && (!need_h || ldh >= (int64_t)nviews * p), "kr_predict_views: bad leading dimension");
+  GPP_REQUIRE((size_t)nviews * q * sizeof(float) <= 48 * 1024 && grad_smem_bytes(p, q, nviews) <= kGradSmemMax &&
+                  predict_hc_smem_bytes(q, nviews) <= kGradSmemMax,
+              "kr_predict_views: view table or q too large for one tile of B^-1 in shared memory");
+  int off[3] = {-1, -1, -1};
+  for (int b = 0; b < k; ++b) off[lay.kind[b]] = lay.off[b];
+  cudaStream_t st = (cudaStream_t)stream;
+  if (need_h) {
+    const int jc = with_k ? grad_tile_jc(p, q) : p;
+    const size_t smem = with_k ? grad_smem_bytes(p, q, nviews) : (size_t)nviews * q * sizeof(float);
+    GPP_TRY(grad_set_smem((const void*)kr_predict_h_kernel, smem));
+    kr_predict_h_kernel<<<dim3((unsigned)p, (unsigned)ceil_div(p, jc)), 256, smem, st>>>(
+        Binv, ldb, wn, p, q, nviews, jc, off[GPP_EFFECT_KR], off[GPP_EFFECT_OBJECT], H, ldh);
+    GPP_LAUNCH_CHECK();
+  }
+  if (need_hc) {
+    const size_t smem = predict_hc_smem_bytes(q, nviews);
+    GPP_TRY(grad_set_smem((const void*)kr_predict_hc_kernel, smem));
+    kr_predict_hc_kernel<<<(unsigned)(p + 1), 256, smem, st>>>(Binv, ldb, wn, p, q, nviews, off[GPP_EFFECT_KR],
+                                                                off[GPP_EFFECT_OBJECT], off[GPP_EFFECT_VIEW], h, c);
+    GPP_LAUNCH_CHECK();
+  }
+  return GPP_OK;
+}
+
+extern "C" int gpp_kr_predict_rows(const float* Y, int64_t ldy, const float* R, int64_t ldr, const float* YH,
+                                   int64_t ldyh, const float* xn, const float* h, const float* c, const int64_t* d,
+                                   const int64_t* w, int64_t m, int64_t P, int32_t p, int32_t nviews, int32_t L,
+                                   const double* scal, float* mean, int64_t ldmean, float* var, gpp_stream_t stream) {
+  GPP_REQUIRE(d && w && scal && mean && var && (Y || R) && (!YH || xn) && (!R || c), "kr_predict_rows: null pointer");
+  GPP_REQUIRE(m >= 0 && P > 0 && p > 0 && nviews > 0 && L > 0 && L % 4 == 0, "kr_predict_rows: bad shape");
+  GPP_REQUIRE((!Y || (ldy >= (int64_t)nviews * L && ldy % 4 == 0 && aligned16(Y))) &&
+                  (!R || (ldr >= L && ldr % 4 == 0 && aligned16(R))) && (!YH || ldyh >= (int64_t)nviews * p) &&
+                  ldmean >= L && ldmean % 4 == 0 && aligned16(mean),
+              "kr_predict_rows: bad leading dimension / alignment");
+  if (m == 0) return GPP_OK;
+  const int grid = (int)(ceil_div(m, 8) < 8192 ? ceil_div(m, 8) : 8192);
+  kr_predict_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(Y, ldy, R, ldr, YH, ldyh, xn, h, c, d, w, m, P, p,
+                                                                 nviews, L, scal, mean, ldmean, var);
+  GPP_LAUNCH_CHECK();
+  return GPP_OK;
+}
+
+extern "C" int gpp_rows_dot(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t m, int32_t cols,
+                            const double* scal, float* out, gpp_stream_t stream) {
+  GPP_REQUIRE(A && B && scal && out, "rows_dot: null pointer");
+  GPP_REQUIRE(m >= 0 && cols > 0 && cols % 4 == 0, "rows_dot: cols must be a positive multiple of 4");
+  GPP_REQUIRE(lda >= cols && lda % 4 == 0 && ldb >= cols && ldb % 4 == 0 && aligned16(A) && aligned16(B),
+              "rows_dot: bad leading dimension / alignment");
+  if (m == 0) return GPP_OK;
+  const int grid = (int)(ceil_div(m, 8) < 8192 ? ceil_div(m, 8) : 8192);
+  rows_dot_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(A, lda, B, ldb, m, cols, scal, out);
   GPP_LAUNCH_CHECK();
   return GPP_OK;
 }

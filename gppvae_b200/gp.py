@@ -787,6 +787,137 @@ class GP(nn.Module):
         Xb = c["Xb"][:, :L] if Lk != L else c["Xb"]
         return Xb, Vbs, vbs, c["nll"]
 
+    # ------------------------------------------------------------------ posterior prediction (DESIGN 5.9)
+    def predict(self, X: torch.Tensor, Vs: Sequence, Vs_new: Sequence) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Posterior mean (m x L) and variance (m x 1) of the noise-free latents at the new rows `Vs_new`, given the
+        training latents X and designs Vs (what taylor_coeff / nll take); float32, detached.
+
+            mean* = u W = v0 u V^T K^-1 X,    var* = scal[V0] u Binv u^T = v0 (u u^T - v0 u V^T K^-1 V u^T)
+
+        for a new stacked row u (W and Binv of the factorisation, Binv = D B^-1 D and scal[V0] = 1 for k designs).  One
+        variance per row, shared by the L columns; the observation z* has variance var* + vn.
+
+        `Vs_new` has the form of Vs: dense tensors of the same widths, or factored designs over the same (equal) tables
+        with the same kinds in the same order (`vm.lazy(dv, wv)`, `vm.lazy_effects(dv, wv, kinds)`); of those only d and w
+        are read.  Note that `vm.lazy(dv, wv)` replaces Vmodel's one-entry slot-index cache, so the next
+        `vm.lazy(Dt, Wt)` sorts the training rows again.  The factorisation goes through the cache with B^-1: after
+        taylor_coeff(X, Vs) it is a hit, and only C, the solve and the prediction stages run.  With row shards X and Vs
+        are this rank's rows and every rank predicts its own new rows without further communication.  New rows with an
+        index outside the tables get NaN.  Factored new rows form nothing of size m x Q (DESIGN 5.9)."""
+        with torch.no_grad():
+            return self._predict(X, list(Vs), list(Vs_new))
+
+    def _predict(self, X, Vs, Vs_new):
+        is_f = [isinstance(V, (KhatriRao, _FactoredEffect)) for V in Vs + Vs_new]
+        if any(is_f) and not all(is_f):
+            raise ValueError("predict: dense and factored designs cannot be mixed in Vs and Vs_new")
+        if len(Vs_new) != len(Vs):
+            raise ValueError(f"predict: Vs has {len(Vs)} designs but Vs_new has {len(Vs_new)}")
+        for i, (V, Vn) in enumerate(zip(Vs, Vs_new)):
+            if V.shape[1] != Vn.shape[1]:
+                raise ValueError(f"predict: Vs_new[{i}] has {Vn.shape[1]} columns but Vs[{i}] has {V.shape[1]}")
+        if not torch.is_tensor(X):
+            raise ValueError("predict: X must be a tensor")
+        devs = {X.device} | {V.device for V in Vs + Vs_new}
+        if len(devs) != 1:
+            raise ValueError(f"predict: X, Vs and Vs_new must be on one device (got {sorted(map(str, devs))})")
+        if all(is_f):
+            return self._predict_factored(X, Vs, Vs_new)
+        m = Vs_new[0].shape[0]
+        if m == 0 or any(Vn.shape[0] != m for Vn in Vs_new):
+            raise ValueError(f"predict: the new designs must have the same, positive number of rows "
+                             f"(got {[Vn.shape[0] for Vn in Vs_new]})")
+        return self._predict_dense(X, Vs, Vs_new, m)
+
+    def _predict_factored(self, X, Vs, Vs_new):
+        vs_attached = self.get_vs()
+        vs = vs_attached.detach()
+        if self.n_rand_effs == 1:
+            if len(Vs) != 1 or not isinstance(Vs[0], KhatriRao) or not isinstance(Vs_new[0], KhatriRao):
+                raise ValueError("predict: GP(n_rand_effs=1) takes one Khatri-Rao design (Vmodel.lazy) in Vs and Vs_new")
+            base, new, kinds = Vs[0], Vs_new[0], ["kr"]
+        else:
+            base, new = self._effects(Vs), self._effects(Vs_new)
+            kinds = [effect_kind(V) for V in Vs]
+            if [effect_kind(V) for V in Vs_new] != kinds:
+                raise ValueError(f"predict: Vs_new has kinds {[effect_kind(V) for V in Vs_new]} but Vs has {kinds}")
+        if new.n == 0:
+            raise ValueError("predict: Vs_new has no rows")
+        for name in ("xn", "wn"):
+            a, b = getattr(base, name), getattr(new, name)
+            if a.shape != b.shape or not torch.equal(a, b):
+                raise ValueError(f"predict: the tables of Vs_new differ from those of Vs ({name}): build both from the "
+                                 "same Vmodel state")
+        Xm, ldx = ops.as_matrix(X, "X")
+        n, L = X.shape
+        if base.n != n:
+            raise ValueError(f"X has {n} rows but the designs have {base.n}")
+        Lk = Xm.shape[1]
+        n_total = self._n_total(n, X.device)
+        if self.n_rand_effs == 1:
+            fac, C = self._kr_factorise(base, vs, True, Xm, ldx, Lk, vs_origin=vs_attached)
+            W, scal = ops.solve_w(fac, C, C.stride(0), Lk, L, n_total)
+            M, R = ops.kr_assemble_m(W, base.wn, base.p, Lk), None
+        else:
+            lay = self._effects_layout(base, kinds)
+            fac, C = self._effects_factorise(Vs, base, kinds, lay, vs, True, Xm, ldx, Lk, vs_origin=vs_attached)
+            W, scal, _ = ops.solve_w_blocks(fac, C, C.stride(0), Lk, L, n_total)
+            M, R = ops.kr_assemble_m_blocks(W, base.wn, base.p, kinds, Lk)
+        self._stage("solve:end")
+        Y = self._kr_y(base, M) if M is not None else None
+        H, h, c = ops.kr_predict_views(fac.Binv, base.wn, base.p, kinds)
+        YH = self._kr_y(base, H) if H is not None else None
+        mean, var = ops.kr_predict_rows(Y, R, YH, base.xn, h, c, new.d, new.w, base.P, base.nviews, Lk, scal)
+        self._stage("predict:end")
+        return (mean[:, :L] if Lk != L else mean), var
+
+    def _predict_dense(self, X, Vs, Vs_new, m, chunk: int = 65536):
+        vs_attached = self.get_vs()
+        vs = vs_attached.detach()
+        Xm, ldx = ops.as_matrix(X, "X")
+        n, L = X.shape
+        Lk = Xm.shape[1]
+        if any(V.shape[0] != n for V in Vs):
+            raise ValueError(f"X has {n} rows but the designs have {[V.shape[0] for V in Vs]}")
+        n_total = self._n_total(n, X.device)
+        if self.n_rand_effs == 1:
+            Vm, ldv, Q, _ = self._cat(Vs, vs)
+            fac, C, _ = self._factorise(Vm, ldv, Q, vs, True, Xm, ldx, Lk, vs_origin=vs_attached)
+            W, scal = ops.solve_w(fac, C, C.stride(0), Lk, L, n_total)
+            offsets = [0]
+        else:
+            stk = self._stack(Vs, Lk)
+            Q, offsets = stk.Q, stk.offsets
+            fac, C, _ = self._factorise(stk.V, stk.Q, stk.Q, vs, True, Xm, ldx, Lk, vs_origin=vs_attached, stk=stk)
+            W, scal, _ = ops.solve_w_blocks(fac, C, C.stride(0), Lk, L, n_total)
+        self._stage("solve:end")
+        mean = torch.empty(m, Lk, device=X.device, dtype=torch.float32)
+        var = torch.empty(m, 1, device=X.device, dtype=torch.float32)
+        pW = pB = None
+        for a in range(0, m, chunk):
+            b = min(m, a + chunk)
+            if len(Vs_new) == 1:
+                Vc, ldc = ops.as_matrix(Vs_new[0][a:b], "Vs_new[0]")
+            else:     # the stacked rows, zero-padded per block as the training operand is
+                Vc, ldc = torch.zeros(b - a, Q, device=X.device, dtype=torch.float32), Q
+                for o, Vn in zip(offsets, Vs_new):
+                    Vc[:, o:o + Vn.shape[1]] = Vn[a:b].detach()
+            mc = b - a
+            pV = ops.split_planes(Vc, ldc, mc, Q) if ops.planes_supported(mc, Q, Q) else None
+            if pV is not None and ops.planes_supported(mc, Q, Lk):
+                pW = pW or ops.split_planes(W, W.stride(0), Q, Lk)
+                mean[a:b] = ops.am_planes(pV, pW, mc, Q, Lk)
+            else:
+                mean[a:b] = ops.am(Vc, ldc, W, W.stride(0), mc, Q, Lk)
+            if pV is not None:
+                pB = pB or ops.split_planes(fac.Binv, Q, Q, Q)
+                VB = ops.am_planes(pV, pB, mc, Q, Q)
+            else:
+                VB = ops.am(Vc, ldc, fac.Binv, Q, mc, Q, Q)
+            var[a:b] = ops.rows_dot(VB, Vc, Q, scal)
+        self._stage("predict:end")
+        return (mean[:, :L] if Lk != L else mean), var
+
     def nll(self, X: torch.Tensor, Vs: Sequence[torch.Tensor]) -> torch.Tensor:
         """gp.py:97-110.  Differentiable: backward applies the Taylor coefficients (the exact gradients
         of sum(nll), gp.py:185-221), i.e. it is exact for a uniform upstream gradient (`.sum()`,

@@ -706,6 +706,49 @@ def kr_xb_nll_views(X: torch.Tensor, ldx: int, Y: torch.Tensor, R: torch.Tensor,
     return Xb, nll
 
 
+# ----------------------------------------------------------------------------- posterior prediction (GP.predict)
+@_on_device
+def kr_predict_views(Binv: torch.Tensor, wn: torch.Tensor, p: int, kinds
+                     ) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """(H, h, c) of the factored designs `kinds`: H = [H_0 | ..] (p x nviews p, None without K and O), h (nviews x p)
+    and c (nviews), both None without W (include/gppvae_b200.h, gpp_kr_predict_views)."""
+    nv, q = wn.shape
+    dev = wn.device
+    H = torch.empty(p, nv * p, device=dev, dtype=torch.float32) if ("kr" in kinds or "object" in kinds) else None
+    h = torch.empty(nv, p, device=dev, dtype=torch.float32) if "view" in kinds else None
+    c = torch.empty(nv, device=dev, dtype=torch.float32) if "view" in kinds else None
+    check(_lib.load().gpp_kr_predict_views(_p(Binv), Binv.stride(0), _p(wn), p, q, nv, len(kinds),
+                                           _lib.host_i32([EFFECT_KINDS[k] for k in kinds]), _p(H),
+                                           H.stride(0) if H is not None else 0, _p(h), _p(c), _stream()),
+          "kr_predict_views")
+    return H, h, c
+
+
+@_on_device
+def kr_predict_rows(Y: Optional[torch.Tensor], R: Optional[torch.Tensor], YH: Optional[torch.Tensor], xn: torch.Tensor,
+                    h: Optional[torch.Tensor], c: Optional[torch.Tensor], d: torch.Tensor, w: torch.Tensor, P: int,
+                    nviews: int, L: int, scal: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(mean (m x L), var (m x 1)) of the new rows (d, w) from the P-long products Y = xn M and YH = xn H."""
+    m, p = d.shape[0], xn.shape[1]
+    mean = torch.empty(m, L, device=d.device, dtype=torch.float32)
+    var = torch.empty(m, 1, device=d.device, dtype=torch.float32)
+    check(_lib.load().gpp_kr_predict_rows(_p(Y), Y.stride(0) if Y is not None else 0, _p(R),
+                                          R.stride(0) if R is not None else 0, _p(YH),
+                                          YH.stride(0) if YH is not None else 0, _p(xn), _p(h), _p(c), _p(d), _p(w), m, P,
+                                          p, nviews, L, _p(scal), _p(mean), L, _p(var), _stream()), "kr_predict_rows")
+    return mean, var
+
+
+@_on_device
+def rows_dot(A: torch.Tensor, B: torch.Tensor, cols: int, scal: torch.Tensor) -> torch.Tensor:
+    """out (m x 1) = scal[V0] * sum_c A[:, c] B[:, c] over the first `cols` columns."""
+    m = A.shape[0]
+    out = torch.empty(m, 1, device=A.device, dtype=torch.float32)
+    check(_lib.load().gpp_rows_dot(_p(A), A.stride(0), _p(B), B.stride(0), m, cols, _p(scal), _p(out), _stream()),
+          "rows_dot")
+    return out
+
+
 # ----------------------------------------------------------------------------- autograd glue
 class _NormalizeRows(torch.autograd.Function):
     @staticmethod

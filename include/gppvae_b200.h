@@ -349,6 +349,40 @@ int gpp_kr_xb_nll_views(const float* X, int64_t ldx, const float* Y, int64_t ldy
                         double* scal, float* Xb, int64_t ldxb, float* nll, void* workspace, size_t workspace_bytes,
                         gpp_stream_t stream);
 
+/* ---------------- posterior prediction at new rows (GP.predict; DESIGN 5.9) ----------------
+ * For a new row u of the stacked design (the designs' Binv as gpp_factor or gpp_factor_blocks leaves it, W from
+ * gpp_solve_w(_blocks)):  mean* = u W,  var* = scal[V0] u Binv u^T  -- the posterior mean and variance of the noise-free
+ * latent, one variance shared by all L columns (the observation adds scal[VN]).  On factored designs the row at
+ * (o, v) is u = A_v x + b_v with x = xn[o] (p) and w = wn[v] (q): A_v puts x (x) w in the K block and x in the O block,
+ * b_v puts w in the W block, so  var* = scal[V0] (x^T H_v x + 2 x^T h_v + c_v)  and  mean* = Y[o, v L ..] + R[v]  (Y, R
+ * from gpp_kr_assemble_m(_blocks) and gpp_am).  The kinds list is that of gpp_kr_assemble_m_blocks; a single Khatri-Rao
+ * design (gpp_factor with Q = p q) is kinds = {GPP_EFFECT_KR}.
+ *   gpp_kr_predict_views  H = [H_0 | ... | H_{nviews-1}] (p x nviews p, ld = ldh; NULL without K and O):
+ *                           H_v[j',j] = sum_{k',k} w_k' w_k Binv[K(j',k'), K(j,k)] + sum_k' w_k' Binv[K(j',k'), O j]
+ *                                       + sum_k w_k Binv[O j', K(j,k)] + Binv[O j', O j];
+ *                         h (nviews x p, contiguous) and c (nviews), both NULL without W:
+ *                           h_v[j] = sum_{k,k'} w_k Binv[K(j,k), W k'] w_k' + sum_k' Binv[O j, W k'] w_k',
+ *                           c_v = sum_{k,k'} w_k Binv[W k, W k'] w_k'.
+ *                         Binv (ld = ldb >= the stacked width) is read once, in tiles of q rows shared by every view (as
+ *                         gpp_kr_grad_rhs does); fixed-order sums without atomics.  Only the q true columns of the W
+ *                         block are read.  p must be a multiple of 4; nviews q floats must fit 48 KB, and one tile of
+ *                         Binv with the view table must fit 160 KB of shared memory (q up to about 200).
+ *   then YH = xn H (P x nviews p) with gpp_am / gpp_am_planes, the P-long product of the structured pass 2.
+ *   gpp_kr_predict_rows   one warp per new row i (o = d_i, v = w_i):  mean (m x L, ld = ldmean) = Y[o, v L ..] + R[v],
+ *                         var (m) = scal[V0] (xn[o] . YH[o, v p ..] + 2 xn[o] . h[v] + c[v]).  Y and YH (and xn) are NULL
+ *                         when the kinds are W alone; R, h and c are NULL without W.  A row with an index outside the
+ *                         tables gets NaN for mean and var.  Fixed order: repeats are bit-identical.  L % 4 == 0.
+ *   gpp_rows_dot          out_i = scal[V0] sum_c A[i, c] B[i, c]  (m rows, cols % 4 == 0): the variance of dense new rows
+ *                         from A = V* Binv and B = V*, one warp per row in a fixed order. */
+int gpp_kr_predict_views(const float* Binv, int64_t ldb, const float* wn, int32_t p, int32_t q, int32_t nviews, int32_t k,
+                         const int32_t* kinds_host, float* H, int64_t ldh, float* h, float* c, gpp_stream_t stream);
+int gpp_kr_predict_rows(const float* Y, int64_t ldy, const float* R, int64_t ldr, const float* YH, int64_t ldyh,
+                        const float* xn, const float* h, const float* c, const int64_t* d, const int64_t* w, int64_t m,
+                        int64_t P, int32_t p, int32_t nviews, int32_t L, const double* scal, float* mean, int64_t ldmean,
+                        float* var, gpp_stream_t stream);
+int gpp_rows_dot(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t m, int32_t cols, const double* scal,
+                 float* out, gpp_stream_t stream);
+
 /* Taylor surrogate (gp.py:127-133): out_i = Xb_i.X_i + Vb_i.V_i + <vbs, softmax(lvs)> / n      */
 int gpp_taylor_expansion_fwd(const float* X, int64_t ldx, const float* Xb, int64_t ldxb, const float* V,
                              int64_t ldv, const float* Vb, int64_t ldvb, int64_t n, int32_t L, int32_t Q,
