@@ -1,5 +1,5 @@
 #!/bin/bash
-# Check that tests/test_gpu_kernel_edges.py and tests/test_gpu_structured_kernel_edges.py bite: build deliberately wrong
+# Check that the elementwise edge tests (tests/test_gpu_*kernel_edges.py, tests/test_gpu_featmap_taylor_edges.py) bite: build deliberately wrong
 # variants of the library in throw-away copies of the tree and run the tests that must catch each one.  Every mutation
 # writes or reads LESS than the original or changes a value; none widens a range or changes a trip count that producer
 # and consumer warps must agree on.
@@ -15,6 +15,11 @@
 #   predict_no_h       kr_predict_rows drops the 2 x^T h_v term of the variance                -> predict edges, predict
 #   predict_last_h     kr_predict_views writes zero for the last view's H_v block               -> predict edges, predict
 #   predict_yh_at_l    kr_predict_rows reads YH at w_i L instead of w_i p                      -> predict edges, predict
+#   kr_bwd_last_view   khatri_rao_bwd_kernel skips the last view column (k < q - 1)            -> featmap D
+#   kr_planes_tail     kr_planes_kernel drops the last row of a chunk's tail loop              -> featmap A planes
+#   te_last_design     taylor_fwd_multi_kernel skips the last design                           -> featmap E multi
+#   te_last_glvs       taylor_bwd_multi_lvs_kernel leaves the last glvs unwritten              -> featmap E multi
+#   norm_bwd_sign      normalize_rows_bwd_kernel adds the projection instead of subtracting it -> featmap C
 # usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
 set -u
 OUT=$(mkdir -p "$1" && cd "$1" && pwd)
@@ -68,4 +73,14 @@ run predict_last_h gppvae_b200/csrc/structured.cu "H[(int64_t)jp * ldh + (int64_
   tests/test_gpu_predict_kernel_edges.py tests/test_gpu_predict.py -k "test_kr_predict_views or trained"
 run predict_yh_at_l gppvae_b200/csrc/structured.cu "YH + di * ldyh + wi * p;|||YH + di * ldyh + wi * L;|||1" \
   tests/test_gpu_predict_kernel_edges.py tests/test_gpu_predict.py -k "test_kr_predict_rows or trained"
+run kr_bwd_last_view gppvae_b200/csrc/featmap.cu "for (int k = lane; k < q; k += 32) {  // d/d wn|||for (int k = lane; k < q - 1; k += 32) {  // d/d wn|||1" \
+  tests/test_gpu_featmap_taylor_edges.py -k test_khatri_rao_bwd
+run kr_planes_tail gppvae_b200/csrc/gemm_planes.cu "for (; r < nr; ++r) {|||for (; r < nr - 1; ++r) {|||1" \
+  tests/test_gpu_featmap_taylor_edges.py -k test_khatri_rao_fwd_planes
+run te_last_design gppvae_b200/csrc/taylor.cu "for (int j = 0; j < t.k; ++j) s += row_dot(|||for (int j = 0; j < t.k - 1; ++j) s += row_dot(|||1" \
+  tests/test_gpu_featmap_taylor_edges.py -k test_taylor_multi
+run te_last_glvs gppvae_b200/csrc/taylor.cu "      glvs[b] = (float)(scale * (exp(|||      if (b < m - 1) glvs[b] = (float)(scale * (exp(|||1" \
+  tests/test_gpu_featmap_taylor_edges.py -k test_taylor_multi
+run norm_bwd_sign gppvae_b200/csrc/featmap.cu "(gr[c] - xr[c] * proj)|||(gr[c] + xr[c] * proj)|||1" \
+  tests/test_gpu_featmap_taylor_edges.py -k test_normalize_rows
 exit $status

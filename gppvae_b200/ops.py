@@ -345,15 +345,22 @@ def khatri_rao_fwd(xn: torch.Tensor, wn: torch.Tensor, d: torch.Tensor, w: torch
 def khatri_rao_bwd(gV: torch.Tensor, xn: torch.Tensor, wn: torch.Tensor, d: torch.Tensor, w: torch.Tensor
                    ) -> Tuple[torch.Tensor, torch.Tensor]:
     gV = gV.detach()
-    if gV.stride(1) != 1:
+    n, Q = gV.shape
+    # the kernel reads row r at gV + r * ldg with unit column stride: a broadcast upstream gradient (strides (0, 1) for
+    # V.sum(0), (0, 0) for V.sum()) or any other overlapping layout is copied first
+    if (Q > 1 and gV.stride(1) != 1) or (n > 1 and gV.stride(0) < Q):
         gV = gV.contiguous()
+    ldg = gV.stride(0) if n > 1 else Q
     P, p = xn.shape
     nv, q = wn.shape
-    gxn = torch.zeros_like(xn)
-    gwn = torch.zeros_like(wn)
-    check(_lib.load().gpp_khatri_rao_bwd(_p(gV), gV.stride(0), _p(xn.detach().contiguous()), P, p,
-                                         _p(wn.detach().contiguous()), nv, q, _p(d.contiguous()), _p(w.contiguous()),
-                                         d.shape[0], _p(gxn), _p(gwn), _stream()), "khatri_rao_bwd")
+    # row-major like the kernel's writes, whatever the layout of the tables (zeros_like would keep a transposed one's)
+    gxn = torch.zeros(P, p, device=xn.device, dtype=torch.float32)
+    gwn = torch.zeros(nv, q, device=wn.device, dtype=torch.float32)
+    # held until the launch: a copy passed as `_p(t.contiguous())` is freed before the next argument is built, whose
+    # own copy may then take the same block (a transposed xn was read as wn's copy)
+    xc, wc, dc, wic = xn.detach().contiguous(), wn.detach().contiguous(), d.contiguous(), w.contiguous()
+    check(_lib.load().gpp_khatri_rao_bwd(_p(gV), ldg, _p(xc), P, p, _p(wc), nv, q, _p(dc), _p(wic), d.shape[0], _p(gxn),
+                                         _p(gwn), _stream()), "khatri_rao_bwd")
     return gxn, gwn
 
 

@@ -89,3 +89,44 @@ def test_workspace_sizes_are_consistent(lib):
         assert lib.gpp_factor_state_bytes(Q) >= 3 * ((Q + 63) // 64 * 64) ** 2 * 4
         assert lib.gpp_solve_workspace_bytes(Q, L) > Q * L * 4
         assert lib.gpp_xb_workspace_bytes(n, Q, L) >= n * 4
+
+
+def test_featmap_and_taylor_validation_needs_no_device(lib):
+    """The feature-map and Taylor entries reject shapes their kernels cannot take before any launch: p + q past the
+    48 KB of staged table rows, p q or a design width not a multiple of 4, ldv % 4 != 0, k outside 1..16, ldg < p q."""
+    from gppvae_b200._lib import host_i32, host_i64, host_ptrs
+    ok = 1 << 20          # 16-byte aligned, never dereferenced: every call below is rejected before a launch
+    kr = lambda p, q, ldv: lib.gpp_khatri_rao_fwd(ok, 10, p, ok, 10, q, ok, ok, 100, ok, ldv, None)
+    assert kr(1533, 4, 1533 * 4) == -1 and b"too large" in lib.gpp_last_error()          # p + q = 1537
+    assert kr(3, 3, 12) == -1 and b"multiple of 4" in lib.gpp_last_error()
+    assert kr(4, 3, 14) == -1 and b"ldv" in lib.gpp_last_error()
+    assert kr(4, 3, 8) == -1                                                                # ldv < p q
+    kp = lambda p, q, ldv: lib.gpp_khatri_rao_fwd_planes(ok, 10, p, ok, 10, q, ok, ok, 600, ok, ldv, ok, 1 << 30, ok,
+                                                         1 << 30, None)
+    assert kp(3, 3, 12) == -1 and b"bad shape" in lib.gpp_last_error()
+    assert kp(4, 3, 14) == -1 and b"ldv" in lib.gpp_last_error()
+    assert lib.gpp_khatri_rao_bwd(ok, 11, ok, 10, 4, ok, 10, 3, ok, ok, 100, ok, ok, None) == -1   # ldg < p q
+    assert b"bad shape" in lib.gpp_last_error()
+    assert lib.gpp_normalize_rows_fwd(ok, 10, 0, ok, None) == -1
+    assert lib.gpp_normalize_rows_bwd(ok, ok, 10, 0, ok, None) == -1
+    te = lambda L, Q, ldv: lib.gpp_taylor_expansion_fwd(ok, 8, ok, 8, ok, ldv, ok, 12, 100, L, Q, ok, ok, ok, None)
+    assert te(6, 4, 12) == -1 and te(8, 9, 12) == -1 and b"bad shape" in lib.gpp_last_error()
+    assert te(8, 8, 10) == -1 and b"ld" in lib.gpp_last_error()
+    tb = lambda L, Q: lib.gpp_taylor_expansion_bwd(ok, ok, 8, ok, 12, 100, L, Q, ok, ok, ok, 8, ok, 12, ok, None)
+    assert tb(6, 4) == -1 and tb(8, 9) == -1
+    for k in (0, 17):
+        ptrs, lds, Qs = host_ptrs([ok] * 17), host_i64([8] * 17), host_i32([8] * 17)
+        assert lib.gpp_taylor_expansion_fwd_multi(ok, 8, ok, 8, k, ptrs, lds, ptrs, lds, Qs, 100, 8, ok, ok, ok,
+                                                  None) == -1
+        assert b"designs" in lib.gpp_last_error()
+        assert lib.gpp_taylor_expansion_bwd_multi(ok, ok, 8, k, ptrs, lds, Qs, 100, 8, ok, ok, ok, 8, ptrs, lds, ok,
+                                                  None) == -1
+        assert b"designs" in lib.gpp_last_error()
+    ptrs, lds, Qs = host_ptrs([ok] * 2), host_i64([8, 8]), host_i32([8, 6])
+    assert lib.gpp_taylor_expansion_fwd_multi(ok, 8, ok, 8, 2, ptrs, lds, ptrs, lds, Qs, 100, 8, ok, ok, ok, None) == -1
+    assert b"design 1 has 6 columns" in lib.gpp_last_error()
+    assert lib.gpp_taylor_expansion_bwd_multi(ok, ok, 8, 2, ptrs, lds, Qs, 100, 8, ok, ok, ok, 8, ptrs, lds, ok,
+                                              None) == -1
+    assert b"design 1 has 6 columns" in lib.gpp_last_error()
+    assert lib.gpp_split_planes_stacked(2, ptrs, lds, Qs, 600, 0, ok, 1 << 30, ok, 1 << 30, None) == -1
+    assert b"design 1 has 6 columns" in lib.gpp_last_error()
