@@ -20,7 +20,12 @@
 #   te_last_design     taylor_fwd_multi_kernel skips the last design                           -> featmap E multi
 #   te_last_glvs       taylor_bwd_multi_lvs_kernel leaves the last glvs unwritten              -> featmap E multi
 #   norm_bwd_sign      normalize_rows_bwd_kernel adds the projection instead of subtracting it -> featmap C
+#   host_lvs_slot0     the host entry's compute reads slot 0's lvs whatever its slot            -> host entry B
+#   host_nll_other     the host entry's copy-out takes nll from the other slot                  -> host entry A, B
+#   vbs_no_trb         vbs_kernel drops tr B^-1 from vbs[1]                                      -> host entry F, A
+#   host_planes_ltrue  the planes branch of the host entry runs solve_w with L_true = L - 4      -> host entry A
 # usage: mutation_check.sh OUT_DIR      (one log per mutation in OUT_DIR; exit 0 only if every mutation was caught)
+#        ONLY="name ..." mutation_check.sh OUT_DIR   runs the named mutations only
 set -u
 OUT=$(mkdir -p "$1" && cd "$1" && pwd)
 ROOT=$(cd "$(dirname "$0")/../.." && pwd)
@@ -30,6 +35,7 @@ status=0
 run() {   # name file python-replacement pytest-selection...
   local name=$1 file=$2 repl=$3
   shift 3
+  if [ -n "${ONLY:-}" ] && [[ " $ONLY " != *" $name "* ]]; then return; fi
   local dst=$TMP/$name
   mkdir -p "$dst"
   (cd "$ROOT" && tar --exclude=./.git --exclude="./${OUT#"$ROOT"/}" --exclude=./gppvae_b200/build -cf - .) | tar -xf - -C "$dst"
@@ -83,4 +89,12 @@ run te_last_glvs gppvae_b200/csrc/taylor.cu "      glvs[b] = (float)(scale * (ex
   tests/test_gpu_featmap_taylor_edges.py -k test_taylor_multi
 run norm_bwd_sign gppvae_b200/csrc/featmap.cu "(gr[c] - xr[c] * proj)|||(gr[c] + xr[c] * proj)|||1" \
   tests/test_gpu_featmap_taylor_edges.py -k test_normalize_rows
+run host_lvs_slot0 gppvae_b200/csrc/api.cu "softmax2_kernel<<<1, 32, 0, st>>>(F(o_lvs), F(o_vs));|||softmax2_kernel<<<1, 32, 0, st>>>(F(o_lvss[0]), F(o_vs));|||1" \
+  tests/test_gpu_host_entry.py -k test_every_input_changes_in_flight
+run host_nll_other gppvae_b200/csrc/api.cu "F(o_nll[s]), (size_t)n * 4, cudaMemcpyDeviceToHost|||F(o_nll[1 - s]), (size_t)n * 4, cudaMemcpyDeviceToHost|||1" \
+  tests/test_gpu_host_entry.py -k "test_every_input_changes_in_flight or test_branch_switch"
+run vbs_no_trb gppvae_b200/csrc/qspace.cu "((double)n_total - (double)Q + trb) / vn|||((double)n_total - (double)Q) / vn|||1" \
+  tests/test_gpu_host_entry.py -k "test_vbs_direct or test_branch_switch"
+run host_planes_ltrue gppvae_b200/csrc/api.cu "Q + L, Q, L, L, n, F(o_W)|||Q + L, Q, L, L - 4, n, F(o_W)|||1" \
+  tests/test_gpu_host_entry.py -k test_branch_switch
 exit $status

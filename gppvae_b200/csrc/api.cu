@@ -3,6 +3,7 @@
 #include <stdarg.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <string>
 
@@ -447,6 +448,7 @@ struct gpp_host_ctx {
   void* arena = nullptr;
   size_t arena_bytes = 0;
   unsigned next = 0;
+  int64_t layout[6] = {0, 0, 0, 0, 0, 0};   // (P, p, nviews, q, n, L) of the last submission: the arena's carving
 };
 
 extern "C" int gpp_host_ctx_create(gpp_host_ctx** ctx) {
@@ -571,6 +573,13 @@ extern "C" int gpp_gp_term_host_submit(gpp_host_ctx* ctx, const float* x0_host, 
   // copy-in stream: the inputs of slot s, once the compute that last read this slot is done; small ones first
   cudaStream_t ci = ctx->copy_in;
   if (ctx->used[s]) GPP_CUDA(cudaStreamWaitEvent(ci, ctx->comp_done[s], 0));
+  // A new shape carves the arena differently, so slot s may now overlap the inputs, Xb and nll of the other slot's
+  // submission.  If that one is still in flight, start the copies only once its results have left the device.  The
+  // compute below waits on these copies (small_done), so it is ordered behind them too.  The wait is on the device:
+  // the host is not blocked, and a same-shape submission issues no extra call.
+  const int64_t layout[6] = {P, p, nviews, q, n, L};
+  if (ctx->used[1 - s] && ctx->out_pending[1 - s] && !std::equal(layout, layout + 6, ctx->layout))
+    GPP_CUDA(cudaStreamWaitEvent(ci, ctx->out_done[1 - s], 0));
   GPP_CUDA(cudaMemcpyAsync(F(o_x0), x0_host, (size_t)P * p * 4, cudaMemcpyHostToDevice, ci));
   GPP_CUDA(cudaMemcpyAsync(F(o_v0), v0_host, (size_t)nviews * q * 4, cudaMemcpyHostToDevice, ci));
   GPP_CUDA(cudaMemcpyAsync(d_dev, d_host, (size_t)n * 8, cudaMemcpyHostToDevice, ci));
@@ -623,6 +632,7 @@ extern "C" int gpp_gp_term_host_submit(gpp_host_ctx* ctx, const float* x0_host, 
   GPP_CUDA(cudaEventRecord(ctx->out_done[s], ctx->copy_out));
   ctx->out_pending[s] = true;
   ctx->used[s] = true;
+  std::copy(layout, layout + 6, ctx->layout);
   *ticket = s;
   ++ctx->next;
   return GPP_OK;

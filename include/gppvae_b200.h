@@ -407,7 +407,12 @@ int gpp_taylor_expansion_bwd(const float* gout, const float* Xb, int64_t ldxb, c
  *   gpp_gp_term_host         = submit + wait (synchronous).
  * The host buffers of a submission must stay valid and untouched until its wait returns.  Device buffers live in the
  * context and are reused across calls.  Xb_host or vbs_host may be NULL to skip that copy.  Host buffers should be
- * pinned (page-locked) for the copies to be asynchronous and at full PCIe speed. */
+ * pinned (page-locked) for the copies to be asynchronous and at full PCIe speed.
+ * Shapes: every submission may have its own (P, p, nviews, q, n, L).  Consecutive submissions of one shape overlap as
+ * described above.  A submission whose shape differs from the previous one's starts copying its inputs only once the
+ * results of the submission still in flight have reached the host (a device-side wait; submit does not block for it),
+ * since the device buffers are laid out per shape.  One that needs a larger device arena first waits for all work on
+ * the device (cudaDeviceSynchronize), not only this context's. */
 typedef struct gpp_host_ctx gpp_host_ctx;
 int gpp_host_ctx_create(gpp_host_ctx** ctx);
 int gpp_host_ctx_destroy(gpp_host_ctx* ctx);

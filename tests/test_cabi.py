@@ -130,3 +130,40 @@ def test_featmap_and_taylor_validation_needs_no_device(lib):
     assert b"design 1 has 6 columns" in lib.gpp_last_error()
     assert lib.gpp_split_planes_stacked(2, ptrs, lds, Qs, 600, 0, ok, 1 << 30, ok, 1 << 30, None) == -1
     assert b"design 1 has 6 columns" in lib.gpp_last_error()
+
+
+def test_host_entry_validation_needs_no_device(lib):
+    """The host-buffer entry and gpp_factor_solve reject bad arguments before they touch the context or the device: a
+    null context, tickets other than 0 and 1, a null required pointer, p q or L not a multiple of 4, p q >= 2^30,
+    Q % 4 != 0 and ldgc < Q + L or ldgc % 4 != 0."""
+    import ctypes
+    ok = 1 << 20          # 16-byte aligned, never dereferenced: every call below is rejected before any use
+    tk = ctypes.c_int32(-7)
+    ptrs = dict(ctx=ok, x0=ok, v0=ok, d=ok, w=ok, X=ok, lvs=ok, nll=ok)
+
+    def submit(P=100, p=16, q=8, n=1000, L=64, ticket=True, **null):
+        a = {k: (None if k in null else v) for k, v in ptrs.items()}
+        return lib.gpp_gp_term_host_submit(a["ctx"], a["x0"], P, p, a["v0"], q, q, a["d"], a["w"], a["X"], n, L, a["lvs"],
+                                           a["nll"], ok, ok, ctypes.byref(tk) if ticket else None)
+
+    for k in ptrs:
+        assert submit(**{k: True}) == -1 and b"null pointer" in lib.gpp_last_error(), k
+    assert submit(ticket=False) == -1 and b"null pointer" in lib.gpp_last_error()
+    assert tk.value == -7, "a rejected submission set the ticket"
+    assert submit(p=3, q=3) == -1 and b"multiples of 4" in lib.gpp_last_error()
+    assert submit(L=6) == -1 and b"multiples of 4" in lib.gpp_last_error()
+    assert submit(p=1 << 15, q=1 << 15) == -1 and b"multiples of 4" in lib.gpp_last_error()     # p q = 2^30
+    for bad in dict(P=0), dict(p=0), dict(q=0), dict(n=0), dict(L=0):
+        assert submit(**bad) == -1 and b"bad shape" in lib.gpp_last_error(), bad
+    assert lib.gpp_gp_term_host(None, ok, 100, 16, ok, 8, 8, ok, ok, ok, 1000, 64, ok, ok, ok, ok) == -1
+    for t in (-1, 2):
+        assert lib.gpp_gp_term_host_wait(ok, t) == -1 and b"bad ticket" in lib.gpp_last_error()
+    assert lib.gpp_gp_term_host_wait(None, 0) == -1
+    assert lib.gpp_host_ctx_create(None) == -1
+    assert lib.gpp_host_ctx_destroy(None) == 0
+    fs = lambda Q, L, ldgc: lib.gpp_factor_solve(ok, ldgc, Q, L, ok, 100, 0, ok, L, None, ok, ok, 1 << 30, None)
+    assert fs(6, 4, 12) == -1 and b"bad shape" in lib.gpp_last_error()
+    assert fs(8, 6, 16) == -1 and b"bad shape" in lib.gpp_last_error()
+    assert fs(8, 4, 8) == -1 and b"bad GC" in lib.gpp_last_error()           # ldgc < Q + L
+    assert fs(8, 4, 14) == -1 and b"bad GC" in lib.gpp_last_error()          # ldgc % 4 != 0
+    assert lib.gpp_vbs(None, 100, 8, 4, ok, None) == -1 and lib.gpp_vbs(ok, 0, 8, 4, ok, None) == -1
